@@ -20,6 +20,12 @@ Default run (`python bench.py [--gpus N --steps K --warmup W]`, what the driver 
 `--workload trace` / `--workload render --scene ...` run one part alone (A/B scripts in variants/). `--impl reference` times the
 oracle port (the reference is C#/.NET and cannot run here) on the host cores with the same line shape.
 Only this file's cpu_baseline / --impl reference legs execute oracle/ (as the timed CPU stand-in for the reference's C# path).
+
+`--dump-outputs DIR` writes what the timed path returned in its last timed step as DIR/<name>.npy (float32 / float64, under 64 MB):
+the C2 hits (a miss with distance -1) and occlusion flags of a fixed sample of rank 0's rays, and the resolved frame of every render record at a fixed sample
+of its pixels. The inputs depend only on the arguments, so two builds can be compared output for output. A render's host thread
+picks the kernel of a bounce from the ray counts it has seen so far (csrc/render.cu, evaluate_paths), so a stalled run can differ
+from another one in a few pixels of a frame (measured on one B200 at 1000 W: C3); compare frames with a tolerance.
 """
 import argparse
 import json
@@ -31,6 +37,7 @@ import time
 
 import numpy as np
 
+sys.dont_write_bytecode = True  # the tree it runs from may be read-only: nothing is written there
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
@@ -69,13 +76,36 @@ def parse():
     parser.add_argument("--pattern", default="hilbert", choices=["hilbert", "ordered"],
                         help="render: tile sequence, the HilbertCurvePattern of EvaluationProfile.Pattern (reference default) or an OrderedPattern")
     parser.add_argument("--reduce-every", type=int, default=1, help="--workload render: steps (epochs) accumulated on the device between frame all-reduces")
-    parser.add_argument("--render-steps", type=int, default=12, help="default run: timed steps of each `render` record (at most --steps when that is smaller)")
+    parser.add_argument("--render-steps", type=int, default=None, help="default run: timed steps of each `render` record (default: --steps; at most --steps when given)")
     parser.add_argument("--render-warmup", type=int, default=1, help="default run: warm-up steps of each `render` record (a C5 step is seconds long)")
     parser.add_argument("--no-render", action="store_true", help="default run: skip the `render` records")
     parser.add_argument("--no-cpu-baseline", action="store_true")
     parser.add_argument("--no-tree-build", action="store_true", help="skip the device tree build record (device SweepBuilder beside the host mirror)")
     parser.add_argument("--no-secondary", action="store_true", help="skip the secondary-ray batch reported beside the headline (SURVEY.md 8d)")
-    return parser.parse_args()
+    parser.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step as DIR/<name>.npy (rank 0; --impl b200)")
+    args = parser.parse_args()
+    if args.steps < 1:
+        parser.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        parser.error("--dump-outputs records the outputs of the device path (--impl b200)")
+    return args
+
+
+DUMP_SAMPLES = 1 << 19  # rays per C2 output (12 MiB in all); a render frame keeps half as many pixels (RGBA, 4 MiB): 28 MiB for the default run
+
+
+def dump_sample(count, limit):
+    """A fixed, seeded choice of `limit` of `count` indices, ascending (every index when there are no more than `limit`)."""
+    if count <= limit:
+        return np.arange(count)
+    return np.sort(np.argsort(scenes.uniform(5, np.arange(count, dtype=np.uint64)), kind="stable")[:limit])
+
+
+def dump_outputs(directory, arrays):
+    os.makedirs(directory, exist_ok=True)
+    for name, array in arrays.items():
+        assert array.dtype in (np.float32, np.float64) and np.isfinite(array).all(), name
+        np.save(os.path.join(directory, f"{name}.npy"), array)
 
 
 def peaks():
@@ -548,6 +578,14 @@ def run_trace(ctx, args):
         clocks.mark(1)
         total_ms = ctx.max_over_ranks(start.elapsed_time(stop))
 
+    if args.dump_outputs and ctx.rank == 0:
+        keep = torch.from_numpy(dump_sample(n, DUMP_SAMPLES)).to(device)
+        hits = d_hits.view(n, 16)[keep].cpu().numpy().view(structs.HIT).reshape(-1)
+        # a miss returns the ray's limit, +inf for these rays; the token already marks it, so its distance is stored as -1 (no hit has that)
+        distance = np.where(hits["token"] == structs.TOKEN_EMPTY, np.float32(-1.0), hits["distance"])
+        dump_outputs(args.dump_outputs, {"trace_token": hits["token"].astype(np.float64), "trace_distance": distance, "trace_uv": hits["uv"],
+                                         "occluded": d_occluded[keep].cpu().numpy().astype(np.float32)})
+
     trace_ms = float(np.mean([a.elapsed_time(b) for a, b, _ in events]))
     occlude_ms = float(np.mean([b.elapsed_time(c) for _, b, c in events]))
     value = ctx.world * 2 * n * args.steps / (total_ms * 1e-3) / MRAYS
@@ -724,7 +762,7 @@ def run_render(ctx, args, scene_key, width, height, spp, bounce_limit, steps, wa
             render_ms.append((time.perf_counter() - begin) * 1e3)
             launches += int(stats["kernelLaunches"][0])
             samples += int(stats["sampleEvaluated"][0])
-        if (index + 1) % reduce_every == 0:
+        if (index + 1) % reduce_every == 0 or index + 1 == steps:  # the last step finishes its render
             first, middle, last = (torch.cuda.Event(enable_timing=True) for _ in range(3))
             first.record()
             if ctx.distributed:
@@ -734,7 +772,8 @@ def run_render(ctx, args, scene_key, width, height, spp, bounce_limit, steps, wa
                 dist.all_reduce(frame)  # the accumulation-buffer reduce over NVLink (tile sharding: disjoint pixels, sum with zeros)
             last.record()
             scene.frame_resolve_device(frame.data_ptr(), width, height, stream)
-            frame.zero_()  # the next render starts from an empty accumulation frame
+            if index + 1 < steps:
+                frame.zero_()  # the next render starts from an empty accumulation frame; the last one stays for --dump-outputs
             if timed:
                 reduce_events.append((first, middle, last))
                 launches += 2
@@ -757,6 +796,10 @@ def run_render(ctx, args, scene_key, width, height, spp, bounce_limit, steps, wa
         ctx.barrier()
         clocks.mark(1)
         total_ms = ctx.max_over_ranks(start.elapsed_time(stop))
+
+    if args.dump_outputs and rank == 0:
+        keep = torch.from_numpy(dump_sample(width * height, DUMP_SAMPLES // 2)).to(device)
+        dump_outputs(args.dump_outputs, {f"frame_{scene_key}": frame.view(-1, 4)[keep].cpu().numpy()})
 
     reduce_ms = [b.elapsed_time(c) for _, b, c in reduce_events]
     skew_ms = [a.elapsed_time(b) for a, b, _ in reduce_events]
@@ -842,8 +885,7 @@ def main():
         line = run_trace(ctx, args)
 
         if args.workload == "all" and not args.no_render and not args.instanced:
-            steps = max(1, min(args.render_steps, args.steps))
-            c5_steps = max(4, steps - steps % 4)  # whole 1024-spp renders: one all-reduce per four 256-spp epochs
+            steps = args.steps if args.render_steps is None else max(1, min(args.render_steps, args.steps))
             line["render"] = {"what": "the path tracer measured as the reference reports it (samples/s, ScheduledRender.cs:226-234); records have the shape of a bench line"}
             # ECHO_BENCH_SHRINK=1 (tests/test_gpu_bench.py only): the same code path on scenes and frames that take seconds
             shrink = os.environ.get("ECHO_BENCH_SHRINK") == "1"
@@ -854,8 +896,7 @@ def main():
             c5 = ("c5", "large", 384, 208, 16, 128, 4, lambda: scenes.large_scene(160, 80)) if shrink else ("c5", "large", 3840, 2160, 256, 128, 4, None)
             records = [c1, c3, c4, c5] if ctx.world == 1 else [c5]  # C1, C3 and C4 are one-GPU configurations (BASELINE.json); C5 is the sharded one
             for key, scene_key, width, height, spp, bounce_limit, reduce_every, builder in records:
-                record_steps = c5_steps if reduce_every == 4 else steps
-                line["render"][key] = run_render(ctx, args, scene_key, width, height, spp, bounce_limit, record_steps, args.render_warmup, reduce_every, builder=builder)
+                line["render"][key] = run_render(ctx, args, scene_key, width, height, spp, bounce_limit, steps, args.render_warmup, reduce_every, builder=builder)
             line["gpu_launches"] += sum(record["gpu_launches"] for key, record in line["render"].items() if isinstance(record, dict))
 
     if ctx.rank == 0:

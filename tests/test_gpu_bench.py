@@ -79,12 +79,14 @@ def test_render_bench_line():
     assert line["stats_last_step"]["Sample/Evaluated"] == 256 * 256 * 4
 
 
-def test_default_line_carries_the_render_records(monkeypatch):
-    """`python bench.py` (what the driver runs): the C2 headline plus `render.c1 / c3 / c4 / c5` with roofline, cpu_baseline and the
-    plugin-call e2e. Shrunk through the environment so that the whole default path runs in seconds."""
+def test_default_line_carries_the_render_records(tmp_path):
+    """`python bench.py` (the default run): the C2 headline plus `render.c1 / c3 / c4 / c5` with roofline, cpu_baseline and the
+    plugin-call e2e, every record timed over --steps steps, and --dump-outputs writing the last step's outputs. Shrunk through the
+    environment so that the whole default path runs in seconds."""
     environment = {**os.environ, "ECHO_BENCH_SHRINK": "1"}
-    result = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "4", "--quads", "128", "64", "--rays", str(1 << 18), "--cpu-sample", "65536", "--no-secondary"],
-                            capture_output=True, text=True, timeout=1200, env=environment)
+    outputs = tmp_path / "outputs"
+    result = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "6", "--quads", "128", "64", "--rays", str(1 << 18), "--cpu-sample", "65536", "--no-secondary",
+                             "--dump-outputs", str(outputs)], capture_output=True, text=True, timeout=1200, env=environment)
     assert result.returncode == 0, result.stderr[-2000:]
     lines = [line for line in result.stdout.splitlines() if line.strip()]
     assert len(lines) == 1
@@ -94,5 +96,21 @@ def test_default_line_carries_the_render_records(monkeypatch):
     for key in ("c1", "c3", "c4", "c5"):
         record = line["render"][key]
         check_render_record(record, record["config"]["width"], record["config"]["height"], record["config"]["spp_per_step"])
-    assert line["render"]["c5"]["steps"] % 4 == 0 and "all-reduce every 4" in line["render"]["c5"]["config"]["parallelism"]
+    assert "all-reduce every 4" in line["render"]["c5"]["config"]["parallelism"] and line["render"]["c5"]["all_reduce"]["count"] == 2  # after step 4 and the last
     assert line["gpu_launches"] > 2 * line["steps"]
+    assert all(line["render"][key]["steps"] == line["steps"] == 6 for key in ("c1", "c3", "c4", "c5"))
+
+    import numpy as np
+    from echorenderer_b200 import structs
+    dumped = {path.stem: np.load(path) for path in outputs.iterdir()}
+    assert set(dumped) == {"trace_token", "trace_distance", "trace_uv", "occluded", "frame_cornell", "frame_mixed", "frame_lights", "frame_large"}
+    assert all(array.dtype in (np.float32, np.float64) and np.isfinite(array).all() for array in dumped.values()) and sum(array.nbytes for array in dumped.values()) <= 64 << 20
+    rays = 1 << 18  # fewer than the sample size: every ray is kept, in order
+    assert dumped["trace_token"].shape == dumped["trace_distance"].shape == dumped["occluded"].shape == (rays,) and dumped["trace_uv"].shape == (rays, 2)
+    assert set(np.unique(dumped["occluded"])) <= {0.0, 1.0} and 0 < (dumped["trace_token"] != structs.TOKEN_EMPTY).sum() < rays
+    miss = dumped["trace_token"] == structs.TOKEN_EMPTY
+    assert (dumped["trace_distance"][miss] == -1).all() and (dumped["trace_distance"][~miss] >= 0).all()
+    for key in ("c1", "c3", "c4", "c5"):
+        config = line["render"][key]["config"]
+        frame = dumped["frame_" + {"c1": "cornell", "c3": "mixed", "c4": "lights", "c5": "large"}[key]]
+        assert frame.shape == (min(config["width"] * config["height"], 1 << 18), 4) and np.isfinite(frame).all() and frame[:, :3].max() > 0, key
