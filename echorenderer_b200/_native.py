@@ -34,7 +34,7 @@ EXPORTS = [
     "echo_b200_trace_batch_device_counted", "echo_b200_occlude_batch_device_counted", "echo_b200_debug_bxdf_batch", "echo_b200_debug_math",
     "echo_b200_debug_evaluate_samples",
     "echo_b200_host_alloc", "echo_b200_host_free", "echo_b200_host_register", "echo_b200_host_unregister", "echo_b200_debug_set_option", "echo_b200_debug_measure_peaks", "echo_b200_debug_last_build", "echo_b200_debug_last_light_build", "echo_b200_build_light_tree", "echo_b200_scene_build_light_tree",
-    "echo_b200_scene_create_multi", "echo_b200_scene_gpu_count",
+    "echo_b200_scene_create_multi", "echo_b200_scene_gpu_count", "echo_b200_build_packs", "echo_b200_scene_build_packs", "echo_b200_debug_last_pack_build",
 ]
 
 
@@ -95,6 +95,10 @@ def library():
         "echo_b200_scene_build_light_tree": [p, p, u32, ctypes.POINTER(u32), ctypes.POINTER(u32), ctypes.POINTER(f32)],
         "echo_b200_scene_create_multi": [ctypes.POINTER(p), u64],
         "echo_b200_scene_gpu_count": [p, ctypes.POINTER(i32)],
+        "echo_b200_build_packs": [i32, p, u32, p, u32, p, u32, p, u32, p, u32, p, u32, p, u32, ctypes.POINTER(u32), p, u32, ctypes.POINTER(u32), p, p, u32,
+                                  ctypes.POINTER(u32), ctypes.POINTER(f32)],
+        "echo_b200_scene_build_packs": [p, p, u32, ctypes.POINTER(u32), ctypes.POINTER(u32), ctypes.POINTER(u32), ctypes.POINTER(f32)],
+        "echo_b200_debug_last_pack_build": [p],
     }
 
     for name, argtypes in signatures.items():
@@ -184,6 +188,15 @@ def last_light_build():
     out = np.zeros(4, dtype=np.float32)
     check(library().echo_b200_debug_last_light_build(pointer(out)))
     return {"upload_ms": float(out[0]), "device_build_ms": float(out[1]), "download_ms": float(out[2]), "levels": int(out[3])}
+
+
+def last_pack_build():
+    """echo_b200_debug_last_pack_build: rounds, levels and read-backs of this thread's last build of every pack (echo_b200_build_packs)."""
+    import numpy as np
+    out = np.zeros(8, dtype=np.float32)
+    check(library().echo_b200_debug_last_pack_build(pointer(out)))
+    return {"rounds": int(out[0]), "qbvh_levels": int(out[1]), "light_levels": int(out[2]), "read_backs": int(out[3]), "launches": int(out[4]),
+            "build_ms": float(out[5]), "rebuilt_packs": int(out[6])}
 
 
 def host_register(array):

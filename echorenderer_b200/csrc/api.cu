@@ -11,6 +11,7 @@
 #include "../../include/echo_b200_debug.h"
 #include "echo_internal.h"
 #include "echo_light_build.h"
+#include "echo_pack_build.h"
 
 namespace echo
 {
@@ -655,6 +656,67 @@ int32_t echo_b200_scene_build_light_tree(EchoScene* scene, const EchoPointLight*
 	scene->lightNodes.swap(nodes);
 	scene->emitterTokens.swap(tokens);
 	scene->emitterPaths.swap(paths);
+	scene->pointLights.assign(points, points + pointCount);
+	scene->committed = false;
+	return ECHO_B200_OK;
+}
+
+int32_t echo_b200_build_packs(int32_t device, const EchoTriangle* triangles, uint32_t triangleCount, const EchoSphere* spheres, uint32_t sphereCount,
+                              const EchoMaterial* materials, uint32_t materialCount, const EchoPointLight* points, uint32_t pointCount,
+                              EchoPack* packs, uint32_t packCount, const EchoInstance* instances, uint32_t instanceCount,
+                              EchoQbvhNode* outNodes, uint32_t nodeCapacity, uint32_t* outNodeCount,
+                              EchoLightNode* outLightNodes, uint32_t lightNodeCapacity, uint32_t* outLightNodeCount,
+                              uint32_t* outTokens, uint64_t* outPaths, uint32_t emitterCapacity, uint32_t* outEmitterCount, float* outPower)
+{
+	if ((!triangles && triangleCount) || (!spheres && sphereCount) || (!materials && materialCount) || (!points && pointCount) || !packs || (!instances && instanceCount)
+		|| (!outNodes && nodeCapacity) || (!outLightNodes && lightNodeCapacity) || ((!outTokens || !outPaths) && emitterCapacity)
+		|| !outNodeCount || !outLightNodeCount || !outEmitterCount || !outPower) return fail(ECHO_B200_ERR_INVALID, "null argument");
+	int32_t count = 0;
+	int32_t status = echo_b200_device_count(&count);
+	if (status != ECHO_B200_OK) return status;
+	if (device < 0 || device >= count) return fail(ECHO_B200_ERR_INVALID, "device index out of range");
+	DeviceGuard guard(device);
+	if (!guard.ok) return ECHO_B200_ERR_NO_DEVICE;
+
+	const packbuild::Inputs inputs = { triangles, triangleCount, spheres, sphereCount, materials, materialCount, points, pointCount, packs, packCount, instances, instanceCount };
+	packbuild::Output output;
+	status = build_packs_device(inputs, output);
+	if (status != ECHO_B200_OK) return status;
+
+	std::string message;
+	status = packbuild::deliver(output, packs, outNodes, nodeCapacity, outNodeCount, outLightNodes, lightNodeCapacity, outLightNodeCount, outTokens, outPaths, emitterCapacity,
+	                            outEmitterCount, outPower, message);
+	return status == ECHO_B200_OK ? status : fail(status, message.c_str());
+}
+
+int32_t echo_b200_scene_build_packs(EchoScene* scene, const EchoPointLight* points, uint32_t pointCount, uint32_t* outNodeCount, uint32_t* outLightNodeCount,
+                                    uint32_t* outEmitterCount, float* outPower)
+{
+	if (!scene || (!points && pointCount)) return fail(ECHO_B200_ERR_INVALID, "null argument");
+	if (scene->packs.empty()) return fail(ECHO_B200_ERR_INVALID, "scene_build_packs builds the packs declared with set_packs; a scene without packs uses scene_build_qbvh / scene_build_light_tree");
+	DeviceGuard guard(scene->device); // a multi-device handle builds on its first device; commit replicates the staging
+	if (!guard.ok) return ECHO_B200_ERR_NO_DEVICE;
+
+	const packbuild::Inputs inputs = { scene->triangles.data(), (uint32_t)scene->triangles.size(), scene->spheres.data(), (uint32_t)scene->spheres.size(),
+	                                   scene->materials.data(), (uint32_t)scene->materials.size(), points, pointCount, scene->packs.data(), (uint32_t)scene->packs.size(),
+	                                   scene->instances.data(), (uint32_t)scene->instances.size() };
+	packbuild::Output output;
+	int32_t status = build_packs_device(inputs, output);
+	if (status != ECHO_B200_OK) return status;
+
+	uint32_t maxDepth = 0;
+	for (const EchoPack& pack : output.packs) maxDepth = std::max(maxDepth, pack.maxDepth);
+	if (outNodeCount) *outNodeCount = (uint32_t)output.nodes.size();
+	if (outLightNodeCount) *outLightNodeCount = (uint32_t)output.lightNodes.size();
+	if (outEmitterCount) *outEmitterCount = (uint32_t)output.emitterTokens.size();
+	if (outPower) *outPower = output.power;
+
+	scene->nodes.swap(output.nodes);
+	scene->maxDepth = maxDepth;
+	scene->packs.swap(output.packs);
+	scene->lightNodes.swap(output.lightNodes);
+	scene->emitterTokens.swap(output.emitterTokens);
+	scene->emitterPaths.swap(output.emitterPaths);
 	scene->pointLights.assign(points, points + pointCount);
 	scene->committed = false;
 	return ECHO_B200_OK;
@@ -1314,6 +1376,13 @@ int32_t echo_b200_debug_last_light_build(float* out4)
 {
 	if (!out4) return fail(ECHO_B200_ERR_INVALID, "out4 is null");
 	last_light_build(out4);
+	return ECHO_B200_OK;
+}
+
+int32_t echo_b200_debug_last_pack_build(float* out8)
+{
+	if (!out8) return fail(ECHO_B200_ERR_INVALID, "out8 is null");
+	last_pack_build(out8);
 	return ECHO_B200_OK;
 }
 

@@ -50,6 +50,12 @@ namespace lightbuild { struct Sources; }
 bool build_light_tree_device(const lightbuild::Sources& sources, std::vector<EchoLightNode>& nodes, std::vector<uint32_t>& tokens, std::vector<uint64_t>& paths, bool* refused);
 void last_light_build(float* out4); // the calling thread's last build_light_tree_device: {upload, device build, download} ms, levels
 
+// ---- packbuild.cu: every pack of an instanced scene, QBVH and light tree, in rounds of forests (echo_pack_build.h). Host memory in and
+// out; returns an ECHO_B200_* status with the error set ----
+namespace packbuild { struct Inputs; struct Output; }
+int32_t build_packs_device(const packbuild::Inputs& inputs, packbuild::Output& output);
+void last_pack_build(float* out8); // the calling thread's last build_packs_device: rounds, levels, read-backs, launches, ms
+
 // ---- render.cu ----
 struct RenderState; // wavefront buffers, owned per scene
 

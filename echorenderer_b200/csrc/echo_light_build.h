@@ -570,22 +570,81 @@ LIGHT_HD bool emitter(const Sources& s, uint32_t c, Bound& bound, uint32_t& toke
 
 // ---- passes ----
 
-struct FlagPass // 1 where candidate c is an emitter
+// ---- a FOREST: the light trees of several packs in one run (the single-pack build is the forest of one tree) ----
+
+struct LightPack // one tree: the pack's ranges of the shared arrays, and where its candidates, emitters and nodes start
 {
-	Sources sources;
+	uint32_t triangleOffset, triangleCount, sphereOffset, sphereCount, instanceOffset, instanceCount;
+	uint32_t materialOffset, materialCount; // the pack's own swatch (LightCollection.cs:145,151)
+	uint32_t pointOffset, pointCount;
+	uint32_t candidateBase;                 // candidates lie pack by pack, each pack's in LightCollection.CreateBounds order
+	uint32_t emitterBase, emitterCount;     // filled by the driver once the emitters are counted
+	uint32_t nodeBase;                      // 2 emitterCount - 1 nodes from here
+	uint32_t rootSegment;                   // the pack's root segment, kNone for a pack of one emitter (a leaf) or none
+	uint32_t pad;
+};
+
+LIGHT_HD uint32_t candidate_count(const LightPack& pack) { return pack.pointCount + pack.triangleCount + pack.sphereCount + pack.instanceCount; }
+
+LIGHT_HD uint32_t light_pack_of(const LightPack* packs, uint32_t packCount, uint32_t candidate) // the last pack whose candidates begin at or before
+{
+	uint32_t low = 0u, high = packCount;
+	while (high - low > 1u)
+	{
+		uint32_t middle = (low + high) / 2u;
+		if (packs[middle].candidateBase <= candidate) low = middle;
+		else high = middle;
+	}
+	return low;
+}
+
+struct Forest // the shared arrays (backend memory) and the packs
+{
+	const EchoTriangle* triangles;
+	const EchoSphere* spheres;
+	const EchoMaterial* materials;
+	const EchoPointLight* points;
+	const float* instanceLights; // 12 floats per placement
+	const LightPack* packs;
+	uint32_t packCount;
+
+	LIGHT_HD Sources view(uint32_t p) const // what pack p's own LightCollection sees: its arrays from index 0, tokens relative to them
+	{
+		const LightPack& pack = packs[p];
+		return { triangles + pack.triangleOffset, pack.triangleCount, spheres + pack.sphereOffset, pack.sphereCount, materials + pack.materialOffset, pack.materialCount,
+		         points + pack.pointOffset, pack.pointCount, instanceLights + (size_t)pack.instanceOffset * 12, pack.instanceCount };
+	}
+};
+
+struct FlagPass // 1 where candidate c is an emitter (c == the candidate count: 0, the end of the sum)
+{
+	Forest forest;
+	uint32_t candidates;
 	uint32_t* flags;
 
 	LIGHT_HD void operator()(uint32_t c) const
 	{
 		Bound bound;
 		uint32_t token;
-		flags[c] = c < sources.candidates() && emitter(sources, c, bound, token) ? 1u : 0u;
+		if (c >= candidates) { flags[c] = 0u; return; }
+		uint32_t p = light_pack_of(forest.packs, forest.packCount, c);
+		flags[c] = emitter(forest.view(p), c - forest.packs[p].candidateBase, bound, token) ? 1u : 0u;
 	}
 };
 
-struct EmitterPass // emitter k = the k-th flagged candidate; position k starts as emitter k
+struct PackEmittersPass // the first emitter of every pack (and the total after the last): the exclusive sum at the pack's first candidate
 {
-	Sources sources;
+	const LightPack* packs;
+	uint32_t packCount, candidates;
+	const uint32_t* slots;
+	uint32_t* out;
+
+	LIGHT_HD void operator()(uint32_t p) const { out[p] = slots[p < packCount ? packs[p].candidateBase : candidates]; }
+};
+
+struct EmitterPass // emitter k = the k-th flagged candidate; position k starts as emitter k, in the root segment of its pack
+{
+	Forest forest;
 	const uint32_t* slots; // exclusive sum of the flags
 	Bound* bounds;
 	uint32_t* tokens;
@@ -596,13 +655,14 @@ struct EmitterPass // emitter k = the k-th flagged candidate; position k starts 
 	{
 		Bound bound;
 		uint32_t token;
-		if (!emitter(sources, c, bound, token)) return;
+		uint32_t p = light_pack_of(forest.packs, forest.packCount, c);
+		if (!emitter(forest.view(p), c - forest.packs[p].candidateBase, bound, token)) return;
 
 		uint32_t k = slots[c];
 		bounds[k] = bound;
 		tokens[k] = token;
 		order[k] = k;
-		segmentOf[k] = 0u;
+		segmentOf[k] = forest.packs[p].rootSegment;
 	}
 };
 
@@ -633,27 +693,25 @@ LIGHT_HD Segment new_segment(uint32_t begin, uint32_t length, uint32_t node, uin
 	return segment;
 }
 
-struct RootPass // the whole emitter list as one segment — or as one leaf
+struct RootPass // every pack's emitter list as one segment — or as one leaf, or nothing
 {
-	uint32_t count;
+	const LightPack* packs;
 	const Bound* bounds;
 	const uint32_t* tokens;
 	Segment* segments;
 	uint32_t* internalNodes;
-	uint32_t* segmentOf;
 	LeafWriter leaves;
 
-	LIGHT_HD void operator()(uint32_t) const
+	LIGHT_HD void operator()(uint32_t p) const
 	{
-		if (count == 1u)
-		{
-			leaves(0u, bounds[0], tokens[0], 0ull);
-			segmentOf[0] = kNone;
-			return;
-		}
+		const LightPack& pack = packs[p];
 
-		segments[0] = new_segment(0u, count, 0u, 0u, 0ull);
-		internalNodes[0] = 0u;
+		if (pack.emitterCount == 1u) leaves(pack.nodeBase, bounds[pack.emitterBase], tokens[pack.emitterBase], 0ull);
+		else if (pack.emitterCount > 1u)
+		{
+			segments[pack.rootSegment] = new_segment(pack.emitterBase, pack.emitterCount, pack.nodeBase, 0u, 0ull);
+			internalNodes[pack.rootSegment] = pack.nodeBase;
+		}
 	}
 };
 
@@ -881,6 +939,28 @@ struct BranchPass // LightTree.Node's branch constructor (:160-165): child0.boun
 	}
 };
 
+struct RebasePass // child indices relative to the pack's first node, as every pack's own LightTree numbers them
+{
+	const LightPack* packs;
+	uint32_t packCount;
+	const uint32_t* isLeaf;
+	EchoLightNode* nodes;
+
+	LIGHT_HD void operator()(uint32_t node) const
+	{
+		if (isLeaf[node]) return;
+		uint32_t low = 0u, high = packCount; // the last pack whose nodes begin at or before this one (a pack without nodes shares its base with the next)
+		while (high - low > 1u)
+		{
+			uint32_t middle = (low + high) / 2u;
+			if (packs[middle].nodeBase <= node) low = middle;
+			else high = middle;
+		}
+		nodes[node].child0 -= packs[low].nodeBase;
+		nodes[node].child1 -= packs[low].nodeBase;
+	}
+};
+
 struct MapPass // LightTree.AddToMap (:26-37): the leaves in pre-order
 {
 	const EchoLightNode* nodes;
@@ -917,8 +997,9 @@ struct Arena
 struct Result
 {
 	bool ok = false;          // false: a backend call failed
-	bool unsupported = false; // the tree is deeper than a 64-bit path (LightTree.cs:29)
-	uint32_t emitterCount = 0, nodeCount = 0, levels = 0;
+	bool unsupported = false; // some tree is deeper than a 64-bit path (LightTree.cs:29)
+	uint32_t emitterCount = 0, nodeCount = 0, levels = 0; // all packs
+	std::vector<LightPack> packs; // per pack: emitterBase / emitterCount, nodeBase (2 emitterCount - 1 nodes, or none)
 	// backend memory, valid until the backend goes away
 	EchoLightNode* nodes = nullptr;
 	uint32_t* emitterTokens = nullptr;
@@ -968,29 +1049,75 @@ struct Working // everything sized by the emitter count
 	}
 };
 
-// `sources` points into memory the backend's passes can read (device memory for the CUDA backend).
+// host -> backend: the backend's write(); a backend without one keeps its memory in the host's address space (the sequential CPU backends)
+template<class Backend, class T>
+auto write_to(Backend& backend, T* destination, const T* source, uint32_t n, int) -> decltype(backend.write(destination, source, n))
+{
+	return backend.write(destination, source, n);
+}
+
+template<class Backend, class T>
+bool write_to(Backend&, T* destination, const T* source, uint32_t n, long)
+{
+	memcpy((void*)destination, (const void*)source, sizeof(T) * n);
+	return true;
+}
+
+// Backend concept: allocate, for_each, sort_pairs, exclusive_sum, read, fill_zero as echo_sweep.h describes them; write where the
+// backend's memory is not the host's.
+//
+// The light trees of `packCount` packs in one run: every pack's root is one more segment of the first level, so each level serves all
+// packs and the run reads back as many levels as its deepest tree has. `forest` points into backend memory except `packs`, which is
+// host memory (its ranges and materials; the driver fills in the rest): candidates, emitters and nodes lie pack by pack, and every
+// pack's nodes, emitter tokens and bit paths are what its own single-pack build emits (child indices relative to the pack's first node).
 template<class Backend>
-Result build(Backend& backend, const Sources& sources)
+Result build_forest(Backend& backend, const Forest& forest)
 {
 	Result result;
-	const uint32_t candidates = sources.candidates();
+	const uint32_t packCount = forest.packCount;
+	result.packs.assign(forest.packs, forest.packs + packCount);
+	uint32_t candidates = 0u;
+	for (LightPack& pack : result.packs) { pack.candidateBase = candidates; candidates += candidate_count(pack); pack.emitterBase = pack.emitterCount = pack.nodeBase = 0u; pack.rootSegment = kNone; }
 	if (candidates == 0u) { result.ok = true; return result; }
 
 	// the emitters: flag, rank, scatter
 	Arena first;
 	first.take<uint32_t>(candidates + 1);
 	first.take<uint32_t>(candidates + 1);
+	first.take<LightPack>(packCount);
+	first.take<uint32_t>(packCount + 1);
 	first.base = backend.allocate(first.used + 256);
 	if (!first.base) return result;
 	first.used = 0;
 	uint32_t* flags = first.take<uint32_t>(candidates + 1);
 	uint32_t* emitterSlots = first.take<uint32_t>(candidates + 1);
+	LightPack* packs = first.take<LightPack>(packCount);
+	uint32_t* bases = first.take<uint32_t>(packCount + 1);
 
-	uint32_t count = 0u;
-	if (!backend.for_each(candidates + 1u, FlagPass{ sources, flags })) return result;
+	Forest device = forest;
+	device.packs = packs;
+	if (!write_to(backend, packs, result.packs.data(), packCount, 0)) return result;
+
+	std::vector<uint32_t> emitterBases(packCount + 1);
+	if (!backend.for_each(candidates + 1u, FlagPass{ device, candidates, flags })) return result;
 	if (!backend.exclusive_sum(flags, emitterSlots, candidates + 1u)) return result;
-	if (!backend.read(emitterSlots + candidates, &count, 1u)) return result;
+	if (!backend.for_each(packCount + 1u, PackEmittersPass{ packs, packCount, candidates, emitterSlots, bases })) return result;
+	if (!backend.read(bases, emitterBases.data(), packCount + 1u)) return result;
+	const uint32_t count = emitterBases[packCount];
 	if (count == 0u) { result.ok = true; return result; }
+
+	// every pack's emitters, nodes and root segment
+	uint32_t nodeCount = 0u, live = 0u;
+	for (uint32_t p = 0; p < packCount; p++)
+	{
+		LightPack& pack = result.packs[p];
+		pack.emitterBase = emitterBases[p];
+		pack.emitterCount = emitterBases[p + 1u] - emitterBases[p];
+		pack.nodeBase = nodeCount;
+		if (pack.emitterCount != 0u) nodeCount += 2u * pack.emitterCount - 1u;
+		if (pack.emitterCount > 1u) pack.rootSegment = live++;
+	}
+	if (!write_to(backend, packs, result.packs.data(), packCount, 0)) return result;
 
 	Working w;
 	Arena arena;
@@ -1000,15 +1127,13 @@ Result build(Backend& backend, const Sources& sources)
 	arena.used = 0;
 	w.carve(arena, count);
 
-	const uint32_t nodeCount = 2u * count - 1u;
 	if (!backend.fill_zero(w.nodes, sizeof(EchoLightNode) * nodeCount) || !backend.fill_zero(w.isLeaf, sizeof(uint32_t) * (nodeCount + 1u))) return result;
-	if (!backend.for_each(candidates, EmitterPass{ sources, emitterSlots, w.bounds, w.tokens, w.order[0], w.segmentOf })) return result;
+	if (!backend.for_each(candidates, EmitterPass{ device, emitterSlots, w.bounds, w.tokens, w.order[0], w.segmentOf })) return result;
 
 	LeafWriter leaves{ w.nodes, w.isLeaf, w.pathOfNode };
-	if (!backend.for_each(1u, RootPass{ count, w.bounds, w.tokens, w.segments[0], w.internalNodes, w.segmentOf, leaves })) return result;
+	if (!backend.for_each(packCount, RootPass{ packs, w.bounds, w.tokens, w.segments[0], w.internalNodes, leaves })) return result;
 
 	std::vector<uint32_t> levelOffsets{ 0u }; // into internalNodes, one entry per depth + the end
-	uint32_t live = count > 1u ? 1u : 0u;
 	int side = 0;
 
 	while (live != 0u)
@@ -1045,6 +1170,7 @@ Result build(Backend& backend, const Sources& sources)
 
 	if (!backend.exclusive_sum(w.isLeaf, w.leafSlots, nodeCount + 1u)) return result;
 	if (!backend.for_each(nodeCount, MapPass{ w.nodes, w.isLeaf, w.leafSlots, w.pathOfNode, w.emitterTokens, w.emitterPaths })) return result;
+	if (packCount > 1u && !backend.for_each(nodeCount, RebasePass{ packs, packCount, w.isLeaf, w.nodes })) return result;
 
 	result.ok = true;
 	result.emitterCount = count;
@@ -1053,6 +1179,20 @@ Result build(Backend& backend, const Sources& sources)
 	result.emitterTokens = w.emitterTokens;
 	result.emitterPaths = w.emitterPaths;
 	return result;
+}
+
+// one pack: LightCollection.CreateBounds + LightTree.Build of `sources` (backend memory)
+template<class Backend>
+Result build(Backend& backend, const Sources& sources)
+{
+	LightPack pack = {};
+	pack.triangleCount = sources.triangleCount;
+	pack.sphereCount = sources.sphereCount;
+	pack.instanceCount = sources.instanceCount;
+	pack.materialCount = sources.materialCount;
+	pack.pointCount = sources.pointCount;
+	const Forest forest = { sources.triangles, sources.spheres, sources.materials, sources.points, sources.instanceLights, &pack, 1u };
+	return build_forest(backend, forest);
 }
 
 } // namespace lightbuild

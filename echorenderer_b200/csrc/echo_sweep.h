@@ -205,13 +205,35 @@ SWEEP_HD void atomic_or_u32(uint32_t* address, uint32_t value)
 
 // ---- passes ----
 
-struct BoundsPass // GeometryCollection.CreateBounds (GeometryCollection.cs:52-81): triangles, spheres, then instances; position i starts as primitive i
+struct PackRange // one tree of a forest: the pack's primitives (offsets into the shared arrays) and its first position
 {
+	uint32_t triangleOffset, triangleCount, sphereOffset, sphereCount, instanceOffset, instanceCount;
+	uint32_t begin; // positions [begin, begin + triangleCount + sphereCount + instanceCount) of the build
+};
+
+SWEEP_HD uint32_t range_size(const PackRange& pack) { return pack.triangleCount + pack.sphereCount + pack.instanceCount; }
+
+SWEEP_HD uint32_t pack_of(const PackRange* packs, uint32_t packCount, uint32_t position) // the last pack that begins at or before `position`
+{
+	uint32_t low = 0u, high = packCount;
+	while (high - low > 1u)
+	{
+		uint32_t middle = (low + high) / 2u;
+		if (packs[middle].begin <= position) low = middle;
+		else high = middle;
+	}
+	return low;
+}
+
+// GeometryCollection.CreateBounds (GeometryCollection.cs:52-81) of every pack: triangles, spheres, then instances, tokens relative to the
+// pack's own arrays; position i starts as primitive i, in the segment of its pack (segment p = the root of pack p)
+struct BoundsPass
+{
+	const PackRange* packs;
+	uint32_t packCount;
 	const EchoTriangle* triangles;
-	uint32_t triangleCount;
 	const EchoSphere* spheres;
-	uint32_t sphereCount;
-	const float* instanceBounds; // PreparedInstance.BoxBound of the pack's placements: min xyz, max xyz
+	const float* instanceBounds; // PreparedInstance.BoxBound of the placements: min xyz, max xyz
 	Box* boxes;
 	uint32_t* tokens;
 	uint32_t* perm;
@@ -219,35 +241,61 @@ struct BoundsPass // GeometryCollection.CreateBounds (GeometryCollection.cs:52-8
 
 	SWEEP_HD void operator()(uint32_t i) const
 	{
+		uint32_t p = pack_of(packs, packCount, i);
+		const PackRange pack = packs[p];
+		uint32_t local = i - pack.begin;
 		Box box;
 
-		if (i < triangleCount) // PreparedTriangle.BoxBound, TriangleEntity.cs:142 (Float4 min / max = Sse.Min / Max)
+		if (local < pack.triangleCount) // PreparedTriangle.BoxBound, TriangleEntity.cs:142 (Float4 min / max = Sse.Min / Max)
 		{
-			const EchoTriangle& t = triangles[i];
+			const EchoTriangle& t = triangles[pack.triangleOffset + local];
 			for (int k = 0; k < 3; k++)
 			{
 				float v0 = t.vertex0[k], v1 = f_add(v0, t.edge1[k]), v2 = f_add(v0, t.edge2[k]);
 				box.lo[k] = select_min(select_min(v0, v1), v2);
 				box.hi[k] = select_max(select_max(v0, v1), v2);
 			}
-			tokens[i] = ECHO_TOKEN_MAKE(ECHO_TOKEN_TYPE_TRIANGLE, i);
+			tokens[i] = ECHO_TOKEN_MAKE(ECHO_TOKEN_TYPE_TRIANGLE, local);
 		}
-		else if (i >= triangleCount + sphereCount)
+		else if (local >= pack.triangleCount + pack.sphereCount)
 		{
-			const float* bound = instanceBounds + (size_t)(i - triangleCount - sphereCount) * 6;
+			uint32_t instance = local - pack.triangleCount - pack.sphereCount;
+			const float* bound = instanceBounds + (size_t)(pack.instanceOffset + instance) * 6;
 			for (int k = 0; k < 3; k++) { box.lo[k] = bound[k]; box.hi[k] = bound[3 + k]; }
-			tokens[i] = ECHO_TOKEN_MAKE(ECHO_TOKEN_TYPE_INSTANCE, i - triangleCount - sphereCount);
+			tokens[i] = ECHO_TOKEN_MAKE(ECHO_TOKEN_TYPE_INSTANCE, instance);
 		}
 		else // PreparedSphere.BoxBound, SphereEntity.cs:66
 		{
-			const EchoSphere& s = spheres[i - triangleCount];
+			const EchoSphere& s = spheres[pack.sphereOffset + local - pack.triangleCount];
 			for (int k = 0; k < 3; k++) { box.lo[k] = f_sub(s.position[k], s.radius); box.hi[k] = f_add(s.position[k], s.radius); }
-			tokens[i] = ECHO_TOKEN_MAKE(ECHO_TOKEN_TYPE_SPHERE, i - triangleCount);
+			tokens[i] = ECHO_TOKEN_MAKE(ECHO_TOKEN_TYPE_SPHERE, local - pack.triangleCount);
 		}
 
 		boxes[i] = box;
 		perm[i] = i;
-		segmentOf[i] = 0u;
+		segmentOf[i] = p;
+	}
+};
+
+struct RootPass // Build, SweepBuilder.cs:24-36, once per pack: the root segment over the pack's positions (binary node p) ...
+{
+	const PackRange* packs;
+	Segment* segments;
+
+	SWEEP_HD void operator()(uint32_t p) const { segments[p] = { packs[p].begin, range_size(packs[p]), p, 0u }; }
+};
+
+struct RootAxisPass // ... sorted by the major axis of the bound of everything in the pack: the segmented scan at the segment's end
+{
+	const ScanItem* heads;
+	Segment* segments;
+	unsigned long long* best;
+
+	SWEEP_HD void operator()(uint32_t p) const
+	{
+		Segment segment = segments[p];
+		segments[p].flags = major_axis(to_box(heads[segment.begin + segment.length - 1u])) | kNeedSort;
+		best[p] = kNoCut;
 	}
 };
 
@@ -541,12 +589,26 @@ struct QuadCountPass // quad nodes in the subtree of every internal binary node 
 	}
 };
 
-struct QuadEmitPass // CreateNode, :363-404: pre-order indices for the internal slots, then the node itself
+struct QuadRootPass // the root of pack p is its quad node 0; the packs' nodes follow each other in pack order
+{
+	const uint32_t* rootBase; // exclusive sum of the roots' quad counts
+	uint32_t* quadIndex;
+	uint32_t* quadBase;
+
+	SWEEP_HD void operator()(uint32_t p) const
+	{
+		quadIndex[p] = 0u;
+		quadBase[p] = rootBase[p];
+	}
+};
+
+struct QuadEmitPass // CreateNode, :363-404: pre-order indices (relative to the pack's root) for the internal slots, then the node itself
 {
 	uint32_t first;
 	const BinNode* nodes;
 	const uint32_t* quadCount;
 	uint32_t* quadIndex;
+	uint32_t* quadBase; // where the node's pack starts in `out`
 	EchoQbvhNode* out;
 
 	SWEEP_HD void operator()(uint32_t i) const
@@ -559,7 +621,7 @@ struct QuadEmitPass // CreateNode, :363-404: pre-order indices for the internal 
 		uint32_t axisMinor0 = add_children(nodes, child0, slots);
 		uint32_t axisMinor1 = add_children(nodes, child1, slots + 2);
 
-		uint32_t index = quadIndex[node];
+		uint32_t index = quadIndex[node], base = quadBase[node];
 		uint32_t running = index + 1u;
 
 		EchoQbvhNode quad;
@@ -584,6 +646,7 @@ struct QuadEmitPass // CreateNode, :363-404: pre-order indices for the internal 
 				else
 				{
 					quadIndex[slots[k]] = running;
+					quadBase[slots[k]] = base;
 					token = ECHO_TOKEN_MAKE(ECHO_TOKEN_TYPE_NODE, running);
 					running += quadCount[slots[k]];
 				}
@@ -594,7 +657,7 @@ struct QuadEmitPass // CreateNode, :363-404: pre-order indices for the internal 
 			quad.token4[k] = token;
 		}
 
-		out[index] = quad;
+		out[base + index] = quad;
 	}
 };
 
@@ -652,15 +715,19 @@ struct Arena
 struct Buffers
 {
 	Box* boxes;
-	uint32_t *tokens, *perm[2], *segmentOf[2], *stay, *newPosition, *keep, *newSegment, *totals, *quadCount, *quadDepth, *quadIndex;
+	uint32_t *tokens, *perm[2], *segmentOf[2], *stay, *newPosition, *keep, *newSegment, *totals, *quadCount, *quadDepth, *quadIndex, *quadBase, *rootBase;
 	unsigned long long *keys[2], *best[2];
 	ScanItem *forwards, *backwards, *heads, *tails;
 	Segment *segments[2], *slots;
 	BinNode* nodes;
 	EchoQbvhNode* quads;
 
-	void carve(Arena& arena, uint64_t total)
+	PackRange* packs;
+
+	void carve(Arena& arena, uint64_t total, uint32_t packCount)
 	{
+		packs = arena.take<PackRange>(packCount);
+		rootBase = arena.take<uint32_t>(packCount);
 		boxes = arena.take<Box>(total);
 		tokens = arena.take<uint32_t>(total);
 		for (int k = 0; k < 2; k++)
@@ -685,6 +752,7 @@ struct Buffers
 		quadCount = arena.take<uint32_t>(2 * total);
 		quadDepth = arena.take<uint32_t>(2 * total);
 		quadIndex = arena.take<uint32_t>(2 * total);
+		quadBase = arena.take<uint32_t>(2 * total);
 		quads = arena.take<EchoQbvhNode>(total);
 	}
 };
@@ -692,8 +760,9 @@ struct Buffers
 struct Result
 {
 	bool ok = false;       // false: a backend call failed (its error is set) ...
-	bool gaveUp = false;   // ... or the tree chains deeper than kMaxLevels
-	uint32_t nodeCount = 0, maxDepth = 0, levels = 0;
+	bool gaveUp = false;   // ... or some tree chains deeper than kMaxLevels
+	uint32_t nodeCount = 0, maxDepth = 0, levels = 0; // nodeCount: all packs; maxDepth: pack 0's
+	std::vector<uint32_t> packNodeCount, packMaxDepth, packNodeBase; // per pack: its quad nodes are quads[packNodeBase, + packNodeCount)
 	const EchoQbvhNode* quads = nullptr; // backend memory
 };
 
@@ -706,36 +775,38 @@ struct Result
 //   template<class T> bool read(const T* source, T* destination, uint32_t n)    backend -> host, complete on return
 //   template<class T> bool write(T* destination, const T* source, uint32_t n)   host -> backend
 //   bool fill_zero(void* pointer, size_t bytes)
+//
+// A FOREST: the trees of `packCount` packs in one run. Nothing couples two segments of one level, so each pack is one more root
+// segment; every level of the loop serves all packs at once, and the run reads back as many levels as its deepest tree has. `packs`
+// (host memory) gives each pack's ranges of the shared arrays (backend memory) and its first position; the positions of the packs
+// follow each other without gaps. Every tree is emitted as the single-pack build emits it — tokens and child indices relative to the
+// pack — and the trees lie back to back in `quads`. A single pack is the forest of one tree.
 template<class Backend>
-Result build(Backend& backend, const EchoTriangle* triangles, uint32_t triangleCount, const EchoSphere* spheres, uint32_t sphereCount,
-             const float* instanceBounds, uint32_t instanceCount)
+Result build_forest(Backend& backend, const PackRange* packs, uint32_t packCount, const EchoTriangle* triangles, const EchoSphere* spheres, const float* instanceBounds)
 {
 	Result result;
-	const uint32_t total = triangleCount + sphereCount + instanceCount;
+	if (packCount == 0u) { result.ok = true; return result; }
+	const uint32_t total = packs[packCount - 1u].begin + range_size(packs[packCount - 1u]);
 
 	Buffers b;
 	Arena measure;
-	b.carve(measure, total);
+	b.carve(measure, total, packCount);
 	Arena arena;
 	arena.base = backend.allocate(measure.used);
 	if (!arena.base) return result;
-	b.carve(arena, total);
+	b.carve(arena, total, packCount);
 
-	if (!backend.for_each(total, BoundsPass{ triangles, triangleCount, spheres, sphereCount, instanceBounds, b.boxes, b.tokens, b.perm[0], b.segmentOf[0] })) return result;
+	if (!backend.write(b.packs, packs, packCount)) return result;
+	if (!backend.for_each(total, BoundsPass{ b.packs, packCount, triangles, spheres, instanceBounds, b.boxes, b.tokens, b.perm[0], b.segmentOf[0] })) return result;
 
-	// Build, SweepBuilder.cs:24-36: the root is sorted by the major axis of the bound of everything
-	Segment root = { 0u, total, 0u, 0u };
-	if (!backend.write(b.segments[0], &root, 1)) return result;
+	// Build, SweepBuilder.cs:24-36: each root is sorted by the major axis of the bound of everything in its pack
+	if (!backend.for_each(packCount, RootPass{ b.packs, b.segments[0] })) return result;
 	if (!backend.for_each(total, GatherPass{ total, b.perm[0], b.segmentOf[0], b.segments[0], b.boxes, b.forwards, b.backwards })) return result;
 	if (!backend.scan_items(b.forwards, b.heads, total)) return result;
-	ScanItem everything;
-	if (!backend.read(b.heads + (total - 1u), &everything, 1)) return result;
-	root.flags = major_axis(to_box(everything)) | kNeedSort;
-	unsigned long long noCut = kNoCut;
-	if (!backend.write(b.segments[0], &root, 1) || !backend.write(b.best[0], &noCut, 1)) return result;
+	if (!backend.for_each(packCount, RootAxisPass{ b.heads, b.segments[0], b.best[0] })) return result;
 
-	std::vector<std::pair<uint32_t, uint32_t>> levels = { { 0u, 1u } }; // node id range {first, count} of every binary depth
-	uint32_t count = total, segmentCount = 1u, nodeBase = 1u;
+	std::vector<std::pair<uint32_t, uint32_t>> levels = { { 0u, packCount } }; // node id range {first, count} of every binary depth
+	uint32_t count = total, segmentCount = packCount, nodeBase = packCount;
 	bool anySort = true;
 	int side = 0;                                     // which of the segmentOf / segments / best pairs holds the current level
 	uint32_t *current = b.perm[0], *other = b.perm[1]; // position -> primitive of the current level, and the spare buffer
@@ -783,23 +854,37 @@ Result build(Backend& backend, const EchoTriangle* triangles, uint32_t triangleC
 		side ^= 1;
 	}
 
-	// collapse: sizes bottom-up over the even levels, indices and nodes top-down
-	if (!backend.fill_zero(b.quadIndex, sizeof(uint32_t))) return result; // the root is quad node 0
+	// collapse: sizes bottom-up over the even levels, then every root's place (the packs back to back), indices and nodes top-down
 	int last = (int)levels.size() - 1;
 	for (int level = last - (last & 1); level >= 0; level -= 2)
 		if (!backend.for_each(levels[level].second, QuadCountPass{ levels[level].first, b.nodes, b.quadCount, b.quadDepth })) return result;
-	for (int level = 0; level <= last; level += 2)
-		if (!backend.for_each(levels[level].second, QuadEmitPass{ levels[level].first, b.nodes, b.quadCount, b.quadIndex, b.quads })) return result;
 
-	uint32_t nodeCount = 0, maxDepth = 0;
-	if (!backend.read(b.quadCount, &nodeCount, 1) || !backend.read(b.quadDepth, &maxDepth, 1)) return result;
+	result.packNodeCount.resize(packCount);
+	result.packMaxDepth.resize(packCount);
+	result.packNodeBase.resize(packCount);
+	if (!backend.exclusive_sum(b.quadCount, b.rootBase, packCount)) return result; // the roots are binary nodes 0 .. packCount - 1
+	if (!backend.read(b.quadCount, result.packNodeCount.data(), packCount) || !backend.read(b.quadDepth, result.packMaxDepth.data(), packCount)
+		|| !backend.read(b.rootBase, result.packNodeBase.data(), packCount)) return result;
+	if (!backend.for_each(packCount, QuadRootPass{ b.rootBase, b.quadIndex, b.quadBase })) return result;
+
+	for (int level = 0; level <= last; level += 2)
+		if (!backend.for_each(levels[level].second, QuadEmitPass{ levels[level].first, b.nodes, b.quadCount, b.quadIndex, b.quadBase, b.quads })) return result;
 
 	result.ok = true;
-	result.nodeCount = nodeCount;
-	result.maxDepth = maxDepth;
+	result.nodeCount = result.packNodeBase[packCount - 1u] + result.packNodeCount[packCount - 1u];
+	result.maxDepth = result.packMaxDepth[0];
 	result.levels = (uint32_t)levels.size();
 	result.quads = b.quads;
 	return result;
+}
+
+// one pack: the tree of GeometryCollection.CreateBounds' triangles, spheres and placements
+template<class Backend>
+Result build(Backend& backend, const EchoTriangle* triangles, uint32_t triangleCount, const EchoSphere* spheres, uint32_t sphereCount,
+             const float* instanceBounds, uint32_t instanceCount)
+{
+	const PackRange pack = { 0u, triangleCount, 0u, sphereCount, 0u, instanceCount, 0u };
+	return build_forest(backend, &pack, 1u, triangles, spheres, instanceBounds);
 }
 
 } // namespace sweep

@@ -100,6 +100,12 @@ struct CudaBackend
 			&& check_cuda(cudaStreamSynchronize(stream), "light build level");
 	}
 
+	template<class T>
+	bool write(T* destination, const T* source, uint32_t n) // from pageable host memory: the copy has left `source` on return
+	{
+		return check_cuda(cudaMemcpyAsync(destination, source, sizeof(T) * n, cudaMemcpyHostToDevice, stream), "cudaMemcpyAsync(light write)");
+	}
+
 	bool fill_zero(void* pointer, size_t bytes) { return check_cuda(cudaMemsetAsync(pointer, 0, bytes, stream), "cudaMemsetAsync(light)"); }
 };
 

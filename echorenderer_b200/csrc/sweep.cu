@@ -136,7 +136,7 @@ bool build_qbvh_sweep(const EchoTriangle* triangles, uint32_t triangleCount, con
 	{
 		sweep::Buffers probe;
 		sweep::Arena measure;
-		probe.carve(measure, total64);
+		probe.carve(measure, total64, 1u);
 		size_t freeBytes = 0, totalBytes = 0;
 		if (!check_cuda(cudaMemGetInfo(&freeBytes, &totalBytes), "cudaMemGetInfo")) return false;
 		size_t needed = measure.used + backend.scratchBytes + sizeof(EchoTriangle) * triangleCount + sizeof(EchoSphere) * sphereCount + sizeof(float) * 6 * instanceCount + (1u << 20);

@@ -21,12 +21,16 @@ from .host import PreparedArrays
 class PreparedScene:
     """The flattened scene resident on one B200; the device twin of Echo's PreparedScene."""
 
-    def __init__(self, prepared: PreparedArrays, device: int = 0, devices=None, build_tree_on_device: bool = False, build_light_tree_on_device: bool = False):
+    def __init__(self, prepared: PreparedArrays, device: int = 0, devices=None, build_tree_on_device: bool = False, build_light_tree_on_device: bool = False,
+                 build_packs_on_device: bool = False):
         """`device`: the CUDA device of a single-device scene. `build_tree_on_device`: the library builds the accelerator itself from
         the uploaded triangles and spheres (echo_b200_scene_build_qbvh: the SweepBuilder's tree, on the device) instead of taking
         `prepared.nodes`; `self.built_tree` = (node count, max depth) then. `build_light_tree_on_device`: likewise the light tree
         (echo_b200_scene_build_light_tree: LightTree.Build on the device) instead of `prepared.light_nodes` and the emitter map;
-        `self.built_light_tree` = (node count, emitter count, power) then. `devices` (a list of device indices) instead replicates the scene
+        `self.built_light_tree` = (node count, emitter count, power) then. Both refuse a scene with packs (ValueError /
+        EchoNativeError); `build_packs_on_device`
+        builds every pack of one instead, QBVH and light tree, in one call (echo_b200_scene_build_packs) and ignores `prepared`'s nodes,
+        light trees and the outputs of its pack records; `self.built_packs` = (node count, light node count, emitter count, power) then. `devices` (a list of device indices) instead replicates the scene
         on several devices of this process (echo_b200_scene_create_multi): trace / occlude split their batches over them and
         render_tiles deals blocks of tiles to them; the *_device methods then do not apply."""
         lib = _native.library()
@@ -48,12 +52,18 @@ class PreparedScene:
             triangles, spheres, materials = prepared.triangles, prepared.spheres, prepared.materials
             _native.check(lib.echo_b200_scene_set_triangles(self._handle, ptr(triangles), len(triangles)))
             _native.check(lib.echo_b200_scene_set_spheres(self._handle, ptr(spheres), len(spheres)))
+            instanced = prepared.packs is not None
+            if instanced and build_tree_on_device:  # scene_build_qbvh would see one flat scene: set_packs comes after it
+                raise ValueError("build_tree_on_device builds the accelerator of a scene without packs: use build_packs_on_device=True")
+            if build_packs_on_device and not instanced:
+                raise ValueError("build_packs_on_device builds a scene with packs: use build_tree_on_device / build_light_tree_on_device")
             self.built_tree = None
+            self.built_packs = None
             if build_tree_on_device:
                 count, depth = ctypes.c_uint32(), ctypes.c_uint32()
                 _native.check(lib.echo_b200_scene_build_qbvh(self._handle, ctypes.byref(count), ctypes.byref(depth)))
                 self.built_tree = (count.value, depth.value)
-            else:
+            elif not build_packs_on_device:  # the pack build installs the nodes after set_packs
                 _native.check(lib.echo_b200_scene_set_qbvh(self._handle, ptr(prepared.nodes), len(prepared.nodes), prepared.max_depth))
             _native.check(lib.echo_b200_scene_set_materials(self._handle, ptr(materials), len(materials)))
             if prepared.textures is not None:
@@ -64,7 +74,13 @@ class PreparedScene:
             if prepared.packs is not None:
                 _native.check(lib.echo_b200_scene_set_packs(self._handle, ptr(prepared.packs), len(prepared.packs), ptr(prepared.instances), len(prepared.instances)))
             self.built_light_tree = None
-            if build_light_tree_on_device:
+            if build_packs_on_device:
+                counts = [ctypes.c_uint32() for _ in range(3)]
+                power = ctypes.c_float()
+                _native.check(lib.echo_b200_scene_build_packs(self._handle, ptr(prepared.point_lights), len(prepared.point_lights),
+                                                              *(ctypes.byref(c) for c in counts), ctypes.byref(power)))
+                self.built_packs = (counts[0].value, counts[1].value, counts[2].value, power.value)
+            elif build_light_tree_on_device:
                 count, emitters, power = ctypes.c_uint32(), ctypes.c_uint32(), ctypes.c_float()
                 _native.check(lib.echo_b200_scene_build_light_tree(self._handle, ptr(prepared.point_lights), len(prepared.point_lights),
                                                                    ctypes.byref(count), ctypes.byref(emitters), ctypes.byref(power)))
@@ -472,6 +488,55 @@ def build_light_tree_device(description, instance_lights=None, device=0):
                                                  _native.pointer(points), len(points), _native.pointer(rows), len(rows), _native.pointer(nodes), len(nodes), ctypes.byref(node_count),
                                                  _native.pointer(tokens), _native.pointer(paths), len(tokens), ctypes.byref(emitter_count), ctypes.byref(power)))
     return nodes[:node_count.value].copy(), tokens[:emitter_count.value].copy(), paths[:emitter_count.value].copy(), float(power.value)
+
+
+@dataclass
+class BuiltPacks:
+    """What echo_b200_build_packs returns: the pack records completed (nodeOffset / nodeCount / maxDepth / lightNode* / emitter*),
+    every pack's QBVH nodes, light nodes, emitter tokens and bit paths back to back in pack order, and pack 0's light-tree root power."""
+    packs: np.ndarray
+    nodes: np.ndarray
+    light_nodes: np.ndarray
+    emitter_tokens: np.ndarray
+    emitter_bitpaths: np.ndarray
+    power: float
+
+    @property
+    def max_depth(self):
+        return int(self.packs["maxDepth"].max())
+
+
+def pack_build_arguments(prepared):
+    """The inputs of echo_b200_build_packs from an instanced PreparedArrays: the shared arrays, the pack records with only their input
+    ranges kept (geometry, placements, swatch, point lights), and output arrays with room for any result."""
+    packs = np.zeros(len(prepared.packs), dtype=structs.PACK)
+    for name in ("triangleOffset", "triangleCount", "sphereOffset", "sphereCount", "instanceOffset", "instanceCount", "materialOffset", "pointLightOffset", "pointLightCount"):
+        packs[name] = prepared.packs[name]
+    triangles = np.ascontiguousarray(prepared.triangles, dtype=structs.TRIANGLE)
+    spheres = np.ascontiguousarray(prepared.spheres, dtype=structs.SPHERE)
+    materials = np.ascontiguousarray(prepared.materials, dtype=structs.MATERIAL)
+    points = np.ascontiguousarray(prepared.point_lights, dtype=structs.POINT_LIGHT)
+    instances = np.ascontiguousarray(prepared.instances, dtype=structs.INSTANCE)
+    candidates = len(triangles) + len(spheres) + len(instances) + len(points)
+    outputs = (np.empty(max(len(triangles) + len(spheres) + len(instances), 1), dtype=structs.QBVH_NODE), np.empty(max(2 * candidates, 1), dtype=structs.LIGHT_NODE),
+               np.empty(max(candidates, 1), dtype=np.uint32), np.empty(max(candidates, 1), dtype=np.uint64))
+    return (triangles, spheres, materials, points, packs, instances), outputs
+
+
+def build_packs_device(prepared, device=0):
+    """Every pack of an instanced scene built on the device in one call (echo_b200_build_packs, csrc/packbuild.cu): each pack's QBVH
+    and light tree equal host.build_qbvh / host.build_light_tree's byte for byte, fed with the placements' rows the device computes
+    from the finished child trees. Returns BuiltPacks; the arrays are laid out as host.prepare lays them out."""
+    lib = _native.library()
+    (triangles, spheres, materials, points, packs, instances), (nodes, light_nodes, tokens, paths) = pack_build_arguments(prepared)
+    ptr = _native.pointer
+    node_count, light_count, emitter_count, power = ctypes.c_uint32(), ctypes.c_uint32(), ctypes.c_uint32(), ctypes.c_float()
+    _native.check(lib.echo_b200_build_packs(device, ptr(triangles), len(triangles), ptr(spheres), len(spheres), ptr(materials), len(materials), ptr(points), len(points),
+                                            ptr(packs), len(packs), ptr(instances), len(instances), ptr(nodes), len(nodes), ctypes.byref(node_count),
+                                            ptr(light_nodes), len(light_nodes), ctypes.byref(light_count), ptr(tokens), ptr(paths), len(tokens), ctypes.byref(emitter_count),
+                                            ctypes.byref(power)))
+    return BuiltPacks(packs, nodes[:node_count.value].copy(), light_nodes[:light_count.value].copy(), tokens[:emitter_count.value].copy(),
+                      paths[:emitter_count.value].copy(), float(power.value))
 
 
 def shard_epochs(max_epoch, rank, world_size):

@@ -510,6 +510,69 @@ def instanced_scene(grid=6, rings=24, segments=26, nested=True):
                             infinite_lights=ambient_light((0.3, 0.35, 0.4)), camera=camera, name="instanced")
 
 
+def many_packs_scene(pack_count=40, seed=1, layers=3):
+    """Many distinct packs placed in `layers` (2 or 3) layers: the input of a build that serves all packs of one height together
+    (echo_b200_build_packs). Packs of the bottom layer are small blobs, some with glowing triangles or spheres, some without any
+    emitter, some lit by point lights only; packs of the layers above hold two to four placements of the layer below, some of them
+    nothing else. The scene places every top-layer pack, so host.prepare keeps them all."""
+    from .host import InstanceDescription, PackDescription
+    rng = np.random.default_rng(seed)
+    layers = max(2, min(3, int(layers)))
+    sizes = [pack_count // 2 + pack_count % 2] + [pack_count // (2 * (layers - 1))] * (layers - 1)
+    sizes[-1] += pack_count - sum(sizes)
+    glow = material(structs.MATERIAL_EMISSIVE, (5.0, 4.0, 3.0))
+    packs, previous = [], []
+
+    def placement(candidates):
+        position = tuple(rng.uniform(-3.0, 3.0, 3))
+        rotation = tuple(float(v) for v in rng.integers(0, 360, 3))
+        return InstanceDescription(int(rng.choice(candidates)), position, rotation, float(rng.uniform(0.3, 0.8)))
+
+    for k in range(sizes[0]):
+        kind = k % 4  # 0: glowing triangles, 1: glowing sphere, 2: no emitter, 3: point lights only
+        materials = np.concatenate([material(structs.MATERIAL_DIFFUSE, tuple(rng.uniform(0.2, 0.9, 3))), glow])
+        triangles = blob_triangles(tuple(rng.uniform(-1, 1, 3)), float(rng.uniform(0.5, 1.5)), 0, 4 + k % 5, 5 + k % 4, seed=seed * 1000 + k)
+        if kind == 0:
+            triangles["material"][::7] = 1
+        spheres = np.zeros(1 + k % 3, dtype=structs.SPHERE)
+        spheres["position"] = rng.uniform(-1.5, 1.5, (len(spheres), 3))
+        spheres["radius"] = rng.uniform(0.1, 0.4, len(spheres))
+        spheres["material"] = 1 if kind == 1 else 0
+        points = np.zeros(1 + k % 2 if kind == 3 else 0, dtype=structs.POINT_LIGHT)
+        points["position"], points["intensity"] = rng.uniform(-2, 2, (len(points), 3)), (2.0, 2.0, 2.5)
+        packs.append(PackDescription(triangles=triangles, spheres=spheres, materials=materials, point_lights=points))
+        previous.append(len(packs) - 1)
+
+    for layer in range(1, layers):
+        current = []
+        for k in range(sizes[layer]):
+            instances = [placement(previous) for _ in range(2 + k % 3)]
+            if k % 2 == 0:  # placements only
+                packs.append(PackDescription(instances=instances))
+            else:
+                packs.append(PackDescription(triangles=box(0, tuple(rng.uniform(0.3, 1.0, 3)), tuple(rng.uniform(-1, 1, 3))),
+                                             materials=material(structs.MATERIAL_DIFFUSE, (0.6, 0.6, 0.6)), instances=instances))
+            current.append(len(packs) - 1)
+        previous = current
+
+    used = set()
+    for pack in packs:
+        used.update(instance.pack for instance in pack.instances)
+    roots = [index for index in range(len(packs)) if index not in used]
+    instances = []
+    for k, index in enumerate(roots):
+        position = ((k % 8 - 3.5) * 8.0, 2.0, (k // 8 - 3.0) * 8.0)
+        instances.append(InstanceDescription(index, position, (0.0, float((k * 37) % 360), 0.0), 1.0))
+
+    materials = np.concatenate([material(structs.MATERIAL_DIFFUSE, (0.7, 0.7, 0.7)), material(structs.MATERIAL_EMISSIVE, (8.0, 8.0, 7.0))])
+    extent = 80.0
+    triangles = np.concatenate([plane(0, (extent, extent)), plane(1, (10.0, 10.0), (0, 20, 0), (180, 0, 0))])
+    position = (0.0, 30.0, -60.0)
+    camera = perspective_camera(position, look_rotation(position, (0, 0, 0)), field_of_view=60.0)
+    return SceneDescription(triangles=triangles, materials=materials, instances=instances, packs=packs,
+                            infinite_lights=ambient_light((0.2, 0.2, 0.25)), camera=camera, name="many_packs")
+
+
 def _planar_texcoords(triangles, scale, axes=(0, 2)):
     """Texture coordinates from two position axes (a planar projection), `scale` repeats per unit."""
     v0 = triangles["vertex0"].astype(np.float64)

@@ -469,6 +469,34 @@ int32_t echo_b200_build_light_tree(int32_t device, const EchoTriangle* triangles
 int32_t echo_b200_scene_build_light_tree(EchoScene*, const EchoPointLight* points, uint32_t point_count,
                                          uint32_t* out_node_count, uint32_t* out_emitter_count, float* out_power);
 
+/* Optional device-side build of EVERY PACK of an instanced scene in one call: each pack's QBVH and light tree as echo_b200_build_qbvh_instanced
+ * and echo_b200_build_light_tree build them (byte for byte the host mirror's, pack by pack), and the rows those calls take for the placements
+ * — PreparedInstance.BoxBound (FillBounds(6) of the child's accelerator, centre / extent through EchoInstance.inverse) and LightBound (the
+ * child's light-tree root moved the same way; a zero row without emitters) — computed on the device from the finished child trees. Packs of
+ * equal height (0 without placements, else 1 + the tallest pack placed) are built together, as one forest per driver, so a call reads back
+ * as many levels per height as its deepest pack has (csrc/echo_pack_build.h). Inputs: the arrays of all packs back to back, `packs` with
+ * each pack's triangle / sphere / instance / point-light ranges and materialOffset (a pack's swatch ends where the next swatch of the
+ * array begins, another pack's or a placement's), `instances` with forward / inverse / scales / pack. On return every pack record also
+ * holds nodeOffset / nodeCount / maxDepth / lightNodeOffset / lightNodeCount / emitterOffset / emitterCount, and the outputs hold every
+ * pack's nodes, light nodes, emitter tokens and bit paths back to back in pack order (host.prepare's layout), ready for set_qbvh /
+ * set_light_tree / set_packs. out_power = pack 0's light-tree root power (what echo_host_infinite_threshold takes). Room: nodes <= the
+ * primitives (placements included), light nodes <= 2 x emitters, emitters <= point lights + primitives. Refusals: a pack of fewer than 2
+ * primitives, a cycle, nesting deeper than ECHO_MAX_INSTANCE_LAYERS, too little room (with the needed counts): ECHO_B200_ERR_INVALID; a light
+ * tree deeper than 63 levels: ECHO_B200_ERR_UNSUPPORTED. Trees of a height the forest cannot build as the reference's (see build_qbvh) are
+ * built pack by pack, falling back as echo_b200_build_qbvh does. */
+int32_t echo_b200_build_packs(int32_t device, const EchoTriangle* triangles, uint32_t triangle_count, const EchoSphere* spheres, uint32_t sphere_count,
+                              const EchoMaterial* materials, uint32_t material_count, const EchoPointLight* points, uint32_t point_count,
+                              EchoPack* packs, uint32_t pack_count, const EchoInstance* instances, uint32_t instance_count,
+                              EchoQbvhNode* out_nodes, uint32_t node_capacity, uint32_t* out_node_count,
+                              EchoLightNode* out_light_nodes, uint32_t light_node_capacity, uint32_t* out_light_node_count,
+                              uint32_t* out_emitter_tokens, uint64_t* out_emitter_bitpaths, uint32_t emitter_capacity, uint32_t* out_emitter_count,
+                              float* out_power);
+/* The same build for a scene handle: call it after set_triangles / set_spheres / set_materials / set_packs instead of set_qbvh and
+ * set_light_tree. It builds on the scene's (first) device, installs the nodes, light trees and emitter maps with `points`, and completes the
+ * staged pack records; commit uploads them (to every device of a multi-device handle). out_* are optional. */
+int32_t echo_b200_scene_build_packs(EchoScene*, const EchoPointLight* points, uint32_t point_count,
+                                    uint32_t* out_node_count, uint32_t* out_light_node_count, uint32_t* out_emitter_count, float* out_power);
+
 /* Page-locked host memory for the host-buffer entry points. A P/Invoke caller pins managed arrays with `fixed`
  * (Processes/Composition/OidnDenoise.cs:109-110): that stops the GC from moving them but leaves them PAGEABLE for CUDA, so every
  * copy is staged through the driver's bounce buffer and cannot overlap the kernels (measured: bench.py `e2e_pageable`). Either

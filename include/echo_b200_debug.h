@@ -53,6 +53,10 @@ int32_t echo_b200_debug_set_option(const char* name, int64_t value);
 int32_t echo_b200_debug_last_build(float* out4);
 /* The same for the calling thread's last echo_b200_build_light_tree / echo_b200_scene_build_light_tree (csrc/lightbuild.cu); out4[3] = levels. */
 int32_t echo_b200_debug_last_light_build(float* out4);
+/* The calling thread's last echo_b200_build_packs / echo_b200_scene_build_packs (csrc/packbuild.cu): out8 = {rounds, QBVH levels read back,
+ * light-tree levels read back, synchronising read-backs in all, launches, ms of host wall time for the synchronised build, packs rebuilt one
+ * by one after the forest gave up, 0}. Zeros if no such build ran on this thread. */
+int32_t echo_b200_debug_last_pack_build(float* out8);
 
 #ifdef __cplusplus
 }

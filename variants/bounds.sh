@@ -5,7 +5,7 @@ set -e
 cd "$(dirname "$0")/../echorenderer_b200/csrc"
 out=/tmp/echo_bounds_build
 rm -rf $out && mkdir -p $out
-for f in api trace instanced build sweep render debug peaks; do
+for f in api trace instanced build sweep lightbuild packbuild render debug peaks; do
   nvcc -std=c++17 -O3 -gencode arch=compute_100a,code=sm_100a -lineinfo -fmad=false -Xcompiler -fPIC -DECHO_BOUNDS_CHECK -c $f.cu -o $out/$f.o &
 done
 wait
