@@ -1241,6 +1241,7 @@ int32_t echo_b200_render_tiles(EchoScene* scene, const EchoRenderParams* params,
 	if (!require_renderable(scene)) return ECHO_B200_ERR_INVALID;
 	if (!params || (!tileXY && tileCount) || (!outRGBA && tileCount)) return fail(ECHO_B200_ERR_INVALID, "null argument");
 	if (params->tileSize <= 0) return fail(ECHO_B200_ERR_INVALID, "invalid EchoRenderParams");
+	if (!stratified_extend_valid(*params)) return fail(ECHO_B200_ERR_INVALID, "ECHO_DISTRIBUTION_STRATIFIED takes an extend of 1 to 2^23");
 	if (stats) *stats = EchoStats{};
 	if (tileCount == 0) return ECHO_B200_OK;
 	if (scene->replicas.empty()) return render_tiles_device(scene, params, tileXY, tileCount, outRGBA, stats);
@@ -1303,6 +1304,7 @@ int32_t echo_b200_render_frame_device(EchoScene* scene, const EchoRenderParams* 
 {
 	if (!require_renderable(scene) || !single_device(scene)) return ECHO_B200_ERR_INVALID;
 	if (!params || (!tileXY && tileCount) || !frame) return fail(ECHO_B200_ERR_INVALID, "null argument");
+	if (!stratified_extend_valid(*params)) return fail(ECHO_B200_ERR_INVALID, "ECHO_DISTRIBUTION_STRATIFIED takes an extend of 1 to 2^23");
 	if (stats) *stats = EchoStats{};
 	if (tileCount == 0) return ECHO_B200_OK;
 
@@ -1327,6 +1329,7 @@ int32_t echo_b200_debug_evaluate_samples(EchoScene* scene, const EchoRenderParam
 {
 	if (!require_renderable(scene)) return ECHO_B200_ERR_INVALID;
 	if (!params || !pixelXY || !sampleIndex || !outRGB) return fail(ECHO_B200_ERR_INVALID, "null argument");
+	if (!stratified_extend_valid(*params)) return fail(ECHO_B200_ERR_INVALID, "ECHO_DISTRIBUTION_STRATIFIED takes an extend of 1 to 2^23");
 	DeviceGuard guard(scene->device);
 	if (!guard.ok) return ECHO_B200_ERR_NO_DEVICE;
 	std::lock_guard<std::mutex> turn(scene->compute);
@@ -1353,6 +1356,7 @@ int32_t echo_b200_debug_evaluate_samples4(EchoScene* scene, const EchoRenderPara
 {
 	if (!require_renderable(scene)) return ECHO_B200_ERR_INVALID;
 	if (!params || !pixelXY || !sampleIndex || !outRGBA) return fail(ECHO_B200_ERR_INVALID, "null argument");
+	if (!stratified_extend_valid(*params)) return fail(ECHO_B200_ERR_INVALID, "ECHO_DISTRIBUTION_STRATIFIED takes an extend of 1 to 2^23");
 	DeviceGuard guard(scene->device);
 	if (!guard.ok) return ECHO_B200_ERR_NO_DEVICE;
 	std::lock_guard<std::mutex> turn(scene->compute);

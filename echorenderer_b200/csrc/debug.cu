@@ -155,6 +155,30 @@ __global__ void debug_math_kernel(int op, const float* __restrict__ a, const flo
 	out[i] = r;
 }
 
+// op 103: the stratified sequence's draw (ECHO_DISTRIBUTION_STRATIFIED), one per element pair (2i, 2i + 1), inputs as bits:
+// a = {seed, pixel}, b = {sample index, extend}, c = {first dimension, 1 for a 2D draw}; out = {value, second value or 0}
+__global__ void debug_stratified_kernel(const float* __restrict__ a, const float* __restrict__ b, const float* __restrict__ c, uint64_t pairs, float* __restrict__ out)
+{
+	uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+	if (i >= pairs) return;
+
+	uint32_t seed = __float_as_uint(a[2 * i]), pixel = __float_as_uint(a[2 * i + 1]);
+	uint32_t sample = __float_as_uint(b[2 * i]), extend = __float_as_uint(b[2 * i + 1]);
+	uint32_t dimension = __float_as_uint(c[2 * i]);
+
+	if (extend == 0u || extend > (uint32_t)ECHO_DISTRIBUTION_STRATIFIED_EXTEND_MAX)
+	{
+		out[2 * i] = out[2 * i + 1] = __uint_as_float(0x7FC00000u);
+		return;
+	}
+
+	uint32_t series = stratified_series(seed, pixel, sample / extend);
+	Strata strata = make_strata(extend, sample);
+	vec2 value = __float_as_uint(c[2 * i + 1]) != 0u ? stratified_2d(series, dimension, strata) : vec2{ stratified_1d(series, dimension, strata), 0.0f };
+	out[2 * i] = value.x;
+	out[2 * i + 1] = value.y;
+}
+
 bool launch_debug_bxdf(int32_t kind, const float* params, const float* outgoing, const float* samples, uint64_t n,
                        float* sampled8, float* evaluated4, float* inverse4, cudaStream_t stream)
 {
@@ -167,6 +191,14 @@ bool launch_debug_bxdf(int32_t kind, const float* params, const float* outgoing,
 bool launch_debug_math(int32_t op, const float* a, const float* b, const float* c, uint64_t n, float* out, cudaStream_t stream)
 {
 	if (n == 0) return true;
+
+	if (op == 103)
+	{
+		if (n % 2 != 0) { set_error("op 103 takes element pairs"); return false; }
+		debug_stratified_kernel<<<(unsigned int)((n / 2 + 127) / 128), 128, 0, stream>>>(a, b, c, n / 2, out);
+		return check_cuda(cudaGetLastError(), "debug_stratified_kernel launch");
+	}
+
 	debug_math_kernel<<<(unsigned int)((n + 127) / 128), 128, 0, stream>>>(op, a, b, c, n, out);
 	return check_cuda(cudaGetLastError(), "debug_math_kernel launch");
 }

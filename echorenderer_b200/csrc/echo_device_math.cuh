@@ -385,4 +385,92 @@ ECHO_DEVICE float sample_value(uint32_t key, uint32_t dimension)
 	return sample1d((float)(h >> 8) * 5.9604644775390625e-8f);
 }
 
+// ---- the stratified sequence (ECHO_DISTRIBUTION_STRATIFIED); same constants and operations as its CPU reference, tests/c_client/stratified_oracle.cpp ----
+ECHO_DEVICE uint32_t stratified_series(uint32_t seed, uint32_t pixel, uint32_t epoch)
+{
+	uint32_t h = hash32(seed ^ 0x3C6EF372u);
+	h = hash32(h + pixel * 0x85EBCA6Bu + 0x165667B1u);
+	h = hash32(h ^ (epoch * 0xC2B2AE35u + 0x27D4EB2Fu));
+	return h;
+}
+
+ECHO_DEVICE uint32_t stratified_pattern(uint32_t series, uint32_t dimension) { return hash32(hash32(series + dimension * 0x9E3779B1u) ^ 0x5BD1E995u); }
+ECHO_DEVICE uint32_t stratified_jitter(uint32_t pattern, uint32_t position) { return hash32(hash32(pattern ^ 0xB5297A4Du) + position * 0x68E31DA4u); }
+
+ECHO_DEVICE uint32_t stratified_permute(uint32_t i, uint32_t length, uint32_t p) // Kensler's permute (CMJ, Pixar memo 13-01)
+{
+	uint32_t w = length - 1u; // the next power-of-two mask
+	w |= w >> 1;
+	w |= w >> 2;
+	w |= w >> 4;
+	w |= w >> 8;
+	w |= w >> 16;
+
+	do
+	{
+		i ^= p;
+		i *= 0xE170893Du;
+		i ^= p >> 16;
+		i ^= (i & w) >> 4;
+		i ^= p >> 8;
+		i *= 0x0929EB3Fu;
+		i ^= p >> 23;
+		i ^= (i & w) >> 1;
+		i *= 1u | p >> 27;
+		i *= 0x6935FA69u;
+		i ^= (i & w) >> 11;
+		i *= 0x74DCB303u;
+		i ^= (i & w) >> 2;
+		i *= 0x9E501CC3u;
+		i ^= (i & w) >> 2;
+		i *= 0xC860A3DFu;
+		i &= w;
+		i ^= i >> 5;
+	}
+	while (i >= length);
+
+	return (i + p) % length;
+}
+
+// (stratum + j) / extend in one IEEE division of exact floats, strictly inside the stratum (stratified_point of tests/c_client/stratified_oracle.cpp)
+ECHO_DEVICE float stratified_point(uint32_t stratum, uint32_t jitter, uint32_t extend)
+{
+	uint32_t bits = 32u - __clz(extend - 1u);
+	uint32_t shift = 24u - bits;
+	uint32_t numerator = (stratum << shift) | ((jitter >> 8 >> (bits + 1u)) << 1) | 1u;
+	return sample1d(__fdiv_rn((float)numerator, (float)(extend << shift)));
+}
+
+// a sample's place in its epoch: the epoch's size, the columns m of its 2D grid (the largest divisor not above the root) and its position
+struct Strata
+{
+	uint32_t extend, columns, position;
+};
+
+ECHO_DEVICE Strata make_strata(uint32_t extend, uint32_t sampleIndex)
+{
+	uint32_t m = (uint32_t)__fsqrt_rn((float)extend);
+	while (m * m > extend) m--;
+	while ((m + 1u) * (m + 1u) <= extend) m++;
+	while (extend % m != 0u) m--;
+	return { extend, m, sampleIndex % extend };
+}
+
+ECHO_DEVICE float stratified_1d(uint32_t series, uint32_t dimension, const Strata& s)
+{
+	uint32_t p = stratified_pattern(series, dimension);
+	return stratified_point(stratified_permute(s.position, s.extend, p), stratified_jitter(p, s.position), s.extend);
+}
+
+ECHO_DEVICE vec2 stratified_2d(uint32_t series, uint32_t dimension, const Strata& s) // correlated multi-jittered over m x n
+{
+	uint32_t m = s.columns, n = s.extend / m;
+	uint32_t p = stratified_pattern(series, dimension);
+	uint32_t px = hash32(p ^ 0xA511E9B3u), py = hash32(p ^ 0x63D83595u);
+	uint32_t shuffled = stratified_permute(s.position, s.extend, p);
+	uint32_t x = shuffled % m, y = shuffled / m;
+	uint32_t sx = stratified_permute(x, m, px), sy = stratified_permute(y, n, py);
+	return { stratified_point(x * n + sy, stratified_jitter(px, s.position), s.extend), stratified_point(y * m + sx, stratified_jitter(py, s.position), s.extend) };
+}
+
 } // namespace echo

@@ -65,6 +65,7 @@ void render_state_destroy(RenderState* state);
 // Renders `tileCount` tiles. When `frame` is non-null the per-pixel means are ADDED into the full-frame device buffer
 // (xyz = mean * epochs rendered, w += epochs) for multi-device sample/tile sharding; when `tilesOut` is non-null the
 // tile-major Float4 means are written there (device pointer). Synchronises `stream` internally between wavefront steps.
+bool stratified_extend_valid(const EchoRenderParams& params); // ECHO_DISTRIBUTION_STRATIFIED's extend limit (always true without the flag)
 bool render_tiles(RenderState* state, const DeviceScene& scene, const EchoRenderParams& params, const int32_t* tileXY, uint32_t tileCount,
                   float4* tilesOut, float4* frame, EchoStats* stats, cudaStream_t stream);
 

@@ -52,7 +52,7 @@ struct PathBuffers
 	float4* result;       // rgb, w = bits: bounces done | mode << 16
 	float4* oldPosition;  // MIS: GeometryPoint oldPoint
 	float4* oldNormal;
-	uint32_t* key;        // sample_key(seed, pixel, sample)
+	uint32_t* key;        // sample_key(seed, pixel, sample); stratified: stratified_series(seed, pixel, epoch)
 
 	// shadow rays of the current bounce, compacted: {origin.xyz, direction.x | direction.yz, travel, ignore} + pending value
 	float4* shadowQueue;
@@ -67,6 +67,8 @@ struct PathBuffers
 	uint32_t* classQueue[CLASS_COUNT]; // ray slots sorted by the material class of what they hit
 	uint32_t* counters;
 	unsigned long long* stats; // EchoStats layout
+
+	const uint32_t* sampleIndex; // per path id (WorkerState::sampleIndex): stratified draws take the sample's position in its epoch from it
 };
 
 // ECHO_B200_PROFILE=1: per-kernel device time of the wavefront (CUDA events around every launch, synchronised; the
@@ -1124,6 +1126,32 @@ ECHO_DEVICE void camera_spawn(const EchoCamera& camera, int width, int height, i
 // kernels
 // ---------------------------------------------------------------------------------------------------------------------
 
+// The draws of one sample in the reference's pairing (CameraSample.cs:19-23; PathTracedEvaluator.cs:60-66): the uniform sequence
+// (sample_value), or with STRAT the stratified one (ECHO_DISTRIBUTION_STRATIFIED). STRAT is a template parameter of every kernel
+// that draws, so the uniform instantiations carry no trace of the stratified code (the shading kernels run at the register cap).
+template<bool STRAT>
+ECHO_DEVICE float draw1d(uint32_t key, const Strata& strata, uint32_t dimension)
+{
+	if (STRAT) return stratified_1d(key, dimension, strata);
+	return sample_value(key, dimension);
+}
+
+template<bool STRAT>
+ECHO_DEVICE vec2 draw2d(uint32_t key, const Strata& strata, uint32_t dimension)
+{
+	if (STRAT) return stratified_2d(key, dimension, strata);
+	return { sample_value(key, dimension), sample_value(key, dimension + 1u) };
+}
+
+// the sample's place in its epoch, read only by the stratified instantiations
+template<bool STRAT>
+ECHO_DEVICE Strata path_strata(const EchoRenderParams& params, const PathBuffers& paths, uint32_t id)
+{
+	if (STRAT) return make_strata((uint32_t)params.extend, paths.sampleIndex[id]);
+	return { 0u, 0u, 0u };
+}
+
+template<bool STRAT>
 __global__ void __launch_bounds__(kBlock) raygen_kernel(DeviceScene scene, EchoRenderParams params, uint32_t count, const int2* __restrict__ pixelXY,
                                                        const uint32_t* __restrict__ sampleIndex, PathBuffers paths)
 {
@@ -1131,10 +1159,13 @@ __global__ void __launch_bounds__(kBlock) raygen_kernel(DeviceScene scene, EchoR
 	if (i >= count) return;
 
 	int2 pixel = pixelXY[i];
-	uint32_t key = sample_key(params.seed, (uint32_t)pixel.y * (uint32_t)params.width + (uint32_t)pixel.x, sampleIndex[i]);
+	const uint32_t pixelIndex = (uint32_t)pixel.y * (uint32_t)params.width + (uint32_t)pixel.x;
+	const Strata strata = path_strata<STRAT>(params, paths, i);
+	uint32_t key = STRAT ? stratified_series(params.seed, pixelIndex, sampleIndex[i] / (uint32_t)params.extend) // Distribution.BeginSeries per epoch
+	                     : sample_key(params.seed, pixelIndex, sampleIndex[i]);
 
-	vec2 shift = { sample_value(key, 0u), sample_value(key, 1u) }; // CameraSample.Create, CameraSample.cs:19-23
-	vec2 lens = { sample_value(key, 2u), sample_value(key, 3u) };
+	vec2 shift = draw2d<STRAT>(key, strata, 0u); // CameraSample.Create, CameraSample.cs:19-23
+	vec2 lens = draw2d<STRAT>(key, strata, 2u);
 
 	vec3 origin, direction;
 	camera_spawn(scene.camera, params.width, params.height, pixel.x, pixel.y, shift, lens, origin, direction);
@@ -1378,7 +1409,7 @@ struct ShadeOut
 // One loop body of PathTracedEvaluator.Evaluate for the path whose ray sits in slot `raySlot` of the current queue and whose hit
 // record is in hitQueue[raySlot]. CLASS / KINDS prune the code to what a material-class queue can contain; CLASS < 0 keeps
 // everything (the tail kernel), `missed` then says whether the ray hit anything.
-template<int CLASS, uint32_t KINDS, bool INST, bool COUNT = false>
+template<int CLASS, uint32_t KINDS, bool INST, bool STRAT, bool COUNT = false>
 ECHO_DEVICE void shade_body(const DeviceScene& scene, const EchoRenderParams& params, const PathBuffers& paths, int current, uint32_t raySlot, bool missed, ShadeOut& o)
 {
 	bool &statInfinite = o.statInfinite, &statBounce = o.statBounce, &statSpecular = o.statSpecular, &statMis = o.statMis;
@@ -1502,11 +1533,12 @@ ECHO_DEVICE void shade_body(const DeviceScene& scene, const EchoRenderParams& pa
 		if (bounces < (uint32_t)params.bounceLimit)
 		{
 			uint32_t key = stream_load(paths.key + id);
+			const Strata strata = path_strata<STRAT>(params, paths, id);
 			uint32_t dimension = 4u + 6u * bounces;
-			vec2 bounceSample = { sample_value(key, dimension), sample_value(key, dimension + 1u) };
-			float survivalSample = sample_value(key, dimension + 2u);
-			float lightSample = sample_value(key, dimension + 3u);
-			vec2 radiantSample = { sample_value(key, dimension + 4u), sample_value(key, dimension + 5u) };
+			vec2 bounceSample = draw2d<STRAT>(key, strata, dimension);
+			float survivalSample = draw1d<STRAT>(key, strata, dimension + 2u);
+			float lightSample = draw1d<STRAT>(key, strata, dimension + 3u);
+			vec2 radiantSample = draw2d<STRAT>(key, strata, dimension + 4u);
 
 			// Bounce, :326-354
 			vec3 incident;
@@ -1629,7 +1661,7 @@ ECHO_DEVICE void shade_emit(const PathBuffers& paths, int current, const ShadeOu
 	stat_add(paths.stats, STAT_LIGHT_OCCLUSION_CHECKED, o.statChecked);
 }
 
-template<int CLASS, uint32_t KINDS, bool INST>
+template<int CLASS, uint32_t KINDS, bool INST, bool STRAT>
 __global__ void __launch_bounds__(kBlock, ECHO_SHADE_MIN_BLOCKS) shade_kernel(DeviceScene scene, EchoRenderParams params, const uint32_t* __restrict__ queue,
                                                       const uint32_t* __restrict__ queueCount, PathBuffers paths, int current)
 {
@@ -1637,7 +1669,7 @@ __global__ void __launch_bounds__(kBlock, ECHO_SHADE_MIN_BLOCKS) shade_kernel(De
 	bool active = i < *queueCount;
 
 	ShadeOut o;
-	if (active) shade_body<CLASS, KINDS, INST>(scene, params, paths, current, stream_load(queue + i), false, o);
+	if (active) shade_body<CLASS, KINDS, INST, STRAT>(scene, params, paths, current, stream_load(queue + i), false, o);
 	shade_emit<INST>(paths, current, o);
 }
 
@@ -1645,14 +1677,14 @@ __global__ void __launch_bounds__(kBlock, ECHO_SHADE_MIN_BLOCKS) shade_kernel(De
 // the all-lobes body the tail kernel uses (same operations per path, same bits), instantiated with the light-tree visit counter, so
 // the class kernels of ordinary renders carry no counting code at all (a never-taken branch in the light-tree descent cost the
 // diffuse class 2.4x on the instanced scene: registers at the 80-register cap).
-template<bool INST>
+template<bool INST, bool STRAT>
 __global__ void __launch_bounds__(kBlock) shade_counted_kernel(DeviceScene scene, EchoRenderParams params, const uint32_t* __restrict__ rayCount, PathBuffers paths, int current)
 {
 	uint32_t i = blockIdx.x * kBlock + threadIdx.x;
 	bool active = i < *rayCount;
 
 	ShadeOut o;
-	if (active) shade_body<-1, KINDS_ALL, INST, true>(scene, params, paths, current, i, __float_as_uint(paths.hitQueue[i].x) == ECHO_TOKEN_EMPTY, o);
+	if (active) shade_body<-1, KINDS_ALL, INST, STRAT, true>(scene, params, paths, current, i, __float_as_uint(paths.hitQueue[i].x) == ECHO_TOKEN_EMPTY, o);
 	shade_emit<INST>(paths, current, o);
 }
 
@@ -1799,7 +1831,7 @@ constexpr int kAuxiliaryBounceCap = 1024; // both evaluators loop `while (scene.
 // AlbedoEvaluator.Evaluate (AlbedoEvaluator.cs:18-55) / NormalDepthEvaluator.Evaluate (NormalDepthEvaluator.cs:20-60): one
 // thread per sample follows purely specular bounces from the camera ray raygen_kernel left in rayQueue[0] and reports the
 // first other surface. These passes run at a few samples per pixel for the denoiser: a plain loop, no wavefront.
-template<int STACK, bool INST>
+template<int STACK, bool INST, bool STRAT>
 __global__ void __launch_bounds__(kBlock) auxiliary_kernel(DeviceScene scene, EchoRenderParams params, uint32_t count, PathBuffers paths, float4* __restrict__ out)
 {
 	uint32_t i = blockIdx.x * kBlock + threadIdx.x;
@@ -1809,6 +1841,7 @@ __global__ void __launch_bounds__(kBlock) auxiliary_kernel(DeviceScene scene, Ec
 	vec3 origin = xyz(rayA), direction = { rayA.w, rayB.x, rayB.y };
 	const vec3 cameraDirection = direction;
 	const uint32_t key = paths.key[i];
+	const Strata strata = path_strata<STRAT>(params, paths, i);
 	const int kind = params.evaluator & ECHO_EVALUATOR_KIND_MASK;
 	const bool divergeOnce = (params.evaluator & ECHO_EVALUATOR_DIVERGE_ONCE) != 0;
 
@@ -1883,7 +1916,7 @@ __global__ void __launch_bounds__(kBlock) auxiliary_kernel(DeviceScene scene, Ec
 
 		if (((KINDS_AUXILIARY >> bsdf.kind) & 1u) == 0u) { leave(); continue; } // bsdf.Count != bsdf.CountSpecular: not fully specular
 
-		vec2 sample = { sample_value(key, dimension), sample_value(key, dimension + 1u) };
+		vec2 sample = draw2d<STRAT>(key, strata, dimension);
 		dimension += 2u;
 
 		vec3 incident;
@@ -1919,7 +1952,7 @@ __global__ void __launch_bounds__(kBlock) auxiliary_kernel(DeviceScene scene, Ec
 // loops trace -> shade -> shadow -> next bounce until its path ends, with the same device functions as the wavefront
 // kernels (shade_body with every lobe compiled in) and the same per-path buffers, so every path sees the same sequence of
 // operations and its radiance keeps its bits.
-template<int STACK, bool INST>
+template<int STACK, bool INST, bool STRAT>
 __global__ void __launch_bounds__(kBlock) tail_kernel(DeviceScene scene, EchoRenderParams params, const uint32_t* __restrict__ queueCount, PathBuffers paths, int current)
 {
 	uint32_t i = blockIdx.x * kBlock + threadIdx.x;
@@ -1970,7 +2003,7 @@ __global__ void __launch_bounds__(kBlock) tail_kernel(DeviceScene scene, EchoRen
 
 		// ---- one loop body of Evaluate ----
 		ShadeOut o;
-		shade_body<-1, KINDS_ALL, INST>(scene, params, paths, current, i, !hit, o);
+		shade_body<-1, KINDS_ALL, INST, STRAT>(scene, params, paths, current, i, !hit, o);
 		counted[3] += o.statInfinite; counted[4] += o.statBounce; counted[5] += o.statSpecular;
 		counted[6] += o.statMis; counted[7] += o.statSampled; counted[8] += o.statChecked;
 
@@ -2032,7 +2065,7 @@ __global__ void __launch_bounds__(kBlock) tail_kernel(DeviceScene scene, EchoRen
 // emission (bounceLimit <= 128) and folds them backwards once the path has ended.
 constexpr int kNaiveBounceCap = 128;
 
-template<int STACK, bool INST>
+template<int STACK, bool INST, bool STRAT>
 __global__ void __launch_bounds__(kBlock) naive_kernel(DeviceScene scene, EchoRenderParams params, uint32_t count, PathBuffers paths, float4* __restrict__ out)
 {
 	uint32_t i = blockIdx.x * kBlock + threadIdx.x;
@@ -2044,6 +2077,7 @@ __global__ void __launch_bounds__(kBlock) naive_kernel(DeviceScene scene, EchoRe
 		float4 rayA = paths.rayQueue[0][i * 2u], rayB = paths.rayQueue[0][i * 2u + 1u];
 		vec3 origin = xyz(rayA), direction = { rayA.w, rayB.x, rayB.y };
 		const uint32_t key = paths.key[i];
+		const Strata strata = path_strata<STRAT>(params, paths, i);
 		const bool packs = INST && scene.packCount != 0u;
 		const bool textured = INST && scene.textureCount != 0u;
 		const int limit = params.bounceLimit < kNaiveBounceCap ? params.bounceLimit : kNaiveBounceCap;
@@ -2114,7 +2148,7 @@ __global__ void __launch_bounds__(kBlock) naive_kernel(DeviceScene scene, EchoRe
 			// `material is Emissive emissive ? emissive.Emit(contact.point, contact.outgoing) : RGB128.Black`, :42
 			rgb emission = material.type == ECHO_MATERIAL_EMISSIVE && dot(outgoing, normal) > 0.0f ? material_emission(material) : make_rgb(0.0f);
 
-			vec2 sample = { sample_value(key, 4u + 2u * (uint32_t)depth), sample_value(key, 5u + 2u * (uint32_t)depth) };
+			vec2 sample = draw2d<STRAT>(key, strata, 4u + 2u * (uint32_t)depth);
 			vec3 incident;
 			int selectedType;
 			Sampled sampled = bsdf_sample<KINDS_ALL>(bsdf, outgoing, sample, incident, selectedType);
@@ -2457,6 +2491,7 @@ static bool ensure_capacity(WorkerState* state, uint64_t paths, uint64_t pixels,
 
 	if (!ok) return false;
 
+	b.sampleIndex = state->sampleIndex;
 	state->capacity = paths;
 	state->pixelCapacity = pixels;
 	state->tileCapacity = tiles;
@@ -2600,21 +2635,27 @@ static bool evaluate_paths(WorkerState* state, const DeviceScene& sceneIn, const
 	if (count == 0u) return true;
 	if (!check_cuda(cudaMemsetAsync(counters, 0, sizeof(uint32_t) * 64, stream), "cudaMemsetAsync(counters)")) return false;
 
+	// ECHO_DISTRIBUTION_STRATIFIED: every kernel that draws runs its stratified instantiation
+	const bool stratified = (params.evaluator & ECHO_DISTRIBUTION_STRATIFIED) != 0;
+
 	timer.start(stream);
-	raygen_kernel<<<blocks_for(count), kBlock, 0, stream>>>(sceneIn, params, count, state->pixelXY, state->sampleIndex, paths);
+	if (stratified) raygen_kernel<true><<<blocks_for(count), kBlock, 0, stream>>>(sceneIn, params, count, state->pixelXY, state->sampleIndex, paths);
+	else raygen_kernel<false><<<blocks_for(count), kBlock, 0, stream>>>(sceneIn, params, count, state->pixelXY, state->sampleIndex, paths);
 	timer.stop(KernelTimer::RAYGEN, stream);
 	++launches;
 
 	if ((params.evaluator & ECHO_EVALUATOR_KIND_MASK) == ECHO_EVALUATOR_NAIVE)
 	{
-		naive_kernel<STACK, INST><<<blocks_for(count), kBlock, 0, stream>>>(sceneIn, params, count, paths, state->sampleOut);
+		if (stratified) naive_kernel<STACK, INST, true><<<blocks_for(count), kBlock, 0, stream>>>(sceneIn, params, count, paths, state->sampleOut);
+		else naive_kernel<STACK, INST, false><<<blocks_for(count), kBlock, 0, stream>>>(sceneIn, params, count, paths, state->sampleOut);
 		++launches;
 		return check_cuda(cudaGetLastError(), "naive_kernel launch");
 	}
 
 	if ((params.evaluator & ECHO_EVALUATOR_KIND_MASK) != ECHO_EVALUATOR_PATH_TRACED)
 	{
-		auxiliary_kernel<STACK, INST><<<blocks_for(count), kBlock, 0, stream>>>(sceneIn, params, count, paths, state->sampleOut);
+		if (stratified) auxiliary_kernel<STACK, INST, true><<<blocks_for(count), kBlock, 0, stream>>>(sceneIn, params, count, paths, state->sampleOut);
+		else auxiliary_kernel<STACK, INST, false><<<blocks_for(count), kBlock, 0, stream>>>(sceneIn, params, count, paths, state->sampleOut);
 		++launches;
 		return check_cuda(cudaGetLastError(), "auxiliary_kernel launch");
 	}
@@ -2738,7 +2779,8 @@ static bool evaluate_paths(WorkerState* state, const DeviceScene& sceneIn, const
 		// the tail: finish the few paths that are left in one launch (it traces for itself: the hits of k are simply not used)
 		if (!timer.enabled && !counted && bound < tailLimit)
 		{
-			tail_kernel<STACK, INST><<<blocks, kBlock, 0, stream>>>(scene, iterationParams, activeCount, paths, current);
+			if (stratified) tail_kernel<STACK, INST, true><<<blocks, kBlock, 0, stream>>>(scene, iterationParams, activeCount, paths, current);
+			else tail_kernel<STACK, INST, false><<<blocks, kBlock, 0, stream>>>(scene, iterationParams, activeCount, paths, current);
 			if (!check_cuda(cudaGetLastError(), "tail_kernel launch")) return false;
 			++launches;
 			break;
@@ -2750,7 +2792,8 @@ static bool evaluate_paths(WorkerState* state, const DeviceScene& sceneIn, const
 
 		if (counted)
 		{
-			shade_counted_kernel<INST><<<blocks, kBlock, 0, stream>>>(scene, iterationParams, activeCount, paths, current);
+			if (stratified) shade_counted_kernel<INST, true><<<blocks, kBlock, 0, stream>>>(scene, iterationParams, activeCount, paths, current);
+			else shade_counted_kernel<INST, false><<<blocks, kBlock, 0, stream>>>(scene, iterationParams, activeCount, paths, current);
 			++launches;
 		}
 
@@ -2760,8 +2803,12 @@ static bool evaluate_paths(WorkerState* state, const DeviceScene& sceneIn, const
 		if (classRays[CLASS_VALUE] != 0u)                                                                                                                \
 		{                                                                                                                                                \
 			timer.start(stream);                                                                                                                         \
-			shade_kernel<CLASS_VALUE, KINDS_VALUE, INST><<<blocks_for(classRays[CLASS_VALUE]), kBlock, 0, stream>>>(scene, iterationParams, paths.classQueue[CLASS_VALUE], \
-			                                                                                                        classCounts + CLASS_VALUE, paths, current);         \
+			if (stratified)                                                                                                                              \
+				shade_kernel<CLASS_VALUE, KINDS_VALUE, INST, true><<<blocks_for(classRays[CLASS_VALUE]), kBlock, 0, stream>>>(scene, iterationParams,       \
+				                                                             paths.classQueue[CLASS_VALUE], classCounts + CLASS_VALUE, paths, current);     \
+			else                                                                                                                                         \
+				shade_kernel<CLASS_VALUE, KINDS_VALUE, INST, false><<<blocks_for(classRays[CLASS_VALUE]), kBlock, 0, stream>>>(scene, iterationParams,      \
+				                                                             paths.classQueue[CLASS_VALUE], classCounts + CLASS_VALUE, paths, current);     \
 			timer.stop(SLOT, stream);                                                                                                                    \
 			++launches;                                                                                                                                  \
 		}
@@ -2904,6 +2951,11 @@ static bool render_batch(WorkerState* state, const DeviceScene& scene, const Ech
 	return check_cuda(cudaGetLastError(), "resolve_tiles_kernel launch");
 }
 
+bool stratified_extend_valid(const EchoRenderParams& params)
+{
+	return (params.evaluator & ECHO_DISTRIBUTION_STRATIFIED) == 0 || (params.extend > 0 && params.extend <= ECHO_DISTRIBUTION_STRATIFIED_EXTEND_MAX);
+}
+
 bool render_tiles(RenderState* state, const DeviceScene& scene, const EchoRenderParams& params, const int32_t* tileXY, uint32_t tileCount,
                   float4* tilesOut, float4* frame, EchoStats* stats, cudaStream_t stream)
 {
@@ -2919,7 +2971,8 @@ bool render_tiles(RenderState* state, const DeviceScene& scene, const EchoRender
 		return false;
 	}
 
-	if ((params.evaluator & ECHO_EVALUATOR_KIND_MASK) > ECHO_EVALUATOR_NAIVE || (params.evaluator & ~(ECHO_EVALUATOR_KIND_MASK | ECHO_EVALUATOR_DIVERGE_ONCE | ECHO_EVALUATOR_COUNT_VISITS)) != 0)
+	if ((params.evaluator & ECHO_EVALUATOR_KIND_MASK) > ECHO_EVALUATOR_NAIVE
+	    || (params.evaluator & ~(ECHO_EVALUATOR_KIND_MASK | ECHO_EVALUATOR_DIVERGE_ONCE | ECHO_EVALUATOR_COUNT_VISITS | ECHO_DISTRIBUTION_STRATIFIED)) != 0)
 	{
 		set_error("unknown EchoRenderParams.evaluator");
 		return false;
@@ -2928,6 +2981,12 @@ bool render_tiles(RenderState* state, const DeviceScene& scene, const EchoRender
 	if ((params.evaluator & ECHO_EVALUATOR_COUNT_VISITS) != 0 && (params.evaluator & ECHO_EVALUATOR_KIND_MASK) != ECHO_EVALUATOR_PATH_TRACED)
 	{
 		set_error("ECHO_EVALUATOR_COUNT_VISITS is a switch of the path-traced evaluator");
+		return false;
+	}
+
+	if (!stratified_extend_valid(params))
+	{
+		set_error("ECHO_DISTRIBUTION_STRATIFIED takes an extend of 1 to 2^23");
 		return false;
 	}
 
@@ -3031,6 +3090,12 @@ bool render_tiles(RenderState* state, const DeviceScene& scene, const EchoRender
 bool evaluate_sample_list(RenderState* renderState, const DeviceScene& scene, const EchoRenderParams& params, int channels, const int32_t* pixelXYHost, const uint32_t* sampleIndexHost,
                           uint64_t n, float* outRGBHost, cudaStream_t)
 {
+	if (!stratified_extend_valid(params))
+	{
+		set_error("ECHO_DISTRIBUTION_STRATIFIED takes an extend of 1 to 2^23");
+		return false;
+	}
+
 	WorkerState* state = get_worker(renderState, 0);
 	if (!state) return false;
 	cudaStream_t stream = state->stream;

@@ -291,19 +291,20 @@ class StandardNaiveEvaluator:
 
 @dataclass(frozen=True)
 class EvaluationProfile:
-    """Processes/Evaluation/EvaluationProfile.cs:13-75 (Distribution reduced to its Extend and seed)."""
+    """Processes/Evaluation/EvaluationProfile.cs:13-75 (Distribution reduced to its Extend, its seed and its kind)."""
     evaluator: object = field(default_factory=PathTracedEvaluator)
     extend: int = 16                # ContinuousDistribution.Extend, ContinuousDistribution.cs:25
     min_epoch: int = 1
     max_epoch: int = 20
     noise_threshold: float = 0.045
     seed: int = 1
+    stratified: bool = False        # Distribution is a StratifiedDistribution (StratifiedDistribution.cs:34-50); extend <= 2^23
 
     def validate(self):
         """EvaluationProfile.Validate, EvaluationProfile.cs:65-75."""
         if self.evaluator is None:
             raise ValueError("Evaluator is null")
-        if self.extend <= 0:
+        if self.extend <= 0 or (self.stratified and self.extend > structs.DISTRIBUTION_STRATIFIED_EXTEND_MAX):
             raise ValueError("Distribution.Extend out of bounds")
         if self.min_epoch <= 0 or self.max_epoch < self.min_epoch:
             raise ValueError("MinEpoch / MaxEpoch out of bounds")
@@ -568,7 +569,7 @@ class EvaluationOperation:
         p = self.profile
         return structs.render_params(self.destination.width, self.destination.height, self.destination.tile_size, p.extend, p.min_epoch,
                                      p.max_epoch, p.noise_threshold, p.evaluator.bounce_limit, p.evaluator.survivability, p.seed,
-                                     evaluator=p.evaluator.code)
+                                     evaluator=p.evaluator.code | (structs.DISTRIBUTION_STRATIFIED if p.stratified else 0))
 
     @property
     def total_samples(self):

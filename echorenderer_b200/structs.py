@@ -117,6 +117,8 @@ RENDER_PARAMS = np.dtype([
 EVALUATOR_PATH_TRACED, EVALUATOR_ALBEDO, EVALUATOR_NORMAL_DEPTH, EVALUATOR_NAIVE = 0, 1, 2, 3
 EVALUATOR_DIVERGE_ONCE = 0x100
 EVALUATOR_COUNT_VISITS = 0x200  # counted pass: EchoStats reports node / triangle / sphere / light-node visits (bench roofline)
+DISTRIBUTION_STRATIFIED = 0x400  # StratifiedDistribution: jittered, shuffled strata per epoch and dimension (any evaluator)
+DISTRIBUTION_STRATIFIED_EXTEND_MAX = 1 << 23
 
 STATS_FIELDS = [
     "sampleEvaluated", "sampleRejected", "pixelEvaluated", "bounceCreated", "bounceSpecular", "bounceMis",
@@ -150,7 +152,8 @@ assert STATS.itemsize == 192
 def render_params(width, height, tile_size=16, extend=16, min_epoch=1, max_epoch=1, noise_threshold=0.045,
                   bounce_limit=128, survivability=2.5, seed=1, epoch_offset=0, evaluator=EVALUATOR_PATH_TRACED):
     """EvaluationProfile + PathTracedEvaluator defaults (EvaluationProfile.cs:42-60, PathTracedEvaluator.cs:33,40).
-    evaluator: EVALUATOR_* [| EVALUATOR_DIVERGE_ONCE] (AlbedoEvaluator.cs, NormalDepthEvaluator.cs)."""
+    evaluator: EVALUATOR_* [| EVALUATOR_DIVERGE_ONCE] [| DISTRIBUTION_STRATIFIED] (AlbedoEvaluator.cs, NormalDepthEvaluator.cs,
+    StratifiedDistribution.cs)."""
     params = np.zeros(1, dtype=RENDER_PARAMS)
     params["width"], params["height"], params["tileSize"] = width, height, tile_size
     params["extend"], params["minEpoch"], params["maxEpoch"] = extend, min_epoch, max_epoch

@@ -298,7 +298,7 @@ typedef struct EchoRenderParams
 	float survivability;    /* PathTracedEvaluator.Survivability */
 	uint32_t seed;          /* counter-based sample sequence seed */
 	int32_t epochOffset;    /* first epoch index this call renders (sample sharding across devices) */
-	int32_t evaluator;      /* ECHO_EVALUATOR_* [| ECHO_EVALUATOR_DIVERGE_ONCE]; 0 = PathTracedEvaluator */
+	int32_t evaluator;      /* ECHO_EVALUATOR_* [| ECHO_EVALUATOR_DIVERGE_ONCE] [| ECHO_DISTRIBUTION_STRATIFIED]; 0 = PathTracedEvaluator */
 } EchoRenderParams;
 ECHO_B200_ASSERT_SIZE(EchoRenderParams, 48);
 
@@ -317,6 +317,11 @@ ECHO_B200_ASSERT_SIZE(EchoRenderParams, 48);
 #define ECHO_EVALUATOR_COUNT_VISITS 0x200 /* PathTracedEvaluator only: a counted pass. Same samples, same results, but the traversal runs
                                              on the one-thread-per-query kernels with visit counters and EchoStats reports node / triangle /
                                              sphere / light-node visits. A measurement aid (bench.py's roofline), several times slower. */
+#define ECHO_DISTRIBUTION_STRATIFIED 0x400 /* EvaluationProfile.Distribution is a StratifiedDistribution (StratifiedDistribution.cs:34-50):
+                                              each pixel's epoch of `extend` samples is one jittered, shuffled stratified set per dimension
+                                              (2D draws correlated multi-jittered) instead of independent uniform numbers. Any evaluator,
+                                              counted passes too; extend at most 2^23 (ECHO_B200_ERR_INVALID above). */
+#define ECHO_DISTRIBUTION_STRATIFIED_EXTEND_MAX (1 << 23)
 
 /* ---- EvaluatorStatistics rows on the hot path, same labels/order as the reference reports them
  * (EvaluationOperation.cs:130-140; PathTracedEvaluator.cs:50-199) ---- */

@@ -136,7 +136,7 @@ struct PathTracedEvaluator // Evaluation/Evaluators/PathTracedEvaluator.cs:33,40
 	float Survivability = 2.5f;
 };
 
-struct EvaluationProfile // Processes/Evaluation/EvaluationProfile.cs:13-75 (Distribution reduced to its Extend and a seed)
+struct EvaluationProfile // Processes/Evaluation/EvaluationProfile.cs:13-75 (Distribution reduced to its Extend, a seed and its kind)
 {
 	int32_t Evaluator = ECHO_EVALUATOR_PATH_TRACED; // ECHO_EVALUATOR_* [| ECHO_EVALUATOR_DIVERGE_ONCE]; a negative value stands for a null Evaluator
 	PathTracedEvaluator PathTraced;
@@ -145,11 +145,12 @@ struct EvaluationProfile // Processes/Evaluation/EvaluationProfile.cs:13-75 (Dis
 	int32_t MaxEpoch = 20;
 	float NoiseThreshold = 0.045f;
 	uint32_t Seed = 1;
+	bool Stratified = false; // Distribution is a StratifiedDistribution (ECHO_DISTRIBUTION_STRATIFIED); Extend <= 2^23
 
 	void Validate() const // :65-75
 	{
 		if (Evaluator < 0) throw std::invalid_argument("Evaluator is null");
-		if (Extend <= 0) throw std::invalid_argument("Distribution is null or its Extend is out of bounds");
+		if (Extend <= 0 || (Stratified && Extend > ECHO_DISTRIBUTION_STRATIFIED_EXTEND_MAX)) throw std::invalid_argument("Distribution is null or its Extend is out of bounds");
 		if (MinEpoch <= 0) throw std::invalid_argument("MinEpoch out of bounds");
 		if (MaxEpoch < MinEpoch) throw std::invalid_argument("MaxEpoch out of bounds");
 		if (NoiseThreshold < 0.0f) throw std::invalid_argument("NoiseThreshold out of bounds");
@@ -289,6 +290,25 @@ struct IWorker // Common/Compute/IWorker.cs: what an Operation sees of the threa
 // one echo_b200_render_tiles call over up to TilesPerProcedure consecutive tiles of the sequence. Execute(worker) is entered concurrently by
 // every worker, each claiming the next procedure with one atomic increment (Operation.cs:164-177); the library serialises calls on one scene
 // handle itself, and one call keeps every device of the scene busy, so extra workers simply wait for their turn.
+// the EchoRenderParams an EvaluationOperation renders `destination` with under `profile`
+inline EchoRenderParams RenderParameters(const EvaluationProfile& profile, const RenderTexture& destination)
+{
+	EchoRenderParams parameters = {};
+	parameters.width = destination.size.X;
+	parameters.height = destination.size.Y;
+	parameters.tileSize = destination.tileSize;
+	parameters.extend = profile.Extend;
+	parameters.minEpoch = profile.MinEpoch;
+	parameters.maxEpoch = profile.MaxEpoch;
+	parameters.noiseThreshold = profile.NoiseThreshold;
+	parameters.bounceLimit = profile.PathTraced.BounceLimit;
+	parameters.survivability = profile.PathTraced.Survivability;
+	parameters.seed = profile.Seed;
+	parameters.epochOffset = 0;
+	parameters.evaluator = profile.Evaluator | (profile.Stratified ? ECHO_DISTRIBUTION_STRATIFIED : 0);
+	return parameters;
+}
+
 class EvaluationOperation
 {
 public:
@@ -366,20 +386,7 @@ private:
 		size_t count = tilePositions.size() - first < TilesPerProcedure ? tilePositions.size() - first : TilesPerProcedure;
 		float* pixels = pixelMemory + (size_t)worker.Index() * TilesPerProcedure * tileFloats; // this worker's slice
 
-		EchoRenderParams parameters = {};
-		parameters.width = destination.size.X;
-		parameters.height = destination.size.Y;
-		parameters.tileSize = destination.tileSize;
-		parameters.extend = profile.Extend;
-		parameters.minEpoch = profile.MinEpoch;
-		parameters.maxEpoch = profile.MaxEpoch;
-		parameters.noiseThreshold = profile.NoiseThreshold;
-		parameters.bounceLimit = profile.PathTraced.BounceLimit;
-		parameters.survivability = profile.PathTraced.Survivability;
-		parameters.seed = profile.Seed;
-		parameters.epochOffset = 0;
-		parameters.evaluator = profile.Evaluator;
-
+		EchoRenderParams parameters = RenderParameters(profile, destination);
 		EchoStats stats = {};
 		static_assert(sizeof(Int2) == 2 * sizeof(int32_t), "Int2 is two packed 32-bit integers");
 		ThrowOnNativeError(echo_b200_render_tiles(scene->Handle(), &parameters, &tilePositions[first].X, (uint32_t)count, pixels, &stats), "echo_b200_render_tiles");

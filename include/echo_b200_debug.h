@@ -22,7 +22,11 @@ int32_t echo_b200_occlude_batch_device_counted(EchoScene*, const EchoRay* d_rays
 int32_t echo_b200_debug_bxdf_batch(int32_t device, int32_t kind, const float* params11, const float* outgoing3, const float* samples2,
                                    uint64_t n, float* sampled8, float* evaluated4, float* inverse4);
 
-/* FastMath / sincos shims, same op codes as oracle_fastmath (op 100: sin, 101: cos of the deterministic sincos). Host buffers. */
+/* FastMath / sincos shims, same op codes as oracle_fastmath (op 100: sin, 101: cos of the deterministic sincos). Host buffers.
+ * Op 102: the uniform sequence's first draw of (seed, pixel, sample) = (a, b, c) as bits. Op 103: the stratified sequence
+ * (ECHO_DISTRIBUTION_STRATIFIED, oracle_stratified_value) over element pairs (2i, 2i + 1), inputs as bits: a = {seed, pixel},
+ * b = {sample index, extend}, c = {first dimension, 1 for a 2D draw}; out = {value, the 2D draw's second value or 0}; n even,
+ * NaN for an extend outside 1 to 2^23. */
 int32_t echo_b200_debug_math(int32_t device, int32_t op, const float* a, const float* b, const float* c, uint64_t n, float* out);
 
 /* One Evaluator.Evaluate per listed (pixel, sample index): out_rgb receives n x 3 floats. Host buffers. */
