@@ -379,4 +379,25 @@ ECHO_DEVICE bool traverse_instanced(const DeviceScene& scene, vec3 origin, vec3 
 	return false;
 }
 
+// ---- PreparedScene.Trace / Occlude through the packs: the guards of scene_trace / scene_occlude (PreparedScene.cs:66-86) ----
+// `hitLayers` receives the hit's instance layers when a hit is accepted.
+template<int STACK, bool COUNT>
+ECHO_DEVICE bool scene_trace_layers(const DeviceScene& scene, vec3 origin, vec3 direction, uint32_t ignore, const PathLayers& ignoreLayers,
+                                    float& distance, uint32_t& token, vec2& uv, PathLayers& hitLayers, VisitCounts* counts)
+{
+	if (!positive(distance)) return false;
+	float original = distance;
+	traverse_instanced<STACK, false, COUNT>(scene, origin, direction, ignore, ignoreLayers.tokens, ignoreLayers.count, distance, token, uv, hitLayers.tokens, hitLayers.count, counts);
+	return distance < original;
+}
+
+template<int STACK, bool COUNT>
+ECHO_DEVICE bool scene_occlude_layers(const DeviceScene& scene, vec3 origin, vec3 direction, uint32_t ignore, const PathLayers& ignoreLayers, float travel, VisitCounts* counts)
+{
+	if (!positive(travel)) return false;
+	uint32_t token = ECHO_TOKEN_EMPTY, hitCount = 0u; // an occlusion query records no hit
+	vec2 uv = { 0.0f, 0.0f };
+	return traverse_instanced<STACK, true, COUNT>(scene, origin, direction, ignore, ignoreLayers.tokens, ignoreLayers.count, travel, token, uv, nullptr, hitCount, counts);
+}
+
 } // namespace echo

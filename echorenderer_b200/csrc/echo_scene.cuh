@@ -71,6 +71,22 @@ struct VisitCounts
 	uint32_t nodes, triangles, spheres;
 };
 
+// a per-thread counter summed over the warp and added to stats[slot] by lane 0, one atomic per warp and none for a zero sum;
+// every lane of the warp must call it
+ECHO_DEVICE void warp_add(unsigned long long* stats, int slot, uint32_t value)
+{
+	for (int offset = 16; offset > 0; offset >>= 1) value += __shfl_down_sync(0xFFFFFFFFu, value, offset);
+	if ((threadIdx.x & 31u) == 0u && value) atomicAdd(stats + slot, (unsigned long long)value);
+}
+
+// the visit counters of one thread's queries into stats[firstSlot], [firstSlot + 1], [firstSlot + 2]
+ECHO_DEVICE void visit_flush(unsigned long long* stats, int firstSlot, VisitCounts local)
+{
+	warp_add(stats, firstSlot + 0, local.nodes);
+	warp_add(stats, firstSlot + 1, local.triangles);
+	warp_add(stats, firstSlot + 2, local.spheres);
+}
+
 ECHO_DEVICE uint32_t token_type(uint32_t token) { return token >> ECHO_TOKEN_INDEX_BITS; }
 ECHO_DEVICE uint32_t token_index(uint32_t token) { return token & ((1u << ECHO_TOKEN_INDEX_BITS) - 1u); }
 ECHO_DEVICE bool token_is_geometry(uint32_t token) { return (token_type(token) - 1u) <= 2u; } // Triangle, Sphere, Instance

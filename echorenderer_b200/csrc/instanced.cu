@@ -64,22 +64,7 @@ __global__ void __launch_bounds__(kInstancedBlock) instanced_batch_kernel(Device
 		}
 	}
 
-	if (COUNT)
-	{
-		for (int offset = 16; offset > 0; offset >>= 1)
-		{
-			local.nodes += __shfl_down_sync(0xFFFFFFFFu, local.nodes, offset);
-			local.triangles += __shfl_down_sync(0xFFFFFFFFu, local.triangles, offset);
-			local.spheres += __shfl_down_sync(0xFFFFFFFFu, local.spheres, offset);
-		}
-
-		if ((threadIdx.x & 31) == 0)
-		{
-			atomicAdd(counts + 0, (unsigned long long)local.nodes);
-			atomicAdd(counts + 1, (unsigned long long)local.triangles);
-			atomicAdd(counts + 2, (unsigned long long)local.spheres);
-		}
-	}
+	if (COUNT) visit_flush(counts, 0, local);
 }
 
 template<bool ANY, bool COUNT>

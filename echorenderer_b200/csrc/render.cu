@@ -13,6 +13,7 @@
 #include <string>
 #include <cstring>
 #include <thread>
+#include <type_traits>
 #include <sched.h>
 #include <cstdio>
 #include <cstdlib>
@@ -242,26 +243,6 @@ enum : int
 	STAT_COUNT = 24
 };
 static_assert(sizeof(EchoStats) == sizeof(unsigned long long) * STAT_COUNT, "EchoStats layout");
-
-// counted passes (ECHO_EVALUATOR_COUNT_VISITS): the visit counters of one thread's query into the statistics, one atomic per warp
-// and counter; every lane of the warp must call it
-ECHO_DEVICE void visit_flush(unsigned long long* stats, int firstSlot, VisitCounts local)
-{
-	for (int offset = 16; offset > 0; offset >>= 1)
-	{
-		local.nodes += __shfl_down_sync(0xFFFFFFFFu, local.nodes, offset);
-		local.triangles += __shfl_down_sync(0xFFFFFFFFu, local.triangles, offset);
-		local.spheres += __shfl_down_sync(0xFFFFFFFFu, local.spheres, offset);
-	}
-
-	if ((threadIdx.x & 31u) == 0u)
-	{
-		if (local.nodes) atomicAdd(stats + firstSlot + 0, (unsigned long long)local.nodes);
-		if (local.triangles) atomicAdd(stats + firstSlot + 1, (unsigned long long)local.triangles);
-		if (local.spheres) atomicAdd(stats + firstSlot + 2, (unsigned long long)local.spheres);
-	}
-}
-
 
 ECHO_DEVICE vec3 xyz(float4 v) { return { v.x, v.y, v.z }; }
 ECHO_DEVICE rgb as_rgb(float4 v) { return { v.x, v.y, v.z }; }
@@ -1253,26 +1234,23 @@ struct ExtendLayersIO : ExtendIO
 	}
 };
 
-template<int STACK>
-__global__ void __launch_bounds__(kTraverseBlock, ECHO_INST_MIN_BLOCKS) extend_layers_kernel(DeviceScene scene, ExtendLayersIO io, const uint32_t* __restrict__ queueCount, unsigned long long* __restrict__ nextRay)
-{
-	__shared__ float4 stagedRays[kTraverseBlock * kStagedFloat4];
-	persistent_traverse<STACK, false, true>(scene, io, *queueCount, nextRay, stagedRays);
-	persistent_finish(nextRay);
-}
+template<bool PACKS>
+using ExtendIOFor = std::conditional_t<PACKS, ExtendLayersIO, ExtendIO>;
 
-template<int STACK>
-__global__ void __launch_bounds__(kTraverseBlock, ECHO_MIN_BLOCKS) extend_kernel(DeviceScene scene, ExtendIO io, const uint32_t* __restrict__ queueCount, unsigned long long* __restrict__ nextRay)
+// PACKS: through the instanced packs, with the ignore hierarchy's instance layers in and the hit's instance layers out
+template<int STACK, bool PACKS>
+__global__ void __launch_bounds__(kTraverseBlock, PACKS ? ECHO_INST_MIN_BLOCKS : ECHO_MIN_BLOCKS) extend_kernel(DeviceScene scene, ExtendIOFor<PACKS> io, const uint32_t* __restrict__ queueCount,
+                                                                                                               unsigned long long* __restrict__ nextRay)
 {
 	__shared__ float4 stagedRays[kTraverseBlock * kStagedFloat4];
-	persistent_traverse<STACK, false>(scene, io, *queueCount, nextRay, stagedRays);
+	persistent_traverse<STACK, false, PACKS>(scene, io, *queueCount, nextRay, stagedRays);
 	persistent_finish(nextRay);
 }
 
 // Narrow wavefronts (late bounces) have fewer rays than resident lanes: work replacement has nothing to replace with and
 // the launch is bound by the latency of its longest ray, so the leaner one-thread-per-ray loop is used instead.
-template<int STACK, bool COUNT>
-__global__ void __launch_bounds__(kBlock) extend_narrow_kernel(DeviceScene scene, ExtendIO io, const uint32_t* __restrict__ queueCount, unsigned long long* __restrict__ stats)
+template<int STACK, bool PACKS, bool COUNT>
+__global__ void __launch_bounds__(kBlock) extend_narrow_kernel(DeviceScene scene, ExtendIOFor<PACKS> io, const uint32_t* __restrict__ queueCount, unsigned long long* __restrict__ stats)
 {
 	uint32_t i = blockIdx.x * kBlock + threadIdx.x;
 	VisitCounts local = { 0u, 0u, 0u };
@@ -1283,42 +1261,16 @@ __global__ void __launch_bounds__(kBlock) extend_narrow_kernel(DeviceScene scene
 		float distance = b.z;
 		uint32_t token = ECHO_TOKEN_EMPTY;
 		vec2 uv = { 0.0f, 0.0f };
+		PathLayers hitLayers = no_layers();
+		bool hit;
 
-		bool hit = scene_trace<STACK, COUNT>(scene, { a.x, a.y, a.z }, { a.w, b.x, b.y }, __float_as_uint(b.w), distance, token, uv, COUNT ? &local : nullptr);
-		io.store_closest(i, hit, token, distance, uv, b.z);
-	}
-
-	if (COUNT) visit_flush(stats, STAT_NODE_VISITS, local);
-}
-
-// Instanced scenes: the same query through the packs (echo_instanced.cuh), one thread per ray, with the ignore hierarchy's
-// instance layers in and the hit's instance layers out.
-template<int STACK, bool COUNT>
-__global__ void __launch_bounds__(kBlock) extend_instanced_kernel(DeviceScene scene, ExtendIO io, const uint4* __restrict__ rayLayers, uint4* __restrict__ hitLayers,
-                                                                  const uint32_t* __restrict__ queueCount, unsigned long long* __restrict__ stats)
-{
-	uint32_t i = blockIdx.x * kBlock + threadIdx.x;
-	VisitCounts local = { 0u, 0u, 0u };
-
-	if (i < *queueCount)
-	{
-		float4 a = io.rays[i * 2u], b = io.rays[i * 2u + 1u];
-		PathLayers ignore = load_layers(rayLayers, i);
-		PathLayers hitLayer = no_layers();
-		float distance = b.z;
-		uint32_t token = ECHO_TOKEN_EMPTY;
-		vec2 uv = { 0.0f, 0.0f };
-		bool hit = false;
-
-		if (positive(b.z)) // PreparedScene.Trace, PreparedScene.cs:69
-		{
-			traverse_instanced<STACK, false, COUNT>(scene, { a.x, a.y, a.z }, { a.w, b.x, b.y }, __float_as_uint(b.w), ignore.tokens, ignore.count,
-			                                        distance, token, uv, hitLayer.tokens, hitLayer.count, COUNT ? &local : nullptr);
-			hit = distance < b.z;
-		}
+		if constexpr (PACKS)
+			hit = scene_trace_layers<STACK, COUNT>(scene, { a.x, a.y, a.z }, { a.w, b.x, b.y }, __float_as_uint(b.w), load_layers(io.rayLayers, i),
+			                                       distance, token, uv, hitLayers, COUNT ? &local : nullptr);
+		else hit = scene_trace<STACK, COUNT>(scene, { a.x, a.y, a.z }, { a.w, b.x, b.y }, __float_as_uint(b.w), distance, token, uv, COUNT ? &local : nullptr);
 
 		io.store_closest(i, hit, token, distance, uv, b.z);
-		store_layers(hitLayers, i, hit ? hitLayer : no_layers());
+		if constexpr (PACKS) store_layers(io.hitLayers, i, hit ? hitLayers : no_layers());
 	}
 
 	if (COUNT) visit_flush(stats, STAT_NODE_VISITS, local);
@@ -1394,6 +1346,51 @@ __global__ void __launch_bounds__(kClassifyBlock) classify_kernel(DeviceScene sc
 	if (shadeClass >= 0) stream_store(paths.classQueue[shadeClass] + blockBase[shadeClass] + offset, i);
 }
 
+// ---- PreparedScene.Interact (PreparedScene.cs:95-105) + GeometryCollection.GetContactInfo (:200-232) + material.Scatter ----
+// What a hit becomes: its shading point, material and BSDF. Every evaluator shades its hits through this one function.
+struct Contact
+{
+	SurfacePoint point;
+	vec3 shadeNormal, outgoing;
+	uint32_t materialIndex;
+	vec2 texcoord;
+	MaterialRecord material;
+	Bsdf bsdf;
+};
+
+template<bool INST>
+ECHO_DEVICE void interact(const DeviceScene& scene, uint32_t token, vec2 uv, float distance, const PathLayers& layers, vec3 origin, vec3 direction, Contact& c)
+{
+	Layer layer = find_layer<INST>(scene, layers); // FindLayer, :97
+	const bool textured = INST && scene.textureCount != 0u;
+	vec3 infoNormal, infoShading;
+	c.texcoord = { 0.0f, 0.0f };
+
+	if (token_type(token) == ECHO_TOKEN_TYPE_TRIANGLE)
+	{
+		TriangleData triangle = load_triangle(scene, layer.info.triangleOffset + token_index(token));
+		c.materialIndex = layer.materialOffset + triangle.material; // instance.swatch[info.material], :102
+		infoNormal = triangle_normal(triangle);
+		infoShading = triangle_shading_normal(triangle, uv);
+		if (textured) c.texcoord = triangle_texcoord(scene, layer.info.triangleOffset + token_index(token), uv);
+	}
+	else
+	{
+		c.materialIndex = layer.materialOffset + __ldg(scene.sphereMaterial + layer.info.sphereOffset + token_index(token));
+		infoNormal = infoShading = sphere_normal(uv);
+		if (textured) c.texcoord = sphere_texcoord(uv);
+	}
+
+	c.point.position = direction * max_net(distance, kEpsilon) + origin; // TraceQuery.Position, TraceQuery.cs:76-82
+	c.point.normal = normalized(transform_direction(layer.inverse, infoNormal)); // :100-101 (the identity without layers)
+	c.shadeNormal = normalized(transform_direction(layer.inverse, infoShading));
+	c.outgoing = -direction;
+	if (textured) apply_normal_mapping(scene, c.materialIndex, c.texcoord, c.shadeNormal); // GeometryShade's constructor, GeometryShade.cs:17
+
+	c.material = load_material(scene, c.materialIndex);
+	material_scatter<INST>(scene, c.material, c.outgoing, c.point.normal, c.shadeNormal, c.bsdf, c.materialIndex, c.texcoord);
+}
+
 // What one loop body of PathTracedEvaluator.Evaluate produces for a path: statistics, the next ray if the path goes on, the
 // shadow ray of its light sample if one is needed.
 struct ShadeOut
@@ -1461,46 +1458,16 @@ ECHO_DEVICE void shade_body(const DeviceScene& scene, const EchoRenderParams& pa
 	}
 	else
 	{
-		// ---- PreparedScene.Interact, PreparedScene.cs:95-105 + GeometryCollection.GetContactInfo (:200-232) ----
 		float4 hit4 = stream_load(paths.hitQueue + raySlot);
 		uint32_t token = __float_as_uint(hit4.x);
-		float distance = hit4.y;
-		vec2 uv = { hit4.z, hit4.w };
-		vec3 rayOrigin = xyz(rayA);
-
-		vec3 infoNormal, infoShading;
-		uint32_t materialIndex;
 
 		if (INST) hitLayers = load_layers(paths.hitLayers, raySlot);
-		Layer layer = find_layer<INST>(scene, hitLayers); // FindLayer, :97
-		const bool textured = INST && scene.textureCount != 0u;
-		vec2 texcoord = { 0.0f, 0.0f };
-
-		if (token_type(token) == ECHO_TOKEN_TYPE_TRIANGLE)
-		{
-			TriangleData triangle = load_triangle(scene, layer.info.triangleOffset + token_index(token));
-			materialIndex = layer.materialOffset + triangle.material; // instance.swatch[info.material], :102
-			infoNormal = triangle_normal(triangle);
-			infoShading = triangle_shading_normal(triangle, uv);
-			if (textured) texcoord = triangle_texcoord(scene, layer.info.triangleOffset + token_index(token), uv);
-		}
-		else
-		{
-			materialIndex = layer.materialOffset + __ldg(scene.sphereMaterial + layer.info.sphereOffset + token_index(token));
-			infoNormal = infoShading = sphere_normal(uv);
-			if (textured) texcoord = sphere_texcoord(uv);
-		}
-
-		SurfacePoint point;
-		point.position = direction * max_net(distance, kEpsilon) + rayOrigin; // TraceQuery.Position, TraceQuery.cs:76-82
-		point.normal = normalized(transform_direction(layer.inverse, infoNormal)); // :100-101 (the identity without layers)
-		vec3 shadeNormal = normalized(transform_direction(layer.inverse, infoShading));
-		vec3 outgoing = -direction;
-		if (textured) apply_normal_mapping(scene, materialIndex, texcoord, shadeNormal); // GeometryShade's constructor, GeometryShade.cs:17
-
-		MaterialRecord material = load_material(scene, materialIndex);
-		Bsdf bsdf;
-		material_scatter<INST>(scene, material, outgoing, point.normal, shadeNormal, bsdf, materialIndex, texcoord);
+		Contact contact;
+		interact<INST>(scene, token, { hit4.z, hit4.w }, hit4.y, hitLayers, xyz(rayA), direction, contact);
+		const SurfacePoint& point = contact.point;
+		const vec3 &shadeNormal = contact.shadeNormal, &outgoing = contact.outgoing;
+		const MaterialRecord& material = contact.material;
+		const Bsdf& bsdf = contact.bsdf;
 
 		// ---- emission of the new vertex: ContributeEmissive (:305-311), MIS-weighted after a MIS bounce (:96-109) ----
 		if ((CLASS == CLASS_TERMINAL || CLASS < 0) && material.type == ECHO_MATERIAL_EMISSIVE && positive(emissive_power(material)))
@@ -1729,38 +1696,24 @@ struct ShadowLayersIO : ShadowIO
 	ECHO_DEVICE void store_hit_layers(uint32_t, bool, const uint32_t*, uint32_t) const {}
 };
 
-template<int STACK>
-__global__ void __launch_bounds__(kTraverseBlock, ECHO_INST_MIN_BLOCKS) shadow_layers_kernel(DeviceScene scene, ShadowLayersIO io, const uint32_t* __restrict__ shadowCount, unsigned long long* __restrict__ nextRay,
-                                                                       unsigned long long* __restrict__ stats)
+template<bool PACKS>
+using ShadowIOFor = std::conditional_t<PACKS, ShadowLayersIO, ShadowIO>;
+
+template<int STACK, bool PACKS>
+__global__ void __launch_bounds__(kTraverseBlock, PACKS ? ECHO_INST_MIN_BLOCKS : ECHO_MIN_BLOCKS) shadow_kernel(DeviceScene scene, ShadowIOFor<PACKS> io, const uint32_t* __restrict__ shadowCount,
+                                                                                                               unsigned long long* __restrict__ nextRay, unsigned long long* __restrict__ stats)
 {
 	__shared__ float4 stagedRays[kTraverseBlock * kStagedFloat4];
 	io.passed = 0u;
-	persistent_traverse<STACK, true, true>(scene, io, *shadowCount, nextRay, stagedRays);
+	persistent_traverse<STACK, true, PACKS>(scene, io, *shadowCount, nextRay, stagedRays);
 	persistent_finish(nextRay);
 
-	uint32_t passed = io.passed;
-	for (int offset = 16; offset > 0; offset >>= 1) passed += __shfl_down_sync(0xFFFFFFFFu, passed, offset);
-	if ((threadIdx.x & 31u) == 0u && passed) atomicAdd(stats + STAT_LIGHT_OCCLUSION_PASSED, (unsigned long long)passed);
+	warp_add(stats, STAT_LIGHT_OCCLUSION_PASSED, io.passed);
 	if (blockIdx.x == 0 && threadIdx.x == 0) atomicAdd(stats + STAT_OCCLUDE_QUERIES, (unsigned long long)*shadowCount);
 }
 
-template<int STACK>
-__global__ void __launch_bounds__(kTraverseBlock, ECHO_MIN_BLOCKS) shadow_kernel(DeviceScene scene, ShadowIO io, const uint32_t* __restrict__ shadowCount, unsigned long long* __restrict__ nextRay,
-                                                              unsigned long long* __restrict__ stats)
-{
-	__shared__ float4 stagedRays[kTraverseBlock * kStagedFloat4];
-	io.passed = 0u;
-	persistent_traverse<STACK, true>(scene, io, *shadowCount, nextRay, stagedRays);
-	persistent_finish(nextRay);
-
-	uint32_t passed = io.passed;
-	for (int offset = 16; offset > 0; offset >>= 1) passed += __shfl_down_sync(0xFFFFFFFFu, passed, offset);
-	if ((threadIdx.x & 31u) == 0u && passed) atomicAdd(stats + STAT_LIGHT_OCCLUSION_PASSED, (unsigned long long)passed);
-	if (blockIdx.x == 0 && threadIdx.x == 0) atomicAdd(stats + STAT_OCCLUDE_QUERIES, (unsigned long long)*shadowCount);
-}
-
-template<int STACK, bool COUNT>
-__global__ void __launch_bounds__(kBlock) shadow_narrow_kernel(DeviceScene scene, ShadowIO io, const uint32_t* __restrict__ shadowCount, unsigned long long* __restrict__ stats)
+template<int STACK, bool PACKS, bool COUNT>
+__global__ void __launch_bounds__(kBlock) shadow_narrow_kernel(DeviceScene scene, ShadowIOFor<PACKS> io, const uint32_t* __restrict__ shadowCount, unsigned long long* __restrict__ stats)
 {
 	uint32_t i = blockIdx.x * kBlock + threadIdx.x;
 	bool active = i < *shadowCount;
@@ -1770,37 +1723,12 @@ __global__ void __launch_bounds__(kBlock) shadow_narrow_kernel(DeviceScene scene
 	if (active)
 	{
 		float4 a = io.rays[i * 2u], b = io.rays[i * 2u + 1u];
-		bool occluded = scene_occlude<STACK, COUNT>(scene, { a.x, a.y, a.z }, { a.w, b.x, b.y }, __float_as_uint(b.w), b.z, COUNT ? &local : nullptr);
-		io.store_any(i, occluded);
-	}
+		bool occluded;
 
-	stat_add(stats, STAT_OCCLUDE_QUERIES, active);
-	stat_add(stats, STAT_LIGHT_OCCLUSION_PASSED, io.passed != 0u);
-	if (COUNT) visit_flush(stats, STAT_NODE_VISITS, local);
-}
+		if constexpr (PACKS)
+			occluded = scene_occlude_layers<STACK, COUNT>(scene, { a.x, a.y, a.z }, { a.w, b.x, b.y }, __float_as_uint(b.w), load_layers(io.shadowLayers, i), b.z, COUNT ? &local : nullptr);
+		else occluded = scene_occlude<STACK, COUNT>(scene, { a.x, a.y, a.z }, { a.w, b.x, b.y }, __float_as_uint(b.w), b.z, COUNT ? &local : nullptr);
 
-template<int STACK, bool COUNT>
-__global__ void __launch_bounds__(kBlock) shadow_instanced_kernel(DeviceScene scene, ShadowIO io, const uint4* __restrict__ shadowLayers,
-                                                                  const uint32_t* __restrict__ shadowCount, unsigned long long* __restrict__ stats)
-{
-	uint32_t i = blockIdx.x * kBlock + threadIdx.x;
-	bool active = i < *shadowCount;
-	io.passed = 0u;
-	VisitCounts local = { 0u, 0u, 0u };
-
-	if (active)
-	{
-		float4 a = io.rays[i * 2u], b = io.rays[i * 2u + 1u];
-		PathLayers ignore = load_layers(shadowLayers, i);
-		PathLayers unusedLayers = no_layers();
-		float travel = b.z;
-		uint32_t unusedToken = ECHO_TOKEN_EMPTY;
-		vec2 unusedUV = { 0.0f, 0.0f };
-		bool occluded = false;
-
-		if (positive(b.z)) // PreparedScene.Occlude, PreparedScene.cs:84
-			occluded = traverse_instanced<STACK, true, COUNT>(scene, { a.x, a.y, a.z }, { a.w, b.x, b.y }, __float_as_uint(b.w), ignore.tokens, ignore.count,
-			                                                  travel, unusedToken, unusedUV, unusedLayers.tokens, unusedLayers.count, COUNT ? &local : nullptr);
 		io.store_any(i, occluded);
 	}
 
@@ -1861,74 +1789,41 @@ __global__ void __launch_bounds__(kBlock) auxiliary_kernel(DeviceScene scene, Ec
 		PathLayers hitLayers = no_layers();
 		bool hit;
 
-		if (INST && scene.packCount != 0u) // INST without packs is a textured scene: one pack, ordinary traversal
-		{
-			traverse_instanced<STACK, false, false>(scene, origin, direction, ignore, ignoreLayers.tokens, ignoreLayers.count, distance, token, uv, hitLayers.tokens, hitLayers.count, nullptr);
-			hit = distance < kInfinity;
-		}
-		else hit = scene_trace<STACK, false>(scene, origin, direction, ignore, distance, token, uv, nullptr);
+		if (INST && scene.packCount != 0u) hit = scene_trace_layers<STACK, false>(scene, origin, direction, ignore, ignoreLayers, distance, token, uv, hitLayers, nullptr);
+		else hit = scene_trace<STACK, false>(scene, origin, direction, ignore, distance, token, uv, nullptr); // INST without packs is a textured scene: one pack
 
 		if (!hit) break;
 
-		// PreparedScene.Interact + material.Scatter, as in shade_kernel
-		Layer layer = find_layer<INST>(scene, hitLayers);
-		const bool textured = INST && scene.textureCount != 0u;
-		vec3 infoNormal, infoShading;
-		vec2 texcoord = { 0.0f, 0.0f };
-		uint32_t materialIndex;
-
-		if (token_type(token) == ECHO_TOKEN_TYPE_TRIANGLE)
-		{
-			TriangleData triangle = load_triangle(scene, layer.info.triangleOffset + token_index(token));
-			materialIndex = layer.materialOffset + triangle.material;
-			infoNormal = triangle_normal(triangle);
-			infoShading = triangle_shading_normal(triangle, uv);
-			if (textured) texcoord = triangle_texcoord(scene, layer.info.triangleOffset + token_index(token), uv);
-		}
-		else
-		{
-			materialIndex = layer.materialOffset + __ldg(scene.sphereMaterial + layer.info.sphereOffset + token_index(token));
-			infoNormal = infoShading = sphere_normal(uv);
-			if (textured) texcoord = sphere_texcoord(uv);
-		}
-
-		vec3 position = direction * max_net(distance, kEpsilon) + origin;
-		vec3 normal = normalized(transform_direction(layer.inverse, infoNormal));
-		vec3 shadeNormal = normalized(transform_direction(layer.inverse, infoShading));
-		vec3 outgoing = -direction;
-		if (textured) apply_normal_mapping(scene, materialIndex, texcoord, shadeNormal);
-
-		MaterialRecord material = load_material(scene, materialIndex);
-		Bsdf bsdf;
-		material_scatter<INST>(scene, material, outgoing, normal, shadeNormal, bsdf, materialIndex, texcoord);
-		if (textured) resolve_material_textures(scene, materialIndex, texcoord, material); // (RGB128)material.SampleAlbedo(contact)
+		Contact contact;
+		interact<INST>(scene, token, uv, distance, hitLayers, origin, direction, contact);
+		if (INST && scene.textureCount != 0u) resolve_material_textures(scene, contact.materialIndex, contact.texcoord, contact.material); // (RGB128)material.SampleAlbedo(contact)
 
 		// Exit(): (RGB128)material.SampleAlbedo(contact) / new NormalDepth128(contact.shade.Normal, depth).ToFloat4()
 		auto leave = [&]()
 		{
-			result = kind == ECHO_EVALUATOR_ALBEDO ? make_float4(material.albedo[0], material.albedo[1], material.albedo[2], 0.0f)
-			                                       : make_float4(shadeNormal.x, shadeNormal.y, shadeNormal.z, depth);
+			result = kind == ECHO_EVALUATOR_ALBEDO ? make_float4(contact.material.albedo[0], contact.material.albedo[1], contact.material.albedo[2], 0.0f)
+			                                       : make_float4(contact.shadeNormal.x, contact.shadeNormal.y, contact.shadeNormal.z, depth);
 			exited = true;
 		};
 
 		if (!direct) { leave(); continue; }
 		if (kind == ECHO_EVALUATOR_NORMAL_DEPTH) depth += distance;
 
-		if (((KINDS_AUXILIARY >> bsdf.kind) & 1u) == 0u) { leave(); continue; } // bsdf.Count != bsdf.CountSpecular: not fully specular
+		if (((KINDS_AUXILIARY >> contact.bsdf.kind) & 1u) == 0u) { leave(); continue; } // bsdf.Count != bsdf.CountSpecular: not fully specular
 
 		vec2 sample = draw2d<STRAT>(key, strata, dimension);
 		dimension += 2u;
 
 		vec3 incident;
 		int selectedType;
-		Sampled sampled = bsdf_sample<KINDS_AUXILIARY>(bsdf, outgoing, sample, incident, selectedType);
+		Sampled sampled = bsdf_sample<KINDS_AUXILIARY>(contact.bsdf, contact.outgoing, sample, incident, selectedType);
 		if (!positive(sampled.pdf)) { leave(); continue; } // sample.NotPossible
 
 		if (!float3_equals(incident, cameraDirection)) direct = false; // compared with the CAMERA ray's direction
 		if (!divergeOnce && !direct) { leave(); continue; }
 
 		// query.SpawnTrace(incident), TraceQuery.cs:88
-		origin = position;
+		origin = contact.point.position;
 		direction = incident;
 		ignore = token;
 		ignoreLayers = hitLayers;
@@ -1983,17 +1878,10 @@ __global__ void __launch_bounds__(kBlock) tail_kernel(DeviceScene scene, EchoRen
 
 			if (packs)
 			{
-				PathLayers ignore = load_layers(paths.rayLayers[current], i);
-				PathLayers hitLayer = no_layers();
-
-				if (positive(b.z))
-				{
-					traverse_instanced<STACK, false, false>(scene, { a.x, a.y, a.z }, { a.w, b.x, b.y }, __float_as_uint(b.w), ignore.tokens, ignore.count,
-					                                        distance, token, uv, hitLayer.tokens, hitLayer.count, nullptr);
-					hit = distance < b.z;
-				}
-
-				store_layers(paths.hitLayers, i, hit ? hitLayer : no_layers());
+				PathLayers hitLayers = no_layers();
+				hit = scene_trace_layers<STACK, false>(scene, { a.x, a.y, a.z }, { a.w, b.x, b.y }, __float_as_uint(b.w), load_layers(paths.rayLayers[current], i),
+				                                       distance, token, uv, hitLayers, nullptr);
+				store_layers(paths.hitLayers, i, hit ? hitLayers : no_layers());
 			}
 			else hit = scene_trace<STACK, false>(scene, { a.x, a.y, a.z }, { a.w, b.x, b.y }, __float_as_uint(b.w), distance, token, uv, nullptr);
 
@@ -2013,18 +1901,8 @@ __global__ void __launch_bounds__(kBlock) tail_kernel(DeviceScene scene, EchoRen
 			vec3 origin = xyz(o.shadowOrigin), direction = { o.shadowOrigin.w, o.shadowDirection.x, o.shadowDirection.y };
 			float travel = o.shadowDirection.z;
 			uint32_t ignore = __float_as_uint(o.shadowDirection.w);
-			bool occluded = false;
-
-			if (packs)
-			{
-				PathLayers unusedLayers = no_layers();
-				uint32_t unusedToken = ECHO_TOKEN_EMPTY;
-				vec2 unusedUV = { 0.0f, 0.0f };
-				if (positive(travel))
-					occluded = traverse_instanced<STACK, true, false>(scene, origin, direction, ignore, o.hitLayers.tokens, o.hitLayers.count, travel, unusedToken, unusedUV,
-					                                                  unusedLayers.tokens, unusedLayers.count, nullptr);
-			}
-			else occluded = scene_occlude<STACK, false>(scene, origin, direction, ignore, travel, nullptr);
+			bool occluded = packs ? scene_occlude_layers<STACK, false>(scene, origin, direction, ignore, o.hitLayers, travel, nullptr)
+			                      : scene_occlude<STACK, false>(scene, origin, direction, ignore, travel, nullptr);
 
 			++counted[1];
 
@@ -2051,6 +1929,7 @@ __global__ void __launch_bounds__(kBlock) tail_kernel(DeviceScene scene, EchoRen
 	const int slots[9] = { STAT_TRACE_QUERIES, STAT_OCCLUDE_QUERIES, STAT_LIGHT_OCCLUSION_PASSED, STAT_LIGHT_EVALUATED_INFINITE, STAT_BOUNCE_CREATED,
 	                       STAT_BOUNCE_SPECULAR, STAT_BOUNCE_MIS, STAT_LIGHT_SAMPLED, STAT_LIGHT_OCCLUSION_CHECKED };
 
+	// spelled out rather than nine warp_add calls, which compile this kernel to a different register allocation
 #pragma unroll
 	for (int k = 0; k < 9; k++)
 	{
@@ -2079,7 +1958,6 @@ __global__ void __launch_bounds__(kBlock) naive_kernel(DeviceScene scene, EchoRe
 		const uint32_t key = paths.key[i];
 		const Strata strata = path_strata<STRAT>(params, paths, i);
 		const bool packs = INST && scene.packCount != 0u;
-		const bool textured = INST && scene.textureCount != 0u;
 		const int limit = params.bounceLimit < kNaiveBounceCap ? params.bounceLimit : kNaiveBounceCap;
 
 		rgb scatters[kNaiveBounceCap], emissions[kNaiveBounceCap];
@@ -2100,11 +1978,7 @@ __global__ void __launch_bounds__(kBlock) naive_kernel(DeviceScene scene, EchoRe
 			{
 				++traced;
 
-				if (packs)
-				{
-					traverse_instanced<STACK, false, false>(scene, origin, direction, ignore, ignoreLayers.tokens, ignoreLayers.count, distance, token, uv, hitLayers.tokens, hitLayers.count, nullptr);
-					hit = distance < kInfinity;
-				}
+				if (packs) hit = scene_trace_layers<STACK, false>(scene, origin, direction, ignore, ignoreLayers, distance, token, uv, hitLayers, nullptr);
 				else hit = scene_trace<STACK, false>(scene, origin, direction, ignore, distance, token, uv, nullptr);
 			}
 
@@ -2114,44 +1988,16 @@ __global__ void __launch_bounds__(kBlock) naive_kernel(DeviceScene scene, EchoRe
 				break;
 			}
 
-			// scene.Interact + material.Scatter, as in shade_body
-			Layer layer = find_layer<INST>(scene, hitLayers);
-			vec3 infoNormal, infoShading;
-			vec2 texcoord = { 0.0f, 0.0f };
-			uint32_t materialIndex;
-
-			if (token_type(token) == ECHO_TOKEN_TYPE_TRIANGLE)
-			{
-				TriangleData triangle = load_triangle(scene, layer.info.triangleOffset + token_index(token));
-				materialIndex = layer.materialOffset + triangle.material;
-				infoNormal = triangle_normal(triangle);
-				infoShading = triangle_shading_normal(triangle, uv);
-				if (textured) texcoord = triangle_texcoord(scene, layer.info.triangleOffset + token_index(token), uv);
-			}
-			else
-			{
-				materialIndex = layer.materialOffset + __ldg(scene.sphereMaterial + layer.info.sphereOffset + token_index(token));
-				infoNormal = infoShading = sphere_normal(uv);
-				if (textured) texcoord = sphere_texcoord(uv);
-			}
-
-			vec3 position = direction * max_net(distance, kEpsilon) + origin;
-			vec3 normal = normalized(transform_direction(layer.inverse, infoNormal));
-			vec3 shadeNormal = normalized(transform_direction(layer.inverse, infoShading));
-			vec3 outgoing = -direction;
-			if (textured) apply_normal_mapping(scene, materialIndex, texcoord, shadeNormal);
-
-			MaterialRecord material = load_material(scene, materialIndex);
-			Bsdf bsdf;
-			material_scatter<INST>(scene, material, outgoing, normal, shadeNormal, bsdf, materialIndex, texcoord);
+			Contact contact;
+			interact<INST>(scene, token, uv, distance, hitLayers, origin, direction, contact);
 
 			// `material is Emissive emissive ? emissive.Emit(contact.point, contact.outgoing) : RGB128.Black`, :42
-			rgb emission = material.type == ECHO_MATERIAL_EMISSIVE && dot(outgoing, normal) > 0.0f ? material_emission(material) : make_rgb(0.0f);
+			rgb emission = contact.material.type == ECHO_MATERIAL_EMISSIVE && dot(contact.outgoing, contact.point.normal) > 0.0f ? material_emission(contact.material) : make_rgb(0.0f);
 
 			vec2 sample = draw2d<STRAT>(key, strata, 4u + 2u * (uint32_t)depth);
 			vec3 incident;
 			int selectedType;
-			Sampled sampled = bsdf_sample<KINDS_ALL>(bsdf, outgoing, sample, incident, selectedType);
+			Sampled sampled = bsdf_sample<KINDS_ALL>(contact.bsdf, contact.outgoing, sample, incident, selectedType);
 			++bounced;
 
 			if (!positive(sampled.pdf) || is_zero(sampled.content)) // "Exit if the BSDF sample is not promising", :46
@@ -2160,11 +2006,11 @@ __global__ void __launch_bounds__(kBlock) naive_kernel(DeviceScene scene, EchoRe
 				break;
 			}
 
-			scatters[depth] = (sampled.content / sampled.pdf) * abs_bits(dot(incident, shadeNormal));
+			scatters[depth] = (sampled.content / sampled.pdf) * abs_bits(dot(incident, contact.shadeNormal));
 			emissions[depth] = emission;
 			++depth;
 
-			origin = position; // query.SpawnTrace(incident)
+			origin = contact.point.position; // query.SpawnTrace(incident)
 			direction = incident;
 			ignore = token;
 			ignoreLayers = hitLayers;
@@ -2174,6 +2020,7 @@ __global__ void __launch_bounds__(kBlock) naive_kernel(DeviceScene scene, EchoRe
 		out[i] = make4(value, 0.0f);
 	}
 
+	// both sums in one loop rather than two warp_add calls, which compile this kernel to a different register allocation
 	for (int offset = 16; offset > 0; offset >>= 1)
 	{
 		traced += __shfl_down_sync(0xFFFFFFFFu, traced, offset);
@@ -2624,7 +2471,7 @@ static uint32_t run_ahead()
 // blocks only when that window is full. The device therefore never idles between bounces waiting for a host thread to wake
 // up and launch (8 ranks x 8 pipelines share the box's host cores), and when the wavefront empties at most `runAhead`
 // surplus iterations were queued, each nine launches of kernels that find zero counts.
-template<int STACK, bool INST>
+template<int STACK, bool INST, bool STRAT>
 static bool evaluate_paths(WorkerState* state, const DeviceScene& sceneIn, const EchoRenderParams& params, uint32_t count, uint64_t& launches, cudaStream_t stream)
 {
 	PathBuffers& paths = state->paths;
@@ -2635,27 +2482,21 @@ static bool evaluate_paths(WorkerState* state, const DeviceScene& sceneIn, const
 	if (count == 0u) return true;
 	if (!check_cuda(cudaMemsetAsync(counters, 0, sizeof(uint32_t) * 64, stream), "cudaMemsetAsync(counters)")) return false;
 
-	// ECHO_DISTRIBUTION_STRATIFIED: every kernel that draws runs its stratified instantiation
-	const bool stratified = (params.evaluator & ECHO_DISTRIBUTION_STRATIFIED) != 0;
-
 	timer.start(stream);
-	if (stratified) raygen_kernel<true><<<blocks_for(count), kBlock, 0, stream>>>(sceneIn, params, count, state->pixelXY, state->sampleIndex, paths);
-	else raygen_kernel<false><<<blocks_for(count), kBlock, 0, stream>>>(sceneIn, params, count, state->pixelXY, state->sampleIndex, paths);
+	raygen_kernel<STRAT><<<blocks_for(count), kBlock, 0, stream>>>(sceneIn, params, count, state->pixelXY, state->sampleIndex, paths);
 	timer.stop(KernelTimer::RAYGEN, stream);
 	++launches;
 
 	if ((params.evaluator & ECHO_EVALUATOR_KIND_MASK) == ECHO_EVALUATOR_NAIVE)
 	{
-		if (stratified) naive_kernel<STACK, INST, true><<<blocks_for(count), kBlock, 0, stream>>>(sceneIn, params, count, paths, state->sampleOut);
-		else naive_kernel<STACK, INST, false><<<blocks_for(count), kBlock, 0, stream>>>(sceneIn, params, count, paths, state->sampleOut);
+		naive_kernel<STACK, INST, STRAT><<<blocks_for(count), kBlock, 0, stream>>>(sceneIn, params, count, paths, state->sampleOut);
 		++launches;
 		return check_cuda(cudaGetLastError(), "naive_kernel launch");
 	}
 
 	if ((params.evaluator & ECHO_EVALUATOR_KIND_MASK) != ECHO_EVALUATOR_PATH_TRACED)
 	{
-		if (stratified) auxiliary_kernel<STACK, INST, true><<<blocks_for(count), kBlock, 0, stream>>>(sceneIn, params, count, paths, state->sampleOut);
-		else auxiliary_kernel<STACK, INST, false><<<blocks_for(count), kBlock, 0, stream>>>(sceneIn, params, count, paths, state->sampleOut);
+		auxiliary_kernel<STACK, INST, STRAT><<<blocks_for(count), kBlock, 0, stream>>>(sceneIn, params, count, paths, state->sampleOut);
 		++launches;
 		return check_cuda(cudaGetLastError(), "auxiliary_kernel launch");
 	}
@@ -2695,29 +2536,23 @@ static bool evaluate_paths(WorkerState* state, const DeviceScene& sceneIn, const
 		unsigned long long* rayCounters = narrow ? nullptr : ray_counters(stream);
 		if (!narrow && !rayCounters) return false;
 
+		// one-thread-per-ray for narrow and counted passes, persistent otherwise; `io` names the instantiation (with or without packs)
+		auto extend = [&](auto io)
+		{
+			constexpr bool PACKS = std::is_same<decltype(io), ExtendLayersIO>::value;
+			if (counted) extend_narrow_kernel<STACK, PACKS, true><<<blocks, kBlock, 0, stream>>>(scene, io, rayCount, paths.stats);
+			else if (narrow) extend_narrow_kernel<STACK, PACKS, false><<<blocks, kBlock, 0, stream>>>(scene, io, rayCount, paths.stats);
+			else
+			{
+				const int grid = persistent_grid((const void*)extend_kernel<STACK, PACKS>);
+				extend_kernel<STACK, PACKS><<<std::min<unsigned int>(blocks, (unsigned int)grid), kTraverseBlock, 0, stream>>>(scene, io, rayCount, rayCounters);
+			}
+		};
+
 		timer.start(stream);
 		ExtendIO extendIO = { paths.rayQueue[current], paths.hitQueue };
-
-		if (packs && !narrow)
-		{
-			const int layersGrid = persistent_grid((const void*)extend_layers_kernel<STACK>);
-			ExtendLayersIO layersIO;
-			layersIO.rays = extendIO.rays;
-			layersIO.hits = extendIO.hits;
-			layersIO.rayLayers = paths.rayLayers[current];
-			layersIO.hitLayers = paths.hitLayers;
-			extend_layers_kernel<STACK><<<std::min<unsigned int>(blocks, (unsigned int)layersGrid), kTraverseBlock, 0, stream>>>(scene, layersIO, rayCount, rayCounters);
-		}
-		else if (packs && counted) extend_instanced_kernel<STACK, true><<<blocks, kBlock, 0, stream>>>(scene, extendIO, paths.rayLayers[current], paths.hitLayers, rayCount, paths.stats);
-		else if (packs) extend_instanced_kernel<STACK, false><<<blocks, kBlock, 0, stream>>>(scene, extendIO, paths.rayLayers[current], paths.hitLayers, rayCount, paths.stats);
-		else if (counted) extend_narrow_kernel<STACK, true><<<blocks, kBlock, 0, stream>>>(scene, extendIO, rayCount, paths.stats);
-		else if (narrow) extend_narrow_kernel<STACK, false><<<blocks, kBlock, 0, stream>>>(scene, extendIO, rayCount, paths.stats);
-		else
-		{
-			const int extendGrid = persistent_grid((const void*)extend_kernel<STACK>);
-			extend_kernel<STACK><<<std::min<unsigned int>(blocks, (unsigned int)extendGrid), kTraverseBlock, 0, stream>>>(scene, extendIO, rayCount, rayCounters);
-		}
-
+		if (packs) extend(ExtendLayersIO{ extendIO, paths.rayLayers[current], paths.hitLayers });
+		else extend(extendIO);
 		timer.stop(KernelTimer::EXTEND, stream);
 
 		timer.start(stream);
@@ -2779,8 +2614,7 @@ static bool evaluate_paths(WorkerState* state, const DeviceScene& sceneIn, const
 		// the tail: finish the few paths that are left in one launch (it traces for itself: the hits of k are simply not used)
 		if (!timer.enabled && !counted && bound < tailLimit)
 		{
-			if (stratified) tail_kernel<STACK, INST, true><<<blocks, kBlock, 0, stream>>>(scene, iterationParams, activeCount, paths, current);
-			else tail_kernel<STACK, INST, false><<<blocks, kBlock, 0, stream>>>(scene, iterationParams, activeCount, paths, current);
+			tail_kernel<STACK, INST, STRAT><<<blocks, kBlock, 0, stream>>>(scene, iterationParams, activeCount, paths, current);
 			if (!check_cuda(cudaGetLastError(), "tail_kernel launch")) return false;
 			++launches;
 			break;
@@ -2792,8 +2626,7 @@ static bool evaluate_paths(WorkerState* state, const DeviceScene& sceneIn, const
 
 		if (counted)
 		{
-			if (stratified) shade_counted_kernel<INST, true><<<blocks, kBlock, 0, stream>>>(scene, iterationParams, activeCount, paths, current);
-			else shade_counted_kernel<INST, false><<<blocks, kBlock, 0, stream>>>(scene, iterationParams, activeCount, paths, current);
+			shade_counted_kernel<INST, STRAT><<<blocks, kBlock, 0, stream>>>(scene, iterationParams, activeCount, paths, current);
 			++launches;
 		}
 
@@ -2803,12 +2636,8 @@ static bool evaluate_paths(WorkerState* state, const DeviceScene& sceneIn, const
 		if (classRays[CLASS_VALUE] != 0u)                                                                                                                \
 		{                                                                                                                                                \
 			timer.start(stream);                                                                                                                         \
-			if (stratified)                                                                                                                              \
-				shade_kernel<CLASS_VALUE, KINDS_VALUE, INST, true><<<blocks_for(classRays[CLASS_VALUE]), kBlock, 0, stream>>>(scene, iterationParams,       \
-				                                                             paths.classQueue[CLASS_VALUE], classCounts + CLASS_VALUE, paths, current);     \
-			else                                                                                                                                         \
-				shade_kernel<CLASS_VALUE, KINDS_VALUE, INST, false><<<blocks_for(classRays[CLASS_VALUE]), kBlock, 0, stream>>>(scene, iterationParams,      \
-				                                                             paths.classQueue[CLASS_VALUE], classCounts + CLASS_VALUE, paths, current);     \
+			shade_kernel<CLASS_VALUE, KINDS_VALUE, INST, STRAT><<<blocks_for(classRays[CLASS_VALUE]), kBlock, 0, stream>>>(scene, iterationParams,       \
+			                                                              paths.classQueue[CLASS_VALUE], classCounts + CLASS_VALUE, paths, current);     \
 			timer.stop(SLOT, stream);                                                                                                                    \
 			++launches;                                                                                                                                  \
 		}
@@ -2831,29 +2660,22 @@ static bool evaluate_paths(WorkerState* state, const DeviceScene& sceneIn, const
 			unsigned long long* rayCounters = narrow ? nullptr : ray_counters(stream);
 			if (!narrow && !rayCounters) return false;
 
+			auto shadow = [&](auto io)
+			{
+				constexpr bool PACKS = std::is_same<decltype(io), ShadowLayersIO>::value;
+				if (counted) shadow_narrow_kernel<STACK, PACKS, true><<<shadowBlocks, kBlock, 0, stream>>>(scene, io, counters + COUNTER_SHADOW, paths.stats);
+				else if (narrow) shadow_narrow_kernel<STACK, PACKS, false><<<shadowBlocks, kBlock, 0, stream>>>(scene, io, counters + COUNTER_SHADOW, paths.stats);
+				else
+				{
+					const int grid = persistent_grid((const void*)shadow_kernel<STACK, PACKS>);
+					shadow_kernel<STACK, PACKS><<<std::min<unsigned int>(shadowBlocks, (unsigned int)grid), kTraverseBlock, 0, stream>>>(scene, io, counters + COUNTER_SHADOW, rayCounters, paths.stats);
+				}
+			};
+
 			timer.start(stream);
 			ShadowIO shadowIO = { paths.shadowQueue, paths.shadowValue, paths.result, 0u };
-
-			if (packs && !narrow)
-			{
-				const int layersGrid = persistent_grid((const void*)shadow_layers_kernel<STACK>);
-				ShadowLayersIO layersIO;
-				layersIO.rays = shadowIO.rays;
-				layersIO.values = shadowIO.values;
-				layersIO.result = shadowIO.result;
-				layersIO.passed = 0u;
-				layersIO.shadowLayers = paths.shadowLayers;
-				shadow_layers_kernel<STACK><<<std::min<unsigned int>(shadowBlocks, (unsigned int)layersGrid), kTraverseBlock, 0, stream>>>(scene, layersIO, counters + COUNTER_SHADOW, rayCounters, paths.stats);
-			}
-			else if (packs && counted) shadow_instanced_kernel<STACK, true><<<shadowBlocks, kBlock, 0, stream>>>(scene, shadowIO, paths.shadowLayers, counters + COUNTER_SHADOW, paths.stats);
-			else if (packs) shadow_instanced_kernel<STACK, false><<<shadowBlocks, kBlock, 0, stream>>>(scene, shadowIO, paths.shadowLayers, counters + COUNTER_SHADOW, paths.stats);
-			else if (counted) shadow_narrow_kernel<STACK, true><<<shadowBlocks, kBlock, 0, stream>>>(scene, shadowIO, counters + COUNTER_SHADOW, paths.stats);
-			else if (narrow) shadow_narrow_kernel<STACK, false><<<shadowBlocks, kBlock, 0, stream>>>(scene, shadowIO, counters + COUNTER_SHADOW, paths.stats);
-			else
-			{
-				const int shadowGrid = persistent_grid((const void*)shadow_kernel<STACK>);
-				shadow_kernel<STACK><<<std::min<unsigned int>(shadowBlocks, (unsigned int)shadowGrid), kTraverseBlock, 0, stream>>>(scene, shadowIO, counters + COUNTER_SHADOW, rayCounters, paths.stats);
-			}
+			if (packs) shadow(ShadowLayersIO{ shadowIO, paths.shadowLayers });
+			else shadow(shadowIO);
 
 			timer.stop(KernelTimer::SHADOW, stream);
 			++launches;
@@ -2876,15 +2698,25 @@ static bool evaluate_paths(WorkerState* state, const DeviceScene& sceneIn, const
 	return check_cuda(cudaGetLastError(), "finish_kernel launch");
 }
 
+// the instantiation a call needs: the tree's stack class, the full-featured shading kernels for packs or textures, and
+// with ECHO_DISTRIBUTION_STRATIFIED the stratified instantiation of every kernel that draws
+template<int STACK>
+static bool evaluate_paths_stack(WorkerState* state, const DeviceScene& scene, const EchoRenderParams& params, uint32_t count, uint64_t& launches, cudaStream_t stream)
+{
+	const bool instanced = scene.packCount != 0u || scene.textureCount != 0u;
+	const bool stratified = (params.evaluator & ECHO_DISTRIBUTION_STRATIFIED) != 0;
+
+	if (instanced) return stratified ? evaluate_paths<STACK, true, true>(state, scene, params, count, launches, stream) : evaluate_paths<STACK, true, false>(state, scene, params, count, launches, stream);
+	return stratified ? evaluate_paths<STACK, false, true>(state, scene, params, count, launches, stream) : evaluate_paths<STACK, false, false>(state, scene, params, count, launches, stream);
+}
+
 static bool evaluate_paths_dispatch(WorkerState* state, const DeviceScene& scene, const EchoRenderParams& params, uint32_t count, uint64_t& launches, cudaStream_t stream)
 {
-	bool instanced = scene.packCount != 0u || scene.textureCount != 0u; // the full-featured shading kernels
-
 	switch (stack_class(scene.maxDepth))
 	{
-		case 0: return instanced ? evaluate_paths<48, true>(state, scene, params, count, launches, stream) : evaluate_paths<48, false>(state, scene, params, count, launches, stream);
-		case 1: return instanced ? evaluate_paths<96, true>(state, scene, params, count, launches, stream) : evaluate_paths<96, false>(state, scene, params, count, launches, stream);
-		case 2: return instanced ? evaluate_paths<192, true>(state, scene, params, count, launches, stream) : evaluate_paths<192, false>(state, scene, params, count, launches, stream);
+		case 0: return evaluate_paths_stack<48>(state, scene, params, count, launches, stream);
+		case 1: return evaluate_paths_stack<96>(state, scene, params, count, launches, stream);
+		case 2: return evaluate_paths_stack<192>(state, scene, params, count, launches, stream);
 		default: set_error("QBVH deeper than 63 quad levels is not supported"); return false;
 	}
 }

@@ -47,23 +47,7 @@ __global__ void __launch_bounds__(kTraceBlock) trace_batch_kernel(DeviceScene sc
 		hits[i] = out;
 	}
 
-	if (COUNT)
-	{
-		// warp-level reduction, then one atomic per warp per counter
-		for (int offset = 16; offset > 0; offset >>= 1)
-		{
-			local.nodes += __shfl_down_sync(0xFFFFFFFFu, local.nodes, offset);
-			local.triangles += __shfl_down_sync(0xFFFFFFFFu, local.triangles, offset);
-			local.spheres += __shfl_down_sync(0xFFFFFFFFu, local.spheres, offset);
-		}
-
-		if ((threadIdx.x & 31) == 0)
-		{
-			atomicAdd(counts + 0, (unsigned long long)local.nodes);
-			atomicAdd(counts + 1, (unsigned long long)local.triangles);
-			atomicAdd(counts + 2, (unsigned long long)local.spheres);
-		}
-	}
+	if (COUNT) visit_flush(counts, 0, local);
 }
 
 template<int STACK, bool COUNT>
@@ -85,22 +69,7 @@ __global__ void __launch_bounds__(kTraceBlock) occlude_batch_kernel(DeviceScene 
 		occluded[i] = result ? 1 : 0;
 	}
 
-	if (COUNT)
-	{
-		for (int offset = 16; offset > 0; offset >>= 1)
-		{
-			local.nodes += __shfl_down_sync(0xFFFFFFFFu, local.nodes, offset);
-			local.triangles += __shfl_down_sync(0xFFFFFFFFu, local.triangles, offset);
-			local.spheres += __shfl_down_sync(0xFFFFFFFFu, local.spheres, offset);
-		}
-
-		if ((threadIdx.x & 31) == 0)
-		{
-			atomicAdd(counts + 0, (unsigned long long)local.nodes);
-			atomicAdd(counts + 1, (unsigned long long)local.triangles);
-			atomicAdd(counts + 2, (unsigned long long)local.spheres);
-		}
-	}
+	if (COUNT) visit_flush(counts, 0, local);
 }
 
 // AoS EchoRay in (two 128-bit loads), EchoHit out (one 128-bit store) / one byte per occlusion query
