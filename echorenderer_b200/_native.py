@@ -37,6 +37,12 @@ EXPORTS = [
     "echo_b200_scene_create_multi", "echo_b200_scene_gpu_count", "echo_b200_build_packs", "echo_b200_scene_build_packs", "echo_b200_debug_last_pack_build",
 ]
 
+# every symbol include/echo_b200_query.h declares: the batched PreparedScene queries besides Trace / Occlude
+QUERY_EXPORTS = [
+    "echo_b200_interact_batch", "echo_b200_scatter_sample_batch", "echo_b200_scatter_evaluate_batch", "echo_b200_light_pick_batch",
+    "echo_b200_light_mass_batch", "echo_b200_light_sample_batch", "echo_b200_light_pdf_batch", "echo_b200_evaluate_infinite_batch",
+]
+
 
 def library():
     global _lib
@@ -99,6 +105,14 @@ def library():
                                   ctypes.POINTER(u32), ctypes.POINTER(f32)],
         "echo_b200_scene_build_packs": [p, p, u32, ctypes.POINTER(u32), ctypes.POINTER(u32), ctypes.POINTER(u32), ctypes.POINTER(f32)],
         "echo_b200_debug_last_pack_build": [p],
+        "echo_b200_interact_batch": [p, p, p, p, u64, p],
+        "echo_b200_scatter_sample_batch": [p, p, p, p, p, u64, p],
+        "echo_b200_scatter_evaluate_batch": [p, p, p, p, p, u64, p],
+        "echo_b200_light_pick_batch": [p, p, p, u64, p, p, p],
+        "echo_b200_light_mass_batch": [p, p, p, p, u64, p],
+        "echo_b200_light_sample_batch": [p, p, p, p, p, u64, p],
+        "echo_b200_light_pdf_batch": [p, p, p, p, p, u64, p],
+        "echo_b200_evaluate_infinite_batch": [p, p, u64, i32, p],
     }
 
     for name, argtypes in signatures.items():

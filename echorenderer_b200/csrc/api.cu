@@ -449,6 +449,7 @@ int32_t echo_b200_scene_destroy(EchoScene* scene)
 
 	if (scene->tilesOut) cudaFree(scene->tilesOut);
 	for (void* pointer : scene->hierarchyScratch) if (pointer) cudaFree(pointer);
+	for (void* pointer : scene->queryScratch) if (pointer) cudaFree(pointer);
 	if (scene->stream) cudaStreamDestroy(scene->stream);
 	delete scene;
 	return ECHO_B200_OK;
@@ -1171,6 +1172,345 @@ int32_t echo_b200_occlude_batch_hierarchy(EchoScene* scene, const EchoRay* rays,
 		uint64_t first = n * g / devices;
 		return hierarchy_host(target, rays + first, ignore ? ignore + first : nullptr, n * (g + 1) / devices - first, nullptr, nullptr, occluded + first);
 	});
+}
+
+// ---- batched PreparedScene queries (include/echo_b200_query.h) ----
+namespace
+{
+
+// the arrays of one query call by role, host pointers (null: absent) and bytes per query; outputs from SLOT_OUT on
+enum QuerySlot : int { SLOT_RAYS, SLOT_HITS, SLOT_POINTS, SLOT_TOKENS, SLOT_LAYERS, SLOT_VALUES, SLOT_OUT, SLOT_OUT_LAYERS, SLOT_OUT_PMF, SLOT_COUNT };
+static_assert(SLOT_COUNT == EchoScene::kQuerySlots, "one scratch buffer per slot");
+
+struct QueryCall
+{
+	int op = QUERY_INTERACT;
+	const void* host[SLOT_COUNT] = {};
+	size_t bytes[SLOT_COUNT] = {};
+	int32_t direct = 0;
+
+	void set(int slot, const void* pointer, size_t size)
+	{
+		host[slot] = pointer;
+		bytes[slot] = size;
+	}
+
+	QueryCall from(uint64_t first) const // the same call on the queries from `first` on
+	{
+		QueryCall call = *this;
+		for (int s = 0; s < SLOT_COUNT; s++)
+			if (host[s]) call.host[s] = static_cast<const char*>(host[s]) + first * bytes[s];
+		return call;
+	}
+};
+
+// One upload, one launch, one download into grow-only scratch, like hierarchy_host. The caller has validated the inputs.
+int32_t query_host(EchoScene* scene, const QueryCall& call, uint64_t n)
+{
+	if (n == 0) return ECHO_B200_OK;
+	DeviceGuard guard(scene->device);
+	if (!guard.ok) return ECHO_B200_ERR_NO_DEVICE;
+	std::lock_guard<std::mutex> turn(scene->compute);
+
+	cudaStream_t stream = scene->stream;
+	void* device[SLOT_COUNT] = {};
+	bool ok = true;
+
+	for (int s = 0; ok && s < SLOT_COUNT; s++)
+	{
+		if (!call.host[s]) continue;
+		const size_t bytes = call.bytes[s] * n;
+
+		if (scene->queryBytes[s] < bytes)
+		{
+			if (scene->queryScratch[s]) cudaFree(scene->queryScratch[s]);
+			scene->queryScratch[s] = nullptr;
+			scene->queryBytes[s] = 0;
+			ok = check_cuda(cudaMalloc(&scene->queryScratch[s], bytes), "cudaMalloc(scene query)");
+			if (!ok) break;
+			scene->queryBytes[s] = bytes;
+		}
+
+		device[s] = scene->queryScratch[s];
+		if (s < SLOT_OUT) ok = check_cuda(cudaMemcpyAsync(device[s], call.host[s], bytes, cudaMemcpyHostToDevice, stream), "cudaMemcpyAsync(query inputs)");
+	}
+
+	if (ok)
+	{
+		QueryBuffers buffers = { static_cast<const EchoRay*>(device[SLOT_RAYS]), static_cast<const EchoHit*>(device[SLOT_HITS]),
+		                         static_cast<const EchoSurface*>(device[SLOT_POINTS]), static_cast<const uint32_t*>(device[SLOT_TOKENS]),
+		                         static_cast<const EchoTokenHierarchy*>(device[SLOT_LAYERS]), static_cast<const float*>(device[SLOT_VALUES]), device[SLOT_OUT],
+		                         static_cast<EchoTokenHierarchy*>(device[SLOT_OUT_LAYERS]), static_cast<float*>(device[SLOT_OUT_PMF]), call.direct };
+		ok = launch_query(scene->d, call.op, buffers, n, stream);
+	}
+
+	for (int s = SLOT_OUT; ok && s < SLOT_COUNT; s++)
+		if (call.host[s]) ok = check_cuda(cudaMemcpyAsync(const_cast<void*>(call.host[s]), device[s], call.bytes[s] * n, cudaMemcpyDeviceToHost, stream), "cudaMemcpyAsync(query outputs)");
+
+	ok = ok && check_cuda(cudaStreamSynchronize(stream), "scene query");
+	if (!ok) cudaStreamSynchronize(stream); // copies queued before the failure must not outlive the caller's buffers
+	return ok ? ECHO_B200_OK : ECHO_B200_ERR_CUDA;
+}
+
+// one contiguous range of the batch per device of a multi-device scene, as echo_b200_trace_batch_hierarchy cuts it
+int32_t query_run(EchoScene* scene, const QueryCall& call, uint64_t n)
+{
+	if (scene->replicas.empty()) return query_host(scene, call, n);
+	const uint64_t devices = 1 + scene->replicas.size();
+	return fan_out(scene, [&](EchoScene* target, size_t g)
+	{
+		uint64_t first = n * g / devices;
+		return query_host(target, call.from(first), n * (g + 1) / devices - first);
+	});
+}
+
+// ---- host-side validation of the tokens, layers and values a query takes from outside the library (echo_b200_query.h) ----
+
+bool all_finite(const float* values, int count)
+{
+	for (int i = 0; i < count; i++)
+		if (!std::isfinite(values[i])) return false;
+	return true;
+}
+
+bool unit_direction(const float* v)
+{
+	if (!all_finite(v, 3)) return false;
+	double length = std::sqrt((double)v[0] * v[0] + (double)v[1] * v[1] + (double)v[2] * v[2]);
+	return std::fabs(length - 1.0) <= 1e-3;
+}
+
+uint32_t token_kind(uint32_t token) { return token >> ECHO_TOKEN_INDEX_BITS; }
+uint32_t token_number(uint32_t token) { return token & ((1u << ECHO_TOKEN_INDEX_BITS) - 1u); }
+
+// FindLayer on the host copies of the packs and placements: the pack hierarchy i ends in and the swatch offset it selects.
+// Returns why the hierarchy is refused, or an empty string.
+std::string check_layers(const EchoScene* scene, const EchoTokenHierarchy* layers, uint64_t i, EchoPack& pack, uint32_t& materialOffset)
+{
+	if (scene->packs.empty())
+	{
+		pack = EchoPack{};
+		pack.triangleCount = (uint32_t)scene->triangles.size();
+		pack.sphereCount = (uint32_t)scene->spheres.size();
+		pack.pointLightCount = (uint32_t)scene->pointLights.size();
+	}
+	else pack = scene->packs[0];
+
+	materialOffset = pack.materialOffset;
+	if (!layers || layers[i].instanceCount == 0u) return "";
+	if (scene->packs.empty()) return "instance layers on a scene without packs";
+	if (layers[i].instanceCount > ECHO_MAX_INSTANCE_LAYERS) return "more than ECHO_MAX_INSTANCE_LAYERS instance layers";
+
+	for (uint32_t k = 0; k < layers[i].instanceCount; k++)
+	{
+		uint32_t token = layers[i].instances[k];
+		if (token_kind(token) != ECHO_TOKEN_TYPE_INSTANCE || token_number(token) >= pack.instanceCount)
+			return "layer " + std::to_string(k) + " is not an instance of its parent pack";
+		const EchoInstance& instance = scene->instances[pack.instanceOffset + token_number(token)];
+		materialOffset = instance.materialOffset;
+		pack = scene->packs[instance.pack];
+	}
+
+	return "";
+}
+
+std::string check_hit(const EchoScene* scene, const EchoRay& ray, const EchoHit& hit, const EchoPack& pack, uint32_t materialOffset)
+{
+	if (!all_finite(ray.origin, 3) || !unit_direction(ray.direction)) return "the ray needs a finite origin and a unit direction";
+	if (hit.token == ECHO_TOKEN_EMPTY) return "";
+	if (!std::isfinite(hit.distance) || !all_finite(hit.uv, 2)) return "hit distance or uv is not finite";
+
+	const uint32_t index = token_number(hit.token);
+	const float x = hit.uv[0], y = hit.uv[1];
+	uint32_t material;
+
+	if (token_kind(hit.token) == ECHO_TOKEN_TYPE_TRIANGLE)
+	{
+		if (index >= pack.triangleCount) return "triangle index out of range for its pack";
+		if (!(x >= 0.0f && x <= 1.0f && y >= 0.0f && y <= 1.0f)) return "triangle hit uv outside [0, 1]";
+		material = scene->triangles[pack.triangleOffset + index].material;
+	}
+	else if (token_kind(hit.token) == ECHO_TOKEN_TYPE_SPHERE)
+	{
+		if (index >= pack.sphereCount) return "sphere index out of range for its pack";
+		// x = sin(theta), plus 3 behind the sphere; sin(theta) = point.x / sqrt(r^2 - y^2) may pass 1 by rounding near the poles
+		if (!(y >= -1.0f && y <= 1.0f && x >= -1.5f && x <= 4.5f)) return "sphere hit uv outside the encoding of SphereEntity";
+		material = scene->spheres[pack.sphereOffset + index].material;
+	}
+	else return "hit token is neither a triangle, a sphere nor ECHO_TOKEN_EMPTY";
+
+	if ((uint64_t)materialOffset + material >= scene->materials.size()) return "the hit's material index is out of range";
+	return "";
+}
+
+std::string check_light(const EchoScene* scene, uint32_t token, const EchoPack& pack)
+{
+	if (token == ECHO_TOKEN_EMPTY) return "";
+	const uint32_t index = token_number(token);
+
+	if (token_kind(token) == ECHO_TOKEN_TYPE_LIGHT)
+	{
+		const uint32_t lightType = index >> ECHO_LIGHT_INDEX_BITS, lightIndex = index & ((1u << ECHO_LIGHT_INDEX_BITS) - 1u);
+		if (lightType == ECHO_LIGHT_TYPE_INFINITE || lightType == ECHO_LIGHT_TYPE_INFINITE_DELTA)
+			return lightIndex < scene->infiniteLights.size() ? "" : "infinite light index out of range";
+		if (lightType == ECHO_LIGHT_TYPE_POINT) return lightIndex < pack.pointLightCount ? "" : "point light index out of range for its pack";
+		return "unknown light type";
+	}
+
+	uint32_t material;
+
+	if (token_kind(token) == ECHO_TOKEN_TYPE_TRIANGLE)
+	{
+		if (index >= pack.triangleCount) return "triangle emitter index out of range for its pack";
+		material = scene->triangles[pack.triangleOffset + index].material;
+	}
+	else if (token_kind(token) == ECHO_TOKEN_TYPE_SPHERE)
+	{
+		if (index >= pack.sphereCount) return "sphere emitter index out of range for its pack";
+		material = scene->spheres[pack.sphereOffset + index].material;
+	}
+	else return "light token is neither a light, a triangle, a sphere nor ECHO_TOKEN_EMPTY";
+
+	if ((uint64_t)pack.materialOffset + material >= scene->materials.size()) return "the emitter's material index is out of range";
+	return "";
+}
+
+int32_t refuse(const char* call, uint64_t i, const std::string& why) { return fail(ECHO_B200_ERR_INVALID, (std::string(call) + ": query " + std::to_string(i) + ": " + why).c_str()); }
+
+// interact / scatter_sample / scatter_evaluate: `values` holds `valueCount` floats per query (2: samples, 3: an incident direction)
+int32_t contact_query(EchoScene* scene, const char* name, int op, const EchoRay* rays, const EchoHit* hits, const EchoTokenHierarchy* layers,
+                      const float* values, int valueCount, uint64_t n, void* out, size_t outBytes)
+{
+	if (!require_renderable(scene)) return ECHO_B200_ERR_INVALID;
+	if (n == 0) return ECHO_B200_OK;
+	if (!rays || !hits || !out || (valueCount && !values)) return fail(ECHO_B200_ERR_INVALID, (std::string(name) + ": null buffer").c_str());
+
+	for (uint64_t i = 0; i < n; i++)
+	{
+		EchoPack pack;
+		uint32_t materialOffset;
+		std::string why = check_layers(scene, layers, i, pack, materialOffset);
+		if (why.empty()) why = check_hit(scene, rays[i], hits[i], pack, materialOffset);
+		if (why.empty() && valueCount == 2 && !all_finite(values + i * 2, 2)) why = "samples are not finite";
+		if (why.empty() && valueCount == 3 && !unit_direction(values + i * 3)) why = "the incident direction is not a finite unit vector";
+		if (!why.empty()) return refuse(name, i, why);
+	}
+
+	QueryCall call;
+	call.op = op;
+	call.set(SLOT_RAYS, rays, sizeof(EchoRay));
+	call.set(SLOT_HITS, hits, sizeof(EchoHit));
+	if (layers) call.set(SLOT_LAYERS, layers, sizeof(EchoTokenHierarchy));
+	if (valueCount) call.set(SLOT_VALUES, values, sizeof(float) * valueCount);
+	call.set(SLOT_OUT, out, outBytes);
+	return query_run(scene, call, n);
+}
+
+// mass / sample / pdf of light tokens seen from surfaces; `values` as above
+int32_t light_query(EchoScene* scene, const char* name, int op, const uint32_t* tokens, const EchoTokenHierarchy* layers, const EchoSurface* points,
+                    const float* values, int valueCount, uint64_t n, void* out, size_t outBytes)
+{
+	if (!require_committed(scene)) return ECHO_B200_ERR_INVALID;
+	if (n == 0) return ECHO_B200_OK;
+	if (!tokens || !points || !out || (valueCount && !values)) return fail(ECHO_B200_ERR_INVALID, (std::string(name) + ": null buffer").c_str());
+
+	for (uint64_t i = 0; i < n; i++)
+	{
+		EchoPack pack;
+		uint32_t materialOffset;
+		std::string why = check_layers(scene, layers, i, pack, materialOffset);
+		if (why.empty()) why = check_light(scene, tokens[i], pack);
+		if (why.empty() && (!all_finite(points[i].position, 3) || !all_finite(points[i].normal, 3))) why = "the surface is not finite";
+		if (why.empty() && valueCount == 2 && !all_finite(values + i * 2, 2)) why = "samples are not finite";
+		if (why.empty() && valueCount == 3 && !unit_direction(values + i * 3)) why = "the incident direction is not a finite unit vector";
+		if (!why.empty()) return refuse(name, i, why);
+	}
+
+	QueryCall call;
+	call.op = op;
+	call.set(SLOT_TOKENS, tokens, sizeof(uint32_t));
+	if (layers) call.set(SLOT_LAYERS, layers, sizeof(EchoTokenHierarchy));
+	call.set(SLOT_POINTS, points, sizeof(EchoSurface));
+	if (valueCount) call.set(SLOT_VALUES, values, sizeof(float) * valueCount);
+	call.set(SLOT_OUT, out, outBytes);
+	return query_run(scene, call, n);
+}
+
+} // namespace
+
+int32_t echo_b200_interact_batch(EchoScene* scene, const EchoRay* rays, const EchoHit* hits, const EchoTokenHierarchy* hitLayers, uint64_t n, EchoContact* out)
+{
+	return contact_query(scene, "echo_b200_interact_batch", QUERY_INTERACT, rays, hits, hitLayers, nullptr, 0, n, out, sizeof(EchoContact));
+}
+
+int32_t echo_b200_scatter_sample_batch(EchoScene* scene, const EchoRay* rays, const EchoHit* hits, const EchoTokenHierarchy* hitLayers, const float* samples2,
+                                       uint64_t n, EchoScatter* out)
+{
+	return contact_query(scene, "echo_b200_scatter_sample_batch", QUERY_SCATTER_SAMPLE, rays, hits, hitLayers, samples2, 2, n, out, sizeof(EchoScatter));
+}
+
+int32_t echo_b200_scatter_evaluate_batch(EchoScene* scene, const EchoRay* rays, const EchoHit* hits, const EchoTokenHierarchy* hitLayers, const float* incident3,
+                                         uint64_t n, float* outRGBA)
+{
+	return contact_query(scene, "echo_b200_scatter_evaluate_batch", QUERY_SCATTER_EVALUATE, rays, hits, hitLayers, incident3, 3, n, outRGBA, sizeof(float) * 4);
+}
+
+int32_t echo_b200_light_pick_batch(EchoScene* scene, const EchoSurface* points, const float* samples1, uint64_t n, uint32_t* tokens, EchoTokenHierarchy* layers, float* pmf)
+{
+	const char* name = "echo_b200_light_pick_batch";
+	if (!require_committed(scene)) return ECHO_B200_ERR_INVALID;
+	if (n == 0) return ECHO_B200_OK;
+	if (!points || !samples1 || !tokens || !pmf) return fail(ECHO_B200_ERR_INVALID, "echo_b200_light_pick_batch: null buffer");
+
+	for (uint64_t i = 0; i < n; i++)
+	{
+		if (!all_finite(points[i].position, 3) || !all_finite(points[i].normal, 3)) return refuse(name, i, "the surface is not finite");
+		if (!std::isfinite(samples1[i])) return refuse(name, i, "the sample is not finite");
+	}
+
+	QueryCall call;
+	call.op = QUERY_PICK;
+	call.set(SLOT_POINTS, points, sizeof(EchoSurface));
+	call.set(SLOT_VALUES, samples1, sizeof(float));
+	call.set(SLOT_OUT, tokens, sizeof(uint32_t));
+	if (layers) call.set(SLOT_OUT_LAYERS, layers, sizeof(EchoTokenHierarchy));
+	call.set(SLOT_OUT_PMF, pmf, sizeof(float));
+	return query_run(scene, call, n);
+}
+
+int32_t echo_b200_light_mass_batch(EchoScene* scene, const uint32_t* tokens, const EchoTokenHierarchy* layers, const EchoSurface* points, uint64_t n, float* pmf)
+{
+	return light_query(scene, "echo_b200_light_mass_batch", QUERY_MASS, tokens, layers, points, nullptr, 0, n, pmf, sizeof(float));
+}
+
+int32_t echo_b200_light_sample_batch(EchoScene* scene, const uint32_t* tokens, const EchoTokenHierarchy* layers, const EchoSurface* points, const float* samples2,
+                                     uint64_t n, EchoLightSample* out)
+{
+	return light_query(scene, "echo_b200_light_sample_batch", QUERY_SAMPLE, tokens, layers, points, samples2, 2, n, out, sizeof(EchoLightSample));
+}
+
+int32_t echo_b200_light_pdf_batch(EchoScene* scene, const uint32_t* tokens, const EchoTokenHierarchy* layers, const EchoSurface* points, const float* incident3,
+                                  uint64_t n, float* pdf)
+{
+	return light_query(scene, "echo_b200_light_pdf_batch", QUERY_PDF, tokens, layers, points, incident3, 3, n, pdf, sizeof(float));
+}
+
+int32_t echo_b200_evaluate_infinite_batch(EchoScene* scene, const float* directions3, uint64_t n, int32_t direct, float* outRGB3)
+{
+	const char* name = "echo_b200_evaluate_infinite_batch";
+	if (!require_committed(scene)) return ECHO_B200_ERR_INVALID;
+	if (n == 0) return ECHO_B200_OK;
+	if (!directions3 || !outRGB3) return fail(ECHO_B200_ERR_INVALID, "echo_b200_evaluate_infinite_batch: null buffer");
+
+	for (uint64_t i = 0; i < n; i++)
+		if (!unit_direction(directions3 + i * 3)) return refuse(name, i, "the direction is not a finite unit vector");
+
+	QueryCall call;
+	call.op = QUERY_INFINITE;
+	call.direct = direct;
+	call.set(SLOT_VALUES, directions3, sizeof(float) * 3);
+	call.set(SLOT_OUT, outRGB3, sizeof(float) * 3);
+	return query_run(scene, call, n);
 }
 
 int32_t echo_b200_trace_batch_device(EchoScene* scene, const EchoRay* rays, uint64_t n, EchoHit* hits, void* stream)

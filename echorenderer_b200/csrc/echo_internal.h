@@ -6,6 +6,7 @@
 #include <string>
 #include <vector>
 
+#include "../../include/echo_b200_query.h"
 #include "echo_scene.cuh"
 
 namespace echo
@@ -70,6 +71,24 @@ bool render_tiles(RenderState* state, const DeviceScene& scene, const EchoRender
                   float4* tilesOut, float4* frame, EchoStats* stats, cudaStream_t stream);
 
 bool launch_frame_resolve(float4* frame, int32_t width, int32_t height, cudaStream_t stream);
+
+// render.cu: the batched PreparedScene queries of echo_b200_query.h, one thread per query over device buffers, in the instantiation
+// the renderer picks for `scene`. Inputs must have passed the host-side validation of api.cu.
+enum QueryOp : int { QUERY_INTERACT, QUERY_SCATTER_SAMPLE, QUERY_SCATTER_EVALUATE, QUERY_PICK, QUERY_MASS, QUERY_SAMPLE, QUERY_PDF, QUERY_INFINITE };
+struct QueryBuffers
+{
+	const EchoRay* rays;               // interact, scatter
+	const EchoHit* hits;               // interact, scatter
+	const EchoSurface* points;         // light queries
+	const uint32_t* tokens;            // mass, sample, pdf
+	const EchoTokenHierarchy* layers;  // hit layers / light layers (null: empty hierarchies)
+	const float* values;               // samples1, samples2, incident3 or directions3
+	void* out;                         // EchoContact, EchoScatter, float4, uint32_t tokens, float, EchoLightSample or 3 floats per query
+	EchoTokenHierarchy* outLayers;     // pick (nullable)
+	float* outPmf;                     // pick
+	int32_t direct;                    // evaluate_infinite
+};
+bool launch_query(const DeviceScene& scene, int op, const QueryBuffers& buffers, uint64_t n, cudaStream_t stream);
 
 // tuning switches of the wavefront (the ECHO_B200_<NAME> environment variables), changeable at run time; false = unknown name
 bool set_render_option(const char* name, long long value);
@@ -136,6 +155,9 @@ struct EchoScene
 	uint64_t tilesOutBytes = 0;
 	void* hierarchyScratch[4] = {}; // rays, ignore layers, out, hit layers of the *_batch_hierarchy calls, for the same reason
 	uint64_t hierarchyBytes[4] = {};
+	static constexpr int kQuerySlots = 9; // the input and output arrays of the echo_b200_query.h calls (api.cu QuerySlot), grow-only as above
+	void* queryScratch[kQuerySlots] = {};
+	uint64_t queryBytes[kQuerySlots] = {};
 
 	echo::RenderState* render = nullptr;
 

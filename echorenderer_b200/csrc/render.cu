@@ -2243,6 +2243,206 @@ __global__ void __launch_bounds__(kBlock) frame_resolve_kernel(float4* frame, ui
 }
 
 // ---------------------------------------------------------------------------------------------------------------------
+// batched PreparedScene queries (include/echo_b200_query.h): one thread per query over the same device functions the path
+// kernels call (interact, bsdf_*, scene_pick, scene_probability_mass, scene_sample_light, scene_light_pdf, evaluate_infinite),
+// so a query answers what a rendered path computes. api.cu has validated every token, layer and value before the upload.
+// ---------------------------------------------------------------------------------------------------------------------
+
+ECHO_DEVICE PathLayers query_layers(const EchoTokenHierarchy* layers, uint64_t i)
+{
+	if (!layers) return no_layers();
+	const EchoTokenHierarchy h = layers[i];
+	return { h.instanceCount, { h.instances[0], h.instances[1], h.instances[2], h.instances[3], h.instances[4] } };
+}
+
+ECHO_DEVICE vec3 query_vec3(const float* values, uint64_t i) { return { values[i * 3], values[i * 3 + 1], values[i * 3 + 2] }; }
+ECHO_DEVICE vec2 query_sample2(const float* values, uint64_t i) { return { sample1d(values[i * 2]), sample1d(values[i * 2 + 1]) }; } // (Sample2D)
+ECHO_DEVICE SurfacePoint query_point(const EchoSurface& s) { return { { s.position[0], s.position[1], s.position[2] }, { s.normal[0], s.normal[1], s.normal[2] } }; }
+ECHO_DEVICE void query_store(float* out, vec3 v) { out[0] = v.x; out[1] = v.y; out[2] = v.z; }
+ECHO_DEVICE void query_store(float* out, rgb v) { out[0] = v.r; out[1] = v.g; out[2] = v.b; }
+
+// PreparedScene.Interact + Material.Scatter of hit i; false on a miss
+template<bool INST>
+ECHO_DEVICE bool query_contact(const DeviceScene& scene, const QueryBuffers& q, uint64_t i, Contact& c)
+{
+	const EchoHit hit = q.hits[i];
+	if (hit.token == ECHO_TOKEN_EMPTY) return false;
+	const EchoRay ray = q.rays[i];
+	interact<INST>(scene, hit.token, { hit.uv[0], hit.uv[1] }, hit.distance, query_layers(q.layers, i), { ray.origin[0], ray.origin[1], ray.origin[2] },
+	               { ray.direction[0], ray.direction[1], ray.direction[2] }, c);
+	return true;
+}
+
+template<bool INST>
+__global__ void __launch_bounds__(kBlock) query_interact_kernel(DeviceScene scene, QueryBuffers q, uint64_t n)
+{
+	uint64_t i = (uint64_t)blockIdx.x * kBlock + threadIdx.x;
+	if (i >= n) return;
+
+	EchoContact o = {};
+	o.material = ECHO_TOKEN_EMPTY;
+	Contact c;
+
+	if (query_contact<INST>(scene, q, i, c))
+	{
+		query_store(o.position, c.point.position);
+		query_store(o.normal, c.point.normal);
+		query_store(o.shadeNormal, c.shadeNormal);
+		o.texcoord[0] = c.texcoord.x;
+		o.texcoord[1] = c.texcoord.y;
+		o.material = c.materialIndex;
+		// the emission test of shade_body: Emissive with positive power, Emissive.Emit facing the ray
+		bool emits = c.material.type == ECHO_MATERIAL_EMISSIVE && positive(emissive_power(c.material)) && dot(c.outgoing, c.point.normal) > 0.0f;
+		query_store(o.emission, emits ? material_emission(c.material) : make_rgb(0.0f));
+		o.lobes = (uint32_t)bsdf_lobe_count(c.bsdf.kind);
+	}
+
+	static_cast<EchoContact*>(q.out)[i] = o;
+}
+
+template<bool INST>
+__global__ void __launch_bounds__(kBlock) query_scatter_sample_kernel(DeviceScene scene, QueryBuffers q, uint64_t n)
+{
+	uint64_t i = (uint64_t)blockIdx.x * kBlock + threadIdx.x;
+	if (i >= n) return;
+
+	EchoScatter o = {};
+	Contact c;
+
+	if (query_contact<INST>(scene, q, i, c))
+	{
+		vec3 incident;
+		int selectedType;
+		Sampled sampled = bsdf_sample<KINDS_ALL>(c.bsdf, c.outgoing, query_sample2(q.values, i), incident, selectedType);
+		query_store(o.incident, incident);
+		o.pdf = sampled.pdf;
+		query_store(o.value, sampled.content);
+		o.specular = (selectedType & FT_SPECULAR) ? 1u : 0u;
+	}
+
+	static_cast<EchoScatter*>(q.out)[i] = o;
+}
+
+template<bool INST>
+__global__ void __launch_bounds__(kBlock) query_scatter_evaluate_kernel(DeviceScene scene, QueryBuffers q, uint64_t n)
+{
+	uint64_t i = (uint64_t)blockIdx.x * kBlock + threadIdx.x;
+	if (i >= n) return;
+
+	float4 o = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
+	Contact c;
+
+	if (query_contact<INST>(scene, q, i, c))
+	{
+		vec3 incident = query_vec3(q.values, i);
+		o = make4(bsdf_evaluate<KINDS_ALL>(c.bsdf, c.outgoing, incident), bsdf_pdf<KINDS_ALL>(c.bsdf, c.outgoing, incident));
+	}
+
+	static_cast<float4*>(q.out)[i] = o;
+}
+
+template<bool INST>
+__global__ void __launch_bounds__(kBlock) query_pick_kernel(DeviceScene scene, QueryBuffers q, uint64_t n)
+{
+	uint64_t i = (uint64_t)blockIdx.x * kBlock + threadIdx.x;
+	if (i >= n) return;
+
+	float pmf;
+	PathLayers layers;
+	uint32_t token = scene_pick<INST>(scene, query_point(q.points[i]), sample1d(q.values[i]), pmf, layers);
+	if (token == ECHO_TOKEN_EMPTY) layers = no_layers(); // a failed pick has no hierarchy
+
+	static_cast<uint32_t*>(q.out)[i] = token;
+	q.outPmf[i] = pmf;
+
+	if (q.outLayers)
+	{
+		EchoTokenHierarchy h = {};
+		h.instanceCount = layers.count;
+		for (uint32_t k = 0; k < ECHO_MAX_INSTANCE_LAYERS; k++) h.instances[k] = k < layers.count ? layers.tokens[k] : 0u;
+		q.outLayers[i] = h;
+	}
+}
+
+template<bool INST>
+__global__ void __launch_bounds__(kBlock) query_mass_kernel(DeviceScene scene, QueryBuffers q, uint64_t n)
+{
+	uint64_t i = (uint64_t)blockIdx.x * kBlock + threadIdx.x;
+	if (i >= n) return;
+
+	uint32_t token = q.tokens[i];
+	static_cast<float*>(q.out)[i] = token == ECHO_TOKEN_EMPTY ? 0.0f : scene_probability_mass<INST>(scene, token, query_layers(q.layers, i), query_point(q.points[i]));
+}
+
+template<bool INST>
+__global__ void __launch_bounds__(kBlock) query_sample_kernel(DeviceScene scene, QueryBuffers q, uint64_t n)
+{
+	uint64_t i = (uint64_t)blockIdx.x * kBlock + threadIdx.x;
+	if (i >= n) return;
+
+	EchoLightSample o = {};
+	uint32_t token = q.tokens[i];
+
+	if (token != ECHO_TOKEN_EMPTY)
+	{
+		vec3 incident;
+		float travel;
+		Sampled sampled = scene_sample_light<INST>(scene, token, query_layers(q.layers, i), query_point(q.points[i]), query_sample2(q.values, i), incident, travel);
+		query_store(o.radiance, sampled.content);
+		o.pdf = sampled.pdf;
+		query_store(o.incident, incident);
+		o.travel = travel;
+	}
+
+	static_cast<EchoLightSample*>(q.out)[i] = o;
+}
+
+template<bool INST>
+__global__ void __launch_bounds__(kBlock) query_pdf_kernel(DeviceScene scene, QueryBuffers q, uint64_t n)
+{
+	uint64_t i = (uint64_t)blockIdx.x * kBlock + threadIdx.x;
+	if (i >= n) return;
+
+	uint32_t token = q.tokens[i];
+	static_cast<float*>(q.out)[i] = token == ECHO_TOKEN_EMPTY ? 0.0f : scene_light_pdf<INST>(scene, token, query_layers(q.layers, i), query_point(q.points[i]), query_vec3(q.values, i));
+}
+
+__global__ void __launch_bounds__(kBlock) query_infinite_kernel(DeviceScene scene, QueryBuffers q, uint64_t n)
+{
+	uint64_t i = (uint64_t)blockIdx.x * kBlock + threadIdx.x;
+	if (i >= n) return;
+	query_store(static_cast<float*>(q.out) + i * 3, evaluate_infinite(scene, query_vec3(q.values, i), q.direct != 0));
+}
+
+template<bool INST>
+static bool launch_query_inst(const DeviceScene& scene, int op, const QueryBuffers& q, uint64_t n, cudaStream_t stream)
+{
+	const unsigned int blocks = (unsigned int)((n + kBlock - 1) / kBlock);
+
+	switch (op)
+	{
+		case QUERY_INTERACT: query_interact_kernel<INST><<<blocks, kBlock, 0, stream>>>(scene, q, n); break;
+		case QUERY_SCATTER_SAMPLE: query_scatter_sample_kernel<INST><<<blocks, kBlock, 0, stream>>>(scene, q, n); break;
+		case QUERY_SCATTER_EVALUATE: query_scatter_evaluate_kernel<INST><<<blocks, kBlock, 0, stream>>>(scene, q, n); break;
+		case QUERY_PICK: query_pick_kernel<INST><<<blocks, kBlock, 0, stream>>>(scene, q, n); break;
+		case QUERY_MASS: query_mass_kernel<INST><<<blocks, kBlock, 0, stream>>>(scene, q, n); break;
+		case QUERY_SAMPLE: query_sample_kernel<INST><<<blocks, kBlock, 0, stream>>>(scene, q, n); break;
+		case QUERY_PDF: query_pdf_kernel<INST><<<blocks, kBlock, 0, stream>>>(scene, q, n); break;
+		case QUERY_INFINITE: query_infinite_kernel<<<blocks, kBlock, 0, stream>>>(scene, q, n); break;
+		default: set_error("unknown scene query"); return false;
+	}
+
+	return check_cuda(cudaGetLastError(), "scene query launch");
+}
+
+bool launch_query(const DeviceScene& scene, int op, const QueryBuffers& buffers, uint64_t n, cudaStream_t stream)
+{
+	if (n == 0) return true;
+	const bool instanced = scene.packCount != 0u || scene.textureCount != 0u; // evaluate_paths_stack's choice of the shading instantiation
+	return instanced ? launch_query_inst<true>(scene, op, buffers, n, stream) : launch_query_inst<false>(scene, op, buffers, n, stream);
+}
+
+// ---------------------------------------------------------------------------------------------------------------------
 // host side
 // ---------------------------------------------------------------------------------------------------------------------
 

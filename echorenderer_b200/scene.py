@@ -176,6 +176,112 @@ class PreparedScene:
                                                                   len(rays), _native.pointer(occluded)))
         return occluded
 
+    # ---- the rest of PreparedScene for a custom evaluator, batched (include/echo_b200_query.h); host numpy buffers. `layers`
+    # (structs.TOKEN_HIERARCHY, one per query) is optional everywhere: None means empty hierarchies ----
+    def _contact_arguments(self, rays, hits, layers):
+        rays = np.ascontiguousarray(rays, dtype=structs.RAY)
+        hits = np.ascontiguousarray(hits, dtype=structs.HIT)
+        if len(hits) != len(rays):
+            raise ValueError("one hit per ray")
+        return rays, hits, self._layers(layers, len(rays))
+
+    @staticmethod
+    def _layers(layers, count):
+        if layers is None:
+            return None
+        layers = np.ascontiguousarray(layers, dtype=structs.TOKEN_HIERARCHY)
+        if len(layers) != count:
+            raise ValueError("one TOKEN_HIERARCHY per query")
+        return layers
+
+    @staticmethod
+    def _floats(values, count, width, what):
+        values = np.ascontiguousarray(values, dtype=np.float32).reshape(-1, width) if width > 1 else np.ascontiguousarray(values, dtype=np.float32).reshape(-1)
+        if len(values) != count:
+            raise ValueError(f"one {what} per query")
+        return values
+
+    def _light_arguments(self, tokens, points, layers):
+        tokens = np.ascontiguousarray(tokens, dtype=np.uint32).reshape(-1)
+        points = np.ascontiguousarray(points, dtype=structs.SURFACE)
+        if len(points) != len(tokens):
+            raise ValueError("one surface per light token")
+        return tokens, points, self._layers(layers, len(tokens))
+
+    def interact(self, rays, hits, layers=None):
+        """PreparedScene.Interact + Material.Scatter (PreparedScene.cs:95-105) of every (ray, hit, hit layers) of a trace ->
+        structs.CONTACT records (material TOKEN_EMPTY on a miss)."""
+        rays, hits, layers = self._contact_arguments(rays, hits, layers)
+        out = np.empty(len(rays), dtype=structs.CONTACT)
+        _native.check(self._lib.echo_b200_interact_batch(self._handle, _native.pointer(rays), _native.pointer(hits), _native.pointer(layers), len(rays), _native.pointer(out)))
+        return out
+
+    def scatter_sample(self, rays, hits, samples, layers=None):
+        """BSDF.Sample (BSDF.cs:150-208) at the contact of every hit with samples[n, 2] -> structs.SCATTER records."""
+        rays, hits, layers = self._contact_arguments(rays, hits, layers)
+        samples = self._floats(samples, len(rays), 2, "sample pair")
+        out = np.empty(len(rays), dtype=structs.SCATTER)
+        _native.check(self._lib.echo_b200_scatter_sample_batch(self._handle, _native.pointer(rays), _native.pointer(hits), _native.pointer(layers), _native.pointer(samples),
+                                                               len(rays), _native.pointer(out)))
+        return out
+
+    def scatter_evaluate(self, rays, hits, incident, layers=None):
+        """BSDF.Evaluate and BSDF.ProbabilityDensity (BSDF.cs:97-143) at the contact of every hit towards incident[n, 3] ->
+        float32[n, 4]: RGB value, W pdf."""
+        rays, hits, layers = self._contact_arguments(rays, hits, layers)
+        incident = self._floats(incident, len(rays), 3, "incident direction")
+        out = np.empty((len(rays), 4), dtype=np.float32)
+        _native.check(self._lib.echo_b200_scatter_evaluate_batch(self._handle, _native.pointer(rays), _native.pointer(hits), _native.pointer(layers), _native.pointer(incident),
+                                                                 len(rays), _native.pointer(out)))
+        return out
+
+    def pick(self, points, samples):
+        """PreparedScene.Pick (PreparedScene.cs:113-150) from every structs.SURFACE with samples[n] -> (light tokens uint32[n],
+        their structs.TOKEN_HIERARCHY layers, pmf float32[n])."""
+        points = np.ascontiguousarray(points, dtype=structs.SURFACE)
+        samples = self._floats(samples, len(points), 1, "sample")
+        tokens = np.empty(len(points), dtype=np.uint32)
+        layers = np.zeros(len(points), dtype=structs.TOKEN_HIERARCHY)
+        pmf = np.empty(len(points), dtype=np.float32)
+        _native.check(self._lib.echo_b200_light_pick_batch(self._handle, _native.pointer(points), _native.pointer(samples), len(points), _native.pointer(tokens),
+                                                           _native.pointer(layers), _native.pointer(pmf)))
+        return tokens, layers, pmf
+
+    def probability_mass(self, tokens, points, layers=None):
+        """PreparedScene.ProbabilityMass (PreparedScene.cs:158-179) of every light token seen from its surface -> float32[n]."""
+        tokens, points, layers = self._light_arguments(tokens, points, layers)
+        out = np.empty(len(tokens), dtype=np.float32)
+        _native.check(self._lib.echo_b200_light_mass_batch(self._handle, _native.pointer(tokens), _native.pointer(layers), _native.pointer(points), len(tokens), _native.pointer(out)))
+        return out
+
+    def sample(self, tokens, points, samples, layers=None):
+        """PreparedScene.Sample (PreparedScene.cs:182-204) of every light token from its surface with samples[n, 2] ->
+        structs.LIGHT_SAMPLE records."""
+        tokens, points, layers = self._light_arguments(tokens, points, layers)
+        samples = self._floats(samples, len(tokens), 2, "sample pair")
+        out = np.empty(len(tokens), dtype=structs.LIGHT_SAMPLE)
+        _native.check(self._lib.echo_b200_light_sample_batch(self._handle, _native.pointer(tokens), _native.pointer(layers), _native.pointer(points), _native.pointer(samples),
+                                                             len(tokens), _native.pointer(out)))
+        return out
+
+    def probability_density(self, tokens, points, incident, layers=None):
+        """PreparedScene.ProbabilityDensity (PreparedScene.cs:207-225) of every light token from its surface towards
+        incident[n, 3] -> float32[n]."""
+        tokens, points, layers = self._light_arguments(tokens, points, layers)
+        incident = self._floats(incident, len(tokens), 3, "incident direction")
+        out = np.empty(len(tokens), dtype=np.float32)
+        _native.check(self._lib.echo_b200_light_pdf_batch(self._handle, _native.pointer(tokens), _native.pointer(layers), _native.pointer(points), _native.pointer(incident),
+                                                          len(tokens), _native.pointer(out)))
+        return out
+
+    def evaluate_infinite(self, directions, direct=False):
+        """PreparedScene.EvaluateInfinite (PreparedScene.cs:233-253) along directions[n, 3] -> float32[n, 3]; `direct` sums only
+        the directly visible lights."""
+        directions = np.ascontiguousarray(directions, dtype=np.float32).reshape(-1, 3)
+        out = np.empty((len(directions), 3), dtype=np.float32)
+        _native.check(self._lib.echo_b200_evaluate_infinite_batch(self._handle, _native.pointer(directions), len(directions), 1 if direct else 0, _native.pointer(out)))
+        return out
+
     # ---- raw-pointer variants for pinned host memory / device memory owned by the caller (torch tensors) ----
     def trace_pointers(self, rays_pointer, count, hits_pointer):
         _native.check(self._lib.echo_b200_trace_batch(self._handle, ctypes.c_void_p(rays_pointer), count, ctypes.c_void_p(hits_pointer)))

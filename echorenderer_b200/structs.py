@@ -70,6 +70,13 @@ INSTANCE = np.dtype([("forward", "<f4", 12), ("inverse", "<f4", 12), ("forwardSc
                      ("materialOffset", "<u4"), ("reserved", "<u4", 4)])
 TOKEN_HIERARCHY = np.dtype([("instanceCount", "<u4"), ("instances", "<u4", MAX_INSTANCE_LAYERS)])
 
+# include/echo_b200_query.h: GeometryPoint, Contact, BSDF.Sample's result, PreparedScene.Sample's result
+SURFACE = np.dtype([("position", "<f4", 3), ("normal", "<f4", 3)])
+CONTACT = np.dtype([("position", "<f4", 3), ("normal", "<f4", 3), ("shadeNormal", "<f4", 3), ("texcoord", "<f4", 2), ("material", "<u4"),
+                    ("emission", "<f4", 3), ("lobes", "<u4")])
+SCATTER = np.dtype([("incident", "<f4", 3), ("pdf", "<f4"), ("value", "<f4", 3), ("specular", "<u4")])
+LIGHT_SAMPLE = np.dtype([("radiance", "<f4", 3), ("pdf", "<f4"), ("incident", "<f4", 3), ("travel", "<f4")])
+
 MATERIAL = np.dtype([
     ("type", "<u4"), ("flags", "<u4"), ("albedo", "<f4", 4), ("roughness", "<f4", 2), ("ior", "<f4"),
     ("paramA", "<f4", 3), ("paramB", "<f4", 3), ("base", "<u4"),
@@ -147,6 +154,10 @@ assert INFINITE_LIGHT.itemsize == 160
 assert CAMERA.itemsize == 80
 assert RENDER_PARAMS.itemsize == 48
 assert STATS.itemsize == 192
+assert SURFACE.itemsize == 24
+assert CONTACT.itemsize == 64
+assert SCATTER.itemsize == 32
+assert LIGHT_SAMPLE.itemsize == 32
 
 
 def render_params(width, height, tile_size=16, extend=16, min_epoch=1, max_epoch=1, noise_threshold=0.045,
