@@ -33,7 +33,7 @@ EXPORTS = [
     "echo_b200_debug_evaluate_samples4", "echo_b200_debug_bounds_violations",
     "echo_b200_trace_batch_device_counted", "echo_b200_occlude_batch_device_counted", "echo_b200_debug_bxdf_batch", "echo_b200_debug_math",
     "echo_b200_debug_evaluate_samples",
-    "echo_b200_host_alloc", "echo_b200_host_free", "echo_b200_host_register", "echo_b200_host_unregister", "echo_b200_debug_set_option", "echo_b200_debug_measure_peaks", "echo_b200_debug_last_build", "echo_b200_debug_last_light_build", "echo_b200_build_light_tree", "echo_b200_scene_build_light_tree",
+    "echo_b200_host_alloc", "echo_b200_host_free", "echo_b200_host_register", "echo_b200_host_unregister", "echo_b200_debug_set_option", "echo_b200_debug_get_option", "echo_b200_debug_measure_peaks", "echo_b200_debug_last_build", "echo_b200_debug_last_light_build", "echo_b200_build_light_tree", "echo_b200_scene_build_light_tree",
     "echo_b200_scene_create_multi", "echo_b200_scene_gpu_count", "echo_b200_build_packs", "echo_b200_scene_build_packs", "echo_b200_debug_last_pack_build",
 ]
 
@@ -94,6 +94,7 @@ def library():
         "echo_b200_host_register": [p, u64],
         "echo_b200_host_unregister": [p],
         "echo_b200_debug_set_option": [ctypes.c_char_p, ctypes.c_int64],
+        "echo_b200_debug_get_option": [ctypes.c_char_p, ctypes.POINTER(ctypes.c_int64)],
         "echo_b200_debug_measure_peaks": [i32, p],
         "echo_b200_debug_last_build": [p],
         "echo_b200_debug_last_light_build": [p],
@@ -177,6 +178,13 @@ class HostBuffer:
 def set_option(name, value):
     """echo_b200_debug_set_option: one tuning switch of the wavefront (the ECHO_B200_<name> environment variables), at run time."""
     check(library().echo_b200_debug_set_option(name.encode(), int(value)))
+
+
+def get_option(name):
+    """echo_b200_debug_get_option: the value a tuning switch has now."""
+    value = ctypes.c_int64()
+    check(library().echo_b200_debug_get_option(name.encode(), ctypes.byref(value)))
+    return value.value
 
 
 def measure_peaks(device=0):

@@ -1709,6 +1709,15 @@ int32_t echo_b200_debug_set_option(const char* name, int64_t value)
 	return set_render_option(name, (long long)value) || set_build_option(name, (long long)value) ? ECHO_B200_OK : fail(ECHO_B200_ERR_INVALID, "unknown option");
 }
 
+int32_t echo_b200_debug_get_option(const char* name, int64_t* value)
+{
+	if (!name || !value) return fail(ECHO_B200_ERR_INVALID, "null argument");
+	long long current = 0;
+	if (!get_render_option(name, current) && !get_build_option(name, current)) return fail(ECHO_B200_ERR_INVALID, "unknown option");
+	*value = (int64_t)current;
+	return ECHO_B200_OK;
+}
+
 int32_t echo_b200_debug_last_build(float* out4)
 {
 	if (!out4) return fail(ECHO_B200_ERR_INVALID, "out4 is null");

@@ -432,6 +432,15 @@ bool set_build_option(const char* name, long long value)
 	return true;
 }
 
+bool get_build_option(const char* name, long long& value)
+{
+	const std::string key = name ? name : "";
+	if (key == "BUILD_ALGORITHM") value = build_algorithm();
+	else if (key == "BUILD_PLOC_RADIUS") value = ploc_radius();
+	else return false;
+	return true;
+}
+
 static bool build_qbvh_with(bool ploc, const EchoTriangle* triangles, uint32_t triangleCount, const EchoSphere* spheres, uint32_t sphereCount,
                             const float* instanceBounds, uint32_t instanceCount, EchoQbvhNode* outNodes, uint32_t* outNodeCount, uint32_t* outMaxDepth, bool* stalled);
 

@@ -93,6 +93,8 @@ bool launch_query(const DeviceScene& scene, int op, const QueryBuffers& buffers,
 // tuning switches of the wavefront (the ECHO_B200_<NAME> environment variables), changeable at run time; false = unknown name
 bool set_render_option(const char* name, long long value);
 bool set_build_option(const char* name, long long value); // build.cu: BUILD_ALGORITHM (2 = SweepBuilder, 1 = PLOC, 0 = LBVH)
+bool get_render_option(const char* name, long long& value);
+bool get_build_option(const char* name, long long& value);
 
 // ---- peaks.cu: on-chip ceilings measured on the current device: {L2 coalesced read, L2 random 32-byte sectors, L1 random sectors} GB/s
 bool measure_peaks(float* out3);

@@ -1495,6 +1495,14 @@ ECHO_DEVICE void shade_body(const DeviceScene& scene, const EchoRenderParams& pa
 				result = result + energy * (emitted * weight);
 			}
 		}
+		else if (COUNT && INST && mode == MODE_MIS)
+		{
+			// After a MIS bounce the reference asks ProbabilityMass of whatever surface it reached (:96-109). For a surface inside
+			// placements that walks the light trees of the hit's instance layers before the map lookup finds that the token is no
+			// light. The mass is zero and unused here, but a counted pass reports those LightBound.Importance evaluations too.
+			SurfacePoint oldPoint = { xyz(stream_load(paths.oldPosition + id)), xyz(stream_load(paths.oldNormal + id)) };
+			(void)scene_probability_mass<INST, COUNT>(scene, token, hitLayers, oldPoint);
+		}
 
 		// ---- the loop body: `for (int depth = 0; depth < BounceLimit; depth++)`, :57 ----
 		if (bounces < (uint32_t)params.bounceLimit)
@@ -2585,19 +2593,32 @@ static RenderOptions& options()
 	return instance;
 }
 
-bool set_render_option(const char* name, long long value)
+static std::atomic<long long>* render_option(const char* name)
 {
 	RenderOptions& o = options();
 	const std::string key = name ? name : "";
-	if (key == "RENDER_WORKERS") o.renderWorkers = value;
-	else if (key == "BATCH_PATHS") o.batchPaths = value;
-	else if (key == "NARROW_LIMIT") o.narrowLimit = value;
-	else if (key == "TAIL_LIMIT") o.tailLimit = value;
-	else if (key == "RUN_AHEAD") o.runAhead = value;
-	else if (key == "BLOCKING_SYNC") o.blockingSync = value;
-	else if (key == "GUIDED_BATCHES") o.guidedBatches = value;
-	else return false;
-	return true;
+	if (key == "RENDER_WORKERS") return &o.renderWorkers;
+	if (key == "BATCH_PATHS") return &o.batchPaths;
+	if (key == "NARROW_LIMIT") return &o.narrowLimit;
+	if (key == "TAIL_LIMIT") return &o.tailLimit;
+	if (key == "RUN_AHEAD") return &o.runAhead;
+	if (key == "BLOCKING_SYNC") return &o.blockingSync;
+	if (key == "GUIDED_BATCHES") return &o.guidedBatches;
+	return nullptr;
+}
+
+bool set_render_option(const char* name, long long value)
+{
+	std::atomic<long long>* option = render_option(name);
+	if (option) *option = value;
+	return option != nullptr;
+}
+
+bool get_render_option(const char* name, long long& value)
+{
+	std::atomic<long long>* option = render_option(name);
+	if (option) value = *option;
+	return option != nullptr;
 }
 
 // How a pipeline thread waits for the counts of a unit (ECHO_B200_BLOCKING_SYNC):

@@ -51,6 +51,8 @@ int32_t echo_b200_debug_measure_peaks(int32_t device, float* out3);
  * sets its initial value (RENDER_WORKERS, BATCH_PATHS, NARROW_LIMIT, TAIL_LIMIT, RUN_AHEAD, BLOCKING_SYNC; -1 = automatic for the
  * last two). Process-wide; takes effect with the next render call. For A/B runs that keep one uploaded scene. */
 int32_t echo_b200_debug_set_option(const char* name, int64_t value);
+/* The current value of a switch echo_b200_debug_set_option takes, so that a caller can check it left every switch as it found it. */
+int32_t echo_b200_debug_get_option(const char* name, int64_t* value);
 
 /* Phases of the calling thread's last echo_b200_build_qbvh that ran the SweepBuilder build (csrc/sweep.cu): out4 = {upload ms, device
  * build ms, download ms, binary levels}, host wall time around synchronised phases. Zeros if no such build ran on this thread. */
