@@ -43,6 +43,15 @@ QUERY_EXPORTS = [
     "echo_b200_light_mass_batch", "echo_b200_light_sample_batch", "echo_b200_light_pdf_batch", "echo_b200_evaluate_infinite_batch",
 ]
 
+# every symbol include/echo_b200_query_device.h declares: the queries above and the layered trace / occlusion on device buffers
+DEVICE_QUERY_EXPORTS = [
+    "echo_b200_interact_batch_device", "echo_b200_scatter_sample_batch_device", "echo_b200_scatter_evaluate_batch_device",
+    "echo_b200_light_pick_batch_device", "echo_b200_light_mass_batch_device", "echo_b200_light_sample_batch_device", "echo_b200_light_pdf_batch_device",
+    "echo_b200_evaluate_infinite_batch_device", "echo_b200_trace_batch_hierarchy_device", "echo_b200_occlude_batch_hierarchy_device", "echo_b200_query_reason",
+]
+
+QUERY_STATUS_CLEAR = 0xFFFFFFFFFFFFFFFF  # ECHO_QUERY_STATUS_CLEAR: what a status word holds before the calls, and after them when no query was refused
+
 
 def library():
     global _lib
@@ -114,6 +123,16 @@ def library():
         "echo_b200_light_sample_batch": [p, p, p, p, p, u64, p],
         "echo_b200_light_pdf_batch": [p, p, p, p, p, u64, p],
         "echo_b200_evaluate_infinite_batch": [p, p, u64, i32, p],
+        "echo_b200_interact_batch_device": [p, p, p, p, u64, p, p, p],
+        "echo_b200_scatter_sample_batch_device": [p, p, p, p, p, u64, p, p, p],
+        "echo_b200_scatter_evaluate_batch_device": [p, p, p, p, p, u64, p, p, p],
+        "echo_b200_light_pick_batch_device": [p, p, p, u64, p, p, p, p, p],
+        "echo_b200_light_mass_batch_device": [p, p, p, p, u64, p, p, p],
+        "echo_b200_light_sample_batch_device": [p, p, p, p, p, u64, p, p, p],
+        "echo_b200_light_pdf_batch_device": [p, p, p, p, p, u64, p, p, p],
+        "echo_b200_evaluate_infinite_batch_device": [p, p, u64, i32, p, p, p],
+        "echo_b200_trace_batch_hierarchy_device": [p, p, p, u64, p, p, p],
+        "echo_b200_occlude_batch_hierarchy_device": [p, p, p, u64, p, p],
     }
 
     for name, argtypes in signatures.items():
@@ -123,6 +142,8 @@ def library():
 
     lib.echo_b200_last_error.restype = ctypes.c_char_p
     lib.echo_b200_version.restype = ctypes.c_char_p
+    lib.echo_b200_query_reason.argtypes = [u32]
+    lib.echo_b200_query_reason.restype = ctypes.c_char_p
     _lib = lib
     return lib
 
@@ -130,6 +151,19 @@ def library():
 def check(status):
     if status != OK:
         raise EchoNativeError(status, library().echo_b200_last_error().decode("utf-8", "replace"))
+
+
+def query_reason(code):
+    """echo_b200_query_reason: the text of a refusal code (the low 8 bits of a status word)"""
+    return library().echo_b200_query_reason(int(code)).decode("utf-8", "replace")
+
+
+def query_status(value):
+    """Raises EchoNativeError(ERR_INVALID) naming the lowest refused query and its reason when a status word of the
+    include/echo_b200_query_device.h calls is not QUERY_STATUS_CLEAR."""
+    value = int(value) & QUERY_STATUS_CLEAR
+    if value != QUERY_STATUS_CLEAR:
+        raise EchoNativeError(ERR_INVALID, f"query {value >> 8}: {query_reason(value & 0xFF)}")
 
 
 def pointer(array):

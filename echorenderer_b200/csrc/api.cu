@@ -9,9 +9,11 @@
 #include <thread>
 
 #include "../../include/echo_b200_debug.h"
+#include "../../include/echo_b200_query_device.h"
 #include "echo_internal.h"
 #include "echo_light_build.h"
 #include "echo_pack_build.h"
+#include "echo_query_rules.h"
 
 namespace echo
 {
@@ -1241,7 +1243,7 @@ int32_t query_host(EchoScene* scene, const QueryCall& call, uint64_t n)
 		                         static_cast<const EchoSurface*>(device[SLOT_POINTS]), static_cast<const uint32_t*>(device[SLOT_TOKENS]),
 		                         static_cast<const EchoTokenHierarchy*>(device[SLOT_LAYERS]), static_cast<const float*>(device[SLOT_VALUES]), device[SLOT_OUT],
 		                         static_cast<EchoTokenHierarchy*>(device[SLOT_OUT_LAYERS]), static_cast<float*>(device[SLOT_OUT_PMF]), call.direct };
-		ok = launch_query(scene->d, call.op, buffers, n, stream);
+		ok = launch_query(scene->d, call.op, buffers, n, stream, false);
 	}
 
 	for (int s = SLOT_OUT; ok && s < SLOT_COUNT; s++)
@@ -1264,118 +1266,36 @@ int32_t query_run(EchoScene* scene, const QueryCall& call, uint64_t n)
 	});
 }
 
-// ---- host-side validation of the tokens, layers and values a query takes from outside the library (echo_b200_query.h) ----
+// ---- host-side validation of the tokens, layers and values a query takes from outside the library (echo_b200_query.h): the rules of
+// echo_query_rules.h over the host copies of the scene ----
 
-bool all_finite(const float* values, int count)
+struct HostRuleScene
 {
-	for (int i = 0; i < count; i++)
-		if (!std::isfinite(values[i])) return false;
-	return true;
-}
+	const EchoScene* scene;
 
-bool unit_direction(const float* v)
+	uint32_t packCount() const { return (uint32_t)scene->packs.size(); }
+	EchoPack pack(uint32_t p) const { return scene->packs[p]; }
+	void instance(uint32_t i, uint32_t& pack, uint32_t& materialOffset) const
+	{
+		pack = scene->instances[i].pack;
+		materialOffset = scene->instances[i].materialOffset;
+	}
+	uint32_t triangleCount() const { return (uint32_t)scene->triangles.size(); }
+	uint32_t sphereCount() const { return (uint32_t)scene->spheres.size(); }
+	uint32_t pointLightCount() const { return (uint32_t)scene->pointLights.size(); }
+	uint32_t infiniteLightCount() const { return (uint32_t)scene->infiniteLights.size(); }
+	uint32_t materialCount() const { return (uint32_t)scene->materials.size(); }
+	uint32_t triangleMaterial(uint32_t t) const { return scene->triangles[t].material; }
+	uint32_t sphereMaterial(uint32_t s) const { return scene->spheres[s].material; }
+};
+
+// "<call>: query <i>: <reason>", the layer named where a layer is refused
+int32_t refuse(const char* call, uint64_t i, uint32_t code, uint32_t layer = 0)
 {
-	if (!all_finite(v, 3)) return false;
-	double length = std::sqrt((double)v[0] * v[0] + (double)v[1] * v[1] + (double)v[2] * v[2]);
-	return std::fabs(length - 1.0) <= 1e-3;
+	std::string why = rules::reason_text(code);
+	if (code == rules::LAYER_NOT_INSTANCE) why = "layer " + std::to_string(layer) + why.substr(std::strlen("layer"));
+	return fail(ECHO_B200_ERR_INVALID, (std::string(call) + ": query " + std::to_string(i) + ": " + why).c_str());
 }
-
-uint32_t token_kind(uint32_t token) { return token >> ECHO_TOKEN_INDEX_BITS; }
-uint32_t token_number(uint32_t token) { return token & ((1u << ECHO_TOKEN_INDEX_BITS) - 1u); }
-
-// FindLayer on the host copies of the packs and placements: the pack hierarchy i ends in and the swatch offset it selects.
-// Returns why the hierarchy is refused, or an empty string.
-std::string check_layers(const EchoScene* scene, const EchoTokenHierarchy* layers, uint64_t i, EchoPack& pack, uint32_t& materialOffset)
-{
-	if (scene->packs.empty())
-	{
-		pack = EchoPack{};
-		pack.triangleCount = (uint32_t)scene->triangles.size();
-		pack.sphereCount = (uint32_t)scene->spheres.size();
-		pack.pointLightCount = (uint32_t)scene->pointLights.size();
-	}
-	else pack = scene->packs[0];
-
-	materialOffset = pack.materialOffset;
-	if (!layers || layers[i].instanceCount == 0u) return "";
-	if (scene->packs.empty()) return "instance layers on a scene without packs";
-	if (layers[i].instanceCount > ECHO_MAX_INSTANCE_LAYERS) return "more than ECHO_MAX_INSTANCE_LAYERS instance layers";
-
-	for (uint32_t k = 0; k < layers[i].instanceCount; k++)
-	{
-		uint32_t token = layers[i].instances[k];
-		if (token_kind(token) != ECHO_TOKEN_TYPE_INSTANCE || token_number(token) >= pack.instanceCount)
-			return "layer " + std::to_string(k) + " is not an instance of its parent pack";
-		const EchoInstance& instance = scene->instances[pack.instanceOffset + token_number(token)];
-		materialOffset = instance.materialOffset;
-		pack = scene->packs[instance.pack];
-	}
-
-	return "";
-}
-
-std::string check_hit(const EchoScene* scene, const EchoRay& ray, const EchoHit& hit, const EchoPack& pack, uint32_t materialOffset)
-{
-	if (!all_finite(ray.origin, 3) || !unit_direction(ray.direction)) return "the ray needs a finite origin and a unit direction";
-	if (hit.token == ECHO_TOKEN_EMPTY) return "";
-	if (!std::isfinite(hit.distance) || !all_finite(hit.uv, 2)) return "hit distance or uv is not finite";
-
-	const uint32_t index = token_number(hit.token);
-	const float x = hit.uv[0], y = hit.uv[1];
-	uint32_t material;
-
-	if (token_kind(hit.token) == ECHO_TOKEN_TYPE_TRIANGLE)
-	{
-		if (index >= pack.triangleCount) return "triangle index out of range for its pack";
-		if (!(x >= 0.0f && x <= 1.0f && y >= 0.0f && y <= 1.0f)) return "triangle hit uv outside [0, 1]";
-		material = scene->triangles[pack.triangleOffset + index].material;
-	}
-	else if (token_kind(hit.token) == ECHO_TOKEN_TYPE_SPHERE)
-	{
-		if (index >= pack.sphereCount) return "sphere index out of range for its pack";
-		// x = sin(theta), plus 3 behind the sphere; sin(theta) = point.x / sqrt(r^2 - y^2) may pass 1 by rounding near the poles
-		if (!(y >= -1.0f && y <= 1.0f && x >= -1.5f && x <= 4.5f)) return "sphere hit uv outside the encoding of SphereEntity";
-		material = scene->spheres[pack.sphereOffset + index].material;
-	}
-	else return "hit token is neither a triangle, a sphere nor ECHO_TOKEN_EMPTY";
-
-	if ((uint64_t)materialOffset + material >= scene->materials.size()) return "the hit's material index is out of range";
-	return "";
-}
-
-std::string check_light(const EchoScene* scene, uint32_t token, const EchoPack& pack)
-{
-	if (token == ECHO_TOKEN_EMPTY) return "";
-	const uint32_t index = token_number(token);
-
-	if (token_kind(token) == ECHO_TOKEN_TYPE_LIGHT)
-	{
-		const uint32_t lightType = index >> ECHO_LIGHT_INDEX_BITS, lightIndex = index & ((1u << ECHO_LIGHT_INDEX_BITS) - 1u);
-		if (lightType == ECHO_LIGHT_TYPE_INFINITE || lightType == ECHO_LIGHT_TYPE_INFINITE_DELTA)
-			return lightIndex < scene->infiniteLights.size() ? "" : "infinite light index out of range";
-		if (lightType == ECHO_LIGHT_TYPE_POINT) return lightIndex < pack.pointLightCount ? "" : "point light index out of range for its pack";
-		return "unknown light type";
-	}
-
-	uint32_t material;
-
-	if (token_kind(token) == ECHO_TOKEN_TYPE_TRIANGLE)
-	{
-		if (index >= pack.triangleCount) return "triangle emitter index out of range for its pack";
-		material = scene->triangles[pack.triangleOffset + index].material;
-	}
-	else if (token_kind(token) == ECHO_TOKEN_TYPE_SPHERE)
-	{
-		if (index >= pack.sphereCount) return "sphere emitter index out of range for its pack";
-		material = scene->spheres[pack.sphereOffset + index].material;
-	}
-	else return "light token is neither a light, a triangle, a sphere nor ECHO_TOKEN_EMPTY";
-
-	if ((uint64_t)pack.materialOffset + material >= scene->materials.size()) return "the emitter's material index is out of range";
-	return "";
-}
-
-int32_t refuse(const char* call, uint64_t i, const std::string& why) { return fail(ECHO_B200_ERR_INVALID, (std::string(call) + ": query " + std::to_string(i) + ": " + why).c_str()); }
 
 // interact / scatter_sample / scatter_evaluate: `values` holds `valueCount` floats per query (2: samples, 3: an incident direction)
 int32_t contact_query(EchoScene* scene, const char* name, int op, const EchoRay* rays, const EchoHit* hits, const EchoTokenHierarchy* layers,
@@ -1385,15 +1305,13 @@ int32_t contact_query(EchoScene* scene, const char* name, int op, const EchoRay*
 	if (n == 0) return ECHO_B200_OK;
 	if (!rays || !hits || !out || (valueCount && !values)) return fail(ECHO_B200_ERR_INVALID, (std::string(name) + ": null buffer").c_str());
 
+	const HostRuleScene rulesScene = { scene };
+
 	for (uint64_t i = 0; i < n; i++)
 	{
-		EchoPack pack;
-		uint32_t materialOffset;
-		std::string why = check_layers(scene, layers, i, pack, materialOffset);
-		if (why.empty()) why = check_hit(scene, rays[i], hits[i], pack, materialOffset);
-		if (why.empty() && valueCount == 2 && !all_finite(values + i * 2, 2)) why = "samples are not finite";
-		if (why.empty() && valueCount == 3 && !unit_direction(values + i * 3)) why = "the incident direction is not a finite unit vector";
-		if (!why.empty()) return refuse(name, i, why);
+		uint32_t layer = 0;
+		uint32_t code = rules::check_contact(rulesScene, layers ? layers + i : nullptr, rays[i], hits[i], valueCount ? values + i * valueCount : nullptr, valueCount, layer);
+		if (code != rules::ACCEPTED) return refuse(name, i, code, layer);
 	}
 
 	QueryCall call;
@@ -1414,16 +1332,13 @@ int32_t light_query(EchoScene* scene, const char* name, int op, const uint32_t* 
 	if (n == 0) return ECHO_B200_OK;
 	if (!tokens || !points || !out || (valueCount && !values)) return fail(ECHO_B200_ERR_INVALID, (std::string(name) + ": null buffer").c_str());
 
+	const HostRuleScene rulesScene = { scene };
+
 	for (uint64_t i = 0; i < n; i++)
 	{
-		EchoPack pack;
-		uint32_t materialOffset;
-		std::string why = check_layers(scene, layers, i, pack, materialOffset);
-		if (why.empty()) why = check_light(scene, tokens[i], pack);
-		if (why.empty() && (!all_finite(points[i].position, 3) || !all_finite(points[i].normal, 3))) why = "the surface is not finite";
-		if (why.empty() && valueCount == 2 && !all_finite(values + i * 2, 2)) why = "samples are not finite";
-		if (why.empty() && valueCount == 3 && !unit_direction(values + i * 3)) why = "the incident direction is not a finite unit vector";
-		if (!why.empty()) return refuse(name, i, why);
+		uint32_t layer = 0;
+		uint32_t code = rules::check_light_query(rulesScene, layers ? layers + i : nullptr, tokens[i], points[i], valueCount ? values + i * valueCount : nullptr, valueCount, layer);
+		if (code != rules::ACCEPTED) return refuse(name, i, code, layer);
 	}
 
 	QueryCall call;
@@ -1463,10 +1378,7 @@ int32_t echo_b200_light_pick_batch(EchoScene* scene, const EchoSurface* points, 
 	if (!points || !samples1 || !tokens || !pmf) return fail(ECHO_B200_ERR_INVALID, "echo_b200_light_pick_batch: null buffer");
 
 	for (uint64_t i = 0; i < n; i++)
-	{
-		if (!all_finite(points[i].position, 3) || !all_finite(points[i].normal, 3)) return refuse(name, i, "the surface is not finite");
-		if (!std::isfinite(samples1[i])) return refuse(name, i, "the sample is not finite");
-	}
+		if (uint32_t code = rules::check_pick(points[i], samples1[i])) return refuse(name, i, code);
 
 	QueryCall call;
 	call.op = QUERY_PICK;
@@ -1503,7 +1415,7 @@ int32_t echo_b200_evaluate_infinite_batch(EchoScene* scene, const float* directi
 	if (!directions3 || !outRGB3) return fail(ECHO_B200_ERR_INVALID, "echo_b200_evaluate_infinite_batch: null buffer");
 
 	for (uint64_t i = 0; i < n; i++)
-		if (!unit_direction(directions3 + i * 3)) return refuse(name, i, "the direction is not a finite unit vector");
+		if (uint32_t code = rules::check_infinite(directions3 + i * 3)) return refuse(name, i, code);
 
 	QueryCall call;
 	call.op = QUERY_INFINITE;
@@ -1511,6 +1423,124 @@ int32_t echo_b200_evaluate_infinite_batch(EchoScene* scene, const float* directi
 	call.set(SLOT_VALUES, directions3, sizeof(float) * 3);
 	call.set(SLOT_OUT, outRGB3, sizeof(float) * 3);
 	return query_run(scene, call, n);
+}
+
+// ---- the same queries on device buffers, checked on the device (include/echo_b200_query_device.h) ----
+namespace
+{
+
+constexpr uint64_t kMaxDeviceQueries = 0x7FFFFFFFull * 128u; // one launch grid of render.cu's query kernels (kBlock = 128)
+
+// the synchronous refusals, then one asynchronous checked launch on the caller's stream; `buffers` holds device pointers
+int32_t query_device(EchoScene* scene, const char* name, bool contact, int op, QueryBuffers buffers, bool present, uint64_t n, uint64_t* status, void* stream)
+{
+	if (!(contact ? require_renderable(scene) : require_committed(scene)) || !single_device(scene)) return ECHO_B200_ERR_INVALID;
+	if (n == 0) return ECHO_B200_OK;
+	if (!present || !status) return fail(ECHO_B200_ERR_INVALID, (std::string(name) + ": null buffer").c_str());
+	if (n > kMaxDeviceQueries) return fail(ECHO_B200_ERR_INVALID, (std::string(name) + ": more queries than one launch covers").c_str());
+
+	DeviceGuard guard(scene->device);
+	if (!guard.ok) return ECHO_B200_ERR_NO_DEVICE;
+	buffers.status = reinterpret_cast<unsigned long long*>(status);
+	return launch_query(scene->d, op, buffers, n, (cudaStream_t)stream, true) ? ECHO_B200_OK : ECHO_B200_ERR_CUDA;
+}
+
+// hierarchy_host's refusals and launch, on the caller's device buffers and stream
+int32_t hierarchy_device(EchoScene* scene, const EchoRay* rays, const EchoTokenHierarchy* ignore, uint64_t n, EchoHit* hits, EchoTokenHierarchy* hitLayers,
+                         uint8_t* occluded, void* stream)
+{
+	if (!require_committed(scene) || !single_device(scene)) return ECHO_B200_ERR_INVALID;
+	if (n == 0) return ECHO_B200_OK;
+	if (!rays || (!hits && !occluded)) return fail(ECHO_B200_ERR_INVALID, "null buffer");
+	if (scene->d.packCount == 0u) return fail(ECHO_B200_ERR_INVALID, "the scene has no packs: use the plain batch calls");
+
+	DeviceGuard guard(scene->device);
+	if (!guard.ok) return ECHO_B200_ERR_NO_DEVICE;
+	const bool ok = hits ? launch_trace_instanced(scene->d, rays, ignore, n, hits, hitLayers, nullptr, (cudaStream_t)stream)
+	                     : launch_occlude_instanced(scene->d, rays, ignore, n, occluded, nullptr, (cudaStream_t)stream);
+	return ok ? ECHO_B200_OK : ECHO_B200_ERR_CUDA;
+}
+
+} // namespace
+
+int32_t echo_b200_interact_batch_device(EchoScene* scene, const EchoRay* rays, const EchoHit* hits, const EchoTokenHierarchy* hitLayers, uint64_t n, EchoContact* out,
+                                        uint64_t* status, void* stream)
+{
+	QueryBuffers b = {};
+	b.rays = rays, b.hits = hits, b.layers = hitLayers, b.out = out;
+	return query_device(scene, "echo_b200_interact_batch_device", true, QUERY_INTERACT, b, rays && hits && out, n, status, stream);
+}
+
+int32_t echo_b200_scatter_sample_batch_device(EchoScene* scene, const EchoRay* rays, const EchoHit* hits, const EchoTokenHierarchy* hitLayers, const float* samples2,
+                                              uint64_t n, EchoScatter* out, uint64_t* status, void* stream)
+{
+	QueryBuffers b = {};
+	b.rays = rays, b.hits = hits, b.layers = hitLayers, b.values = samples2, b.out = out;
+	return query_device(scene, "echo_b200_scatter_sample_batch_device", true, QUERY_SCATTER_SAMPLE, b, rays && hits && samples2 && out, n, status, stream);
+}
+
+int32_t echo_b200_scatter_evaluate_batch_device(EchoScene* scene, const EchoRay* rays, const EchoHit* hits, const EchoTokenHierarchy* hitLayers, const float* incident3,
+                                                uint64_t n, float* outRGBA, uint64_t* status, void* stream)
+{
+	QueryBuffers b = {};
+	b.rays = rays, b.hits = hits, b.layers = hitLayers, b.values = incident3, b.out = outRGBA;
+	return query_device(scene, "echo_b200_scatter_evaluate_batch_device", true, QUERY_SCATTER_EVALUATE, b, rays && hits && incident3 && outRGBA, n, status, stream);
+}
+
+int32_t echo_b200_light_pick_batch_device(EchoScene* scene, const EchoSurface* points, const float* samples1, uint64_t n, uint32_t* tokens, EchoTokenHierarchy* layers,
+                                          float* pmf, uint64_t* status, void* stream)
+{
+	QueryBuffers b = {};
+	b.points = points, b.values = samples1, b.out = tokens, b.outLayers = layers, b.outPmf = pmf;
+	return query_device(scene, "echo_b200_light_pick_batch_device", false, QUERY_PICK, b, points && samples1 && tokens && pmf, n, status, stream);
+}
+
+int32_t echo_b200_light_mass_batch_device(EchoScene* scene, const uint32_t* tokens, const EchoTokenHierarchy* layers, const EchoSurface* points, uint64_t n, float* pmf,
+                                          uint64_t* status, void* stream)
+{
+	QueryBuffers b = {};
+	b.tokens = tokens, b.layers = layers, b.points = points, b.out = pmf;
+	return query_device(scene, "echo_b200_light_mass_batch_device", false, QUERY_MASS, b, tokens && points && pmf, n, status, stream);
+}
+
+int32_t echo_b200_light_sample_batch_device(EchoScene* scene, const uint32_t* tokens, const EchoTokenHierarchy* layers, const EchoSurface* points, const float* samples2,
+                                            uint64_t n, EchoLightSample* out, uint64_t* status, void* stream)
+{
+	QueryBuffers b = {};
+	b.tokens = tokens, b.layers = layers, b.points = points, b.values = samples2, b.out = out;
+	return query_device(scene, "echo_b200_light_sample_batch_device", false, QUERY_SAMPLE, b, tokens && points && samples2 && out, n, status, stream);
+}
+
+int32_t echo_b200_light_pdf_batch_device(EchoScene* scene, const uint32_t* tokens, const EchoTokenHierarchy* layers, const EchoSurface* points, const float* incident3,
+                                         uint64_t n, float* pdf, uint64_t* status, void* stream)
+{
+	QueryBuffers b = {};
+	b.tokens = tokens, b.layers = layers, b.points = points, b.values = incident3, b.out = pdf;
+	return query_device(scene, "echo_b200_light_pdf_batch_device", false, QUERY_PDF, b, tokens && points && incident3 && pdf, n, status, stream);
+}
+
+int32_t echo_b200_evaluate_infinite_batch_device(EchoScene* scene, const float* directions3, uint64_t n, int32_t direct, float* outRGB3, uint64_t* status, void* stream)
+{
+	QueryBuffers b = {};
+	b.values = directions3, b.out = outRGB3, b.direct = direct;
+	return query_device(scene, "echo_b200_evaluate_infinite_batch_device", false, QUERY_INFINITE, b, directions3 && outRGB3, n, status, stream);
+}
+
+int32_t echo_b200_trace_batch_hierarchy_device(EchoScene* scene, const EchoRay* rays, const EchoTokenHierarchy* ignore, uint64_t n, EchoHit* hits,
+                                               EchoTokenHierarchy* hitLayers, void* stream)
+{
+	return hierarchy_device(scene, rays, ignore, n, hits, hitLayers, nullptr, stream);
+}
+
+int32_t echo_b200_occlude_batch_hierarchy_device(EchoScene* scene, const EchoRay* rays, const EchoTokenHierarchy* ignore, uint64_t n, uint8_t* occluded, void* stream)
+{
+	return hierarchy_device(scene, rays, ignore, n, nullptr, nullptr, occluded, stream);
+}
+
+const char* echo_b200_query_reason(uint32_t code)
+{
+	const char* text = rules::reason_text(code);
+	return text ? text : "not a refusal code";
 }
 
 int32_t echo_b200_trace_batch_device(EchoScene* scene, const EchoRay* rays, uint64_t n, EchoHit* hits, void* stream)

@@ -73,7 +73,9 @@ bool render_tiles(RenderState* state, const DeviceScene& scene, const EchoRender
 bool launch_frame_resolve(float4* frame, int32_t width, int32_t height, cudaStream_t stream);
 
 // render.cu: the batched PreparedScene queries of echo_b200_query.h, one thread per query over device buffers, in the instantiation
-// the renderer picks for `scene`. Inputs must have passed the host-side validation of api.cu.
+// the renderer picks for `scene`. Unchecked (`checked` = false), inputs must have passed the host-side validation of api.cu; checked,
+// every thread runs the same rules (echo_query_rules.h) on its own query first and reports a refusal to `status`
+// (echo_b200_query_device.h).
 enum QueryOp : int { QUERY_INTERACT, QUERY_SCATTER_SAMPLE, QUERY_SCATTER_EVALUATE, QUERY_PICK, QUERY_MASS, QUERY_SAMPLE, QUERY_PDF, QUERY_INFINITE };
 struct QueryBuffers
 {
@@ -87,8 +89,9 @@ struct QueryBuffers
 	EchoTokenHierarchy* outLayers;     // pick (nullable)
 	float* outPmf;                     // pick
 	int32_t direct;                    // evaluate_infinite
+	unsigned long long* status;        // checked launches: atomicMin of (index << 8) | reason of every refused query
 };
-bool launch_query(const DeviceScene& scene, int op, const QueryBuffers& buffers, uint64_t n, cudaStream_t stream);
+bool launch_query(const DeviceScene& scene, int op, const QueryBuffers& buffers, uint64_t n, cudaStream_t stream, bool checked);
 
 // tuning switches of the wavefront (the ECHO_B200_<NAME> environment variables), changeable at run time; false = unknown name
 bool set_render_option(const char* name, long long value);

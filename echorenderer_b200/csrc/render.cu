@@ -22,6 +22,7 @@
 #include "echo_shading.cuh"
 #include "echo_instanced.cuh"
 #include "echo_traverse.cuh"
+#include "echo_query_rules.h"
 
 namespace echo
 {
@@ -2253,8 +2254,64 @@ __global__ void __launch_bounds__(kBlock) frame_resolve_kernel(float4* frame, ui
 // ---------------------------------------------------------------------------------------------------------------------
 // batched PreparedScene queries (include/echo_b200_query.h): one thread per query over the same device functions the path
 // kernels call (interact, bsdf_*, scene_pick, scene_probability_mass, scene_sample_light, scene_light_pdf, evaluate_infinite),
-// so a query answers what a rendered path computes. api.cu has validated every token, layer and value before the upload.
+// so a query answers what a rendered path computes. Unchecked (CHECKED = false, the host-buffer calls), api.cu has validated every
+// token, layer and value before the upload. Checked (the device-buffer calls of include/echo_b200_query_device.h), each thread first
+// runs the same rules (echo_query_rules.h) on its own query; a refused query lowers the status word and gets the zeroed record of a miss.
 // ---------------------------------------------------------------------------------------------------------------------
+
+// the scene as echo_query_rules.h reaches it on the device: EchoPack and EchoInstance records verbatim, materials in triShade[.w]
+struct DeviceRuleScene
+{
+	const DeviceScene& scene;
+
+	ECHO_DEVICE uint32_t packCount() const { return scene.packCount; }
+	ECHO_DEVICE EchoPack pack(uint32_t p) const
+	{
+		const uint4* data = scene.packs + (size_t)p * 4;
+		const uint4 words[4] = { __ldg(data), __ldg(data + 1), __ldg(data + 2), __ldg(data + 3) };
+		EchoPack record;
+		memcpy(&record, words, sizeof record);
+		return record;
+	}
+	ECHO_DEVICE void instance(uint32_t i, uint32_t& pack, uint32_t& materialOffset) const
+	{
+		const float4 tail = __ldg(instance_data(scene, i) + 6); // {forwardScale, inverseScale, pack, materialOffset}
+		pack = __float_as_uint(tail.z);
+		materialOffset = __float_as_uint(tail.w);
+	}
+	ECHO_DEVICE uint32_t triangleCount() const { return scene.triangleCount; }
+	ECHO_DEVICE uint32_t sphereCount() const { return scene.sphereCount; }
+	ECHO_DEVICE uint32_t pointLightCount() const { return scene.pointLightCount; }
+	ECHO_DEVICE uint32_t infiniteLightCount() const { return scene.infiniteLightCount; }
+	ECHO_DEVICE uint32_t materialCount() const { return scene.materialCount; }
+	ECHO_DEVICE uint32_t triangleMaterial(uint32_t t) const { return __float_as_uint(__ldg(scene.triShade + (size_t)t * 3).w); }
+	ECHO_DEVICE uint32_t sphereMaterial(uint32_t s) const { return __ldg(scene.sphereMaterial + s); }
+};
+
+// true when query i is refused: the status keeps the lowest (i << 8) | reason of all refused queries
+ECHO_DEVICE bool query_refused(const QueryBuffers& q, uint64_t i, uint32_t code)
+{
+	if (code == rules::ACCEPTED) return false;
+	atomicMin(q.status, (i << 8) | code);
+	return true;
+}
+
+// the rules of the contact calls (VALUES floats per query: 0, 2 samples, 3 an incident direction) and of the light calls
+template<int VALUES>
+ECHO_DEVICE bool contact_accepted(const DeviceScene& scene, const QueryBuffers& q, uint64_t i)
+{
+	uint32_t layer;
+	return !query_refused(q, i, rules::check_contact(DeviceRuleScene{ scene }, q.layers ? q.layers + i : nullptr, q.rays[i], q.hits[i], VALUES ? q.values + i * VALUES : nullptr,
+	                                                 VALUES, layer));
+}
+
+template<int VALUES>
+ECHO_DEVICE bool light_accepted(const DeviceScene& scene, const QueryBuffers& q, uint64_t i)
+{
+	uint32_t layer;
+	return !query_refused(q, i, rules::check_light_query(DeviceRuleScene{ scene }, q.layers ? q.layers + i : nullptr, q.tokens[i], q.points[i],
+	                                                     VALUES ? q.values + i * VALUES : nullptr, VALUES, layer));
+}
 
 ECHO_DEVICE PathLayers query_layers(const EchoTokenHierarchy* layers, uint64_t i)
 {
@@ -2281,7 +2338,7 @@ ECHO_DEVICE bool query_contact(const DeviceScene& scene, const QueryBuffers& q, 
 	return true;
 }
 
-template<bool INST>
+template<bool INST, bool CHECKED>
 __global__ void __launch_bounds__(kBlock) query_interact_kernel(DeviceScene scene, QueryBuffers q, uint64_t n)
 {
 	uint64_t i = (uint64_t)blockIdx.x * kBlock + threadIdx.x;
@@ -2291,7 +2348,7 @@ __global__ void __launch_bounds__(kBlock) query_interact_kernel(DeviceScene scen
 	o.material = ECHO_TOKEN_EMPTY;
 	Contact c;
 
-	if (query_contact<INST>(scene, q, i, c))
+	if ((!CHECKED || contact_accepted<0>(scene, q, i)) && query_contact<INST>(scene, q, i, c))
 	{
 		query_store(o.position, c.point.position);
 		query_store(o.normal, c.point.normal);
@@ -2308,7 +2365,7 @@ __global__ void __launch_bounds__(kBlock) query_interact_kernel(DeviceScene scen
 	static_cast<EchoContact*>(q.out)[i] = o;
 }
 
-template<bool INST>
+template<bool INST, bool CHECKED>
 __global__ void __launch_bounds__(kBlock) query_scatter_sample_kernel(DeviceScene scene, QueryBuffers q, uint64_t n)
 {
 	uint64_t i = (uint64_t)blockIdx.x * kBlock + threadIdx.x;
@@ -2317,7 +2374,7 @@ __global__ void __launch_bounds__(kBlock) query_scatter_sample_kernel(DeviceScen
 	EchoScatter o = {};
 	Contact c;
 
-	if (query_contact<INST>(scene, q, i, c))
+	if ((!CHECKED || contact_accepted<2>(scene, q, i)) && query_contact<INST>(scene, q, i, c))
 	{
 		vec3 incident;
 		int selectedType;
@@ -2331,7 +2388,7 @@ __global__ void __launch_bounds__(kBlock) query_scatter_sample_kernel(DeviceScen
 	static_cast<EchoScatter*>(q.out)[i] = o;
 }
 
-template<bool INST>
+template<bool INST, bool CHECKED>
 __global__ void __launch_bounds__(kBlock) query_scatter_evaluate_kernel(DeviceScene scene, QueryBuffers q, uint64_t n)
 {
 	uint64_t i = (uint64_t)blockIdx.x * kBlock + threadIdx.x;
@@ -2340,7 +2397,7 @@ __global__ void __launch_bounds__(kBlock) query_scatter_evaluate_kernel(DeviceSc
 	float4 o = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
 	Contact c;
 
-	if (query_contact<INST>(scene, q, i, c))
+	if ((!CHECKED || contact_accepted<3>(scene, q, i)) && query_contact<INST>(scene, q, i, c))
 	{
 		vec3 incident = query_vec3(q.values, i);
 		o = make4(bsdf_evaluate<KINDS_ALL>(c.bsdf, c.outgoing, incident), bsdf_pdf<KINDS_ALL>(c.bsdf, c.outgoing, incident));
@@ -2349,11 +2406,19 @@ __global__ void __launch_bounds__(kBlock) query_scatter_evaluate_kernel(DeviceSc
 	static_cast<float4*>(q.out)[i] = o;
 }
 
-template<bool INST>
+template<bool INST, bool CHECKED>
 __global__ void __launch_bounds__(kBlock) query_pick_kernel(DeviceScene scene, QueryBuffers q, uint64_t n)
 {
 	uint64_t i = (uint64_t)blockIdx.x * kBlock + threadIdx.x;
 	if (i >= n) return;
+
+	if (CHECKED && query_refused(q, i, rules::check_pick(q.points[i], q.values[i])))
+	{
+		static_cast<uint32_t*>(q.out)[i] = ECHO_TOKEN_EMPTY;
+		q.outPmf[i] = 0.0f;
+		if (q.outLayers) q.outLayers[i] = EchoTokenHierarchy{};
+		return;
+	}
 
 	float pmf;
 	PathLayers layers;
@@ -2372,17 +2437,18 @@ __global__ void __launch_bounds__(kBlock) query_pick_kernel(DeviceScene scene, Q
 	}
 }
 
-template<bool INST>
+template<bool INST, bool CHECKED>
 __global__ void __launch_bounds__(kBlock) query_mass_kernel(DeviceScene scene, QueryBuffers q, uint64_t n)
 {
 	uint64_t i = (uint64_t)blockIdx.x * kBlock + threadIdx.x;
 	if (i >= n) return;
 
+	const bool accepted = !CHECKED || light_accepted<0>(scene, q, i);
 	uint32_t token = q.tokens[i];
-	static_cast<float*>(q.out)[i] = token == ECHO_TOKEN_EMPTY ? 0.0f : scene_probability_mass<INST>(scene, token, query_layers(q.layers, i), query_point(q.points[i]));
+	static_cast<float*>(q.out)[i] = !accepted || token == ECHO_TOKEN_EMPTY ? 0.0f : scene_probability_mass<INST>(scene, token, query_layers(q.layers, i), query_point(q.points[i]));
 }
 
-template<bool INST>
+template<bool INST, bool CHECKED>
 __global__ void __launch_bounds__(kBlock) query_sample_kernel(DeviceScene scene, QueryBuffers q, uint64_t n)
 {
 	uint64_t i = (uint64_t)blockIdx.x * kBlock + threadIdx.x;
@@ -2391,7 +2457,7 @@ __global__ void __launch_bounds__(kBlock) query_sample_kernel(DeviceScene scene,
 	EchoLightSample o = {};
 	uint32_t token = q.tokens[i];
 
-	if (token != ECHO_TOKEN_EMPTY)
+	if ((!CHECKED || light_accepted<2>(scene, q, i)) && token != ECHO_TOKEN_EMPTY)
 	{
 		vec3 incident;
 		float travel;
@@ -2405,49 +2471,59 @@ __global__ void __launch_bounds__(kBlock) query_sample_kernel(DeviceScene scene,
 	static_cast<EchoLightSample*>(q.out)[i] = o;
 }
 
-template<bool INST>
+template<bool INST, bool CHECKED>
 __global__ void __launch_bounds__(kBlock) query_pdf_kernel(DeviceScene scene, QueryBuffers q, uint64_t n)
 {
 	uint64_t i = (uint64_t)blockIdx.x * kBlock + threadIdx.x;
 	if (i >= n) return;
 
+	const bool accepted = !CHECKED || light_accepted<3>(scene, q, i);
 	uint32_t token = q.tokens[i];
-	static_cast<float*>(q.out)[i] = token == ECHO_TOKEN_EMPTY ? 0.0f : scene_light_pdf<INST>(scene, token, query_layers(q.layers, i), query_point(q.points[i]), query_vec3(q.values, i));
+	static_cast<float*>(q.out)[i] = !accepted || token == ECHO_TOKEN_EMPTY ? 0.0f : scene_light_pdf<INST>(scene, token, query_layers(q.layers, i), query_point(q.points[i]), query_vec3(q.values, i));
 }
 
+template<bool CHECKED>
 __global__ void __launch_bounds__(kBlock) query_infinite_kernel(DeviceScene scene, QueryBuffers q, uint64_t n)
 {
 	uint64_t i = (uint64_t)blockIdx.x * kBlock + threadIdx.x;
 	if (i >= n) return;
+
+	if (CHECKED && query_refused(q, i, rules::check_infinite(q.values + i * 3)))
+	{
+		query_store(static_cast<float*>(q.out) + i * 3, make_rgb(0.0f));
+		return;
+	}
+
 	query_store(static_cast<float*>(q.out) + i * 3, evaluate_infinite(scene, query_vec3(q.values, i), q.direct != 0));
 }
 
-template<bool INST>
+template<bool INST, bool CHECKED>
 static bool launch_query_inst(const DeviceScene& scene, int op, const QueryBuffers& q, uint64_t n, cudaStream_t stream)
 {
 	const unsigned int blocks = (unsigned int)((n + kBlock - 1) / kBlock);
 
 	switch (op)
 	{
-		case QUERY_INTERACT: query_interact_kernel<INST><<<blocks, kBlock, 0, stream>>>(scene, q, n); break;
-		case QUERY_SCATTER_SAMPLE: query_scatter_sample_kernel<INST><<<blocks, kBlock, 0, stream>>>(scene, q, n); break;
-		case QUERY_SCATTER_EVALUATE: query_scatter_evaluate_kernel<INST><<<blocks, kBlock, 0, stream>>>(scene, q, n); break;
-		case QUERY_PICK: query_pick_kernel<INST><<<blocks, kBlock, 0, stream>>>(scene, q, n); break;
-		case QUERY_MASS: query_mass_kernel<INST><<<blocks, kBlock, 0, stream>>>(scene, q, n); break;
-		case QUERY_SAMPLE: query_sample_kernel<INST><<<blocks, kBlock, 0, stream>>>(scene, q, n); break;
-		case QUERY_PDF: query_pdf_kernel<INST><<<blocks, kBlock, 0, stream>>>(scene, q, n); break;
-		case QUERY_INFINITE: query_infinite_kernel<<<blocks, kBlock, 0, stream>>>(scene, q, n); break;
+		case QUERY_INTERACT: query_interact_kernel<INST, CHECKED><<<blocks, kBlock, 0, stream>>>(scene, q, n); break;
+		case QUERY_SCATTER_SAMPLE: query_scatter_sample_kernel<INST, CHECKED><<<blocks, kBlock, 0, stream>>>(scene, q, n); break;
+		case QUERY_SCATTER_EVALUATE: query_scatter_evaluate_kernel<INST, CHECKED><<<blocks, kBlock, 0, stream>>>(scene, q, n); break;
+		case QUERY_PICK: query_pick_kernel<INST, CHECKED><<<blocks, kBlock, 0, stream>>>(scene, q, n); break;
+		case QUERY_MASS: query_mass_kernel<INST, CHECKED><<<blocks, kBlock, 0, stream>>>(scene, q, n); break;
+		case QUERY_SAMPLE: query_sample_kernel<INST, CHECKED><<<blocks, kBlock, 0, stream>>>(scene, q, n); break;
+		case QUERY_PDF: query_pdf_kernel<INST, CHECKED><<<blocks, kBlock, 0, stream>>>(scene, q, n); break;
+		case QUERY_INFINITE: query_infinite_kernel<CHECKED><<<blocks, kBlock, 0, stream>>>(scene, q, n); break;
 		default: set_error("unknown scene query"); return false;
 	}
 
 	return check_cuda(cudaGetLastError(), "scene query launch");
 }
 
-bool launch_query(const DeviceScene& scene, int op, const QueryBuffers& buffers, uint64_t n, cudaStream_t stream)
+bool launch_query(const DeviceScene& scene, int op, const QueryBuffers& buffers, uint64_t n, cudaStream_t stream, bool checked)
 {
 	if (n == 0) return true;
 	const bool instanced = scene.packCount != 0u || scene.textureCount != 0u; // evaluate_paths_stack's choice of the shading instantiation
-	return instanced ? launch_query_inst<true>(scene, op, buffers, n, stream) : launch_query_inst<false>(scene, op, buffers, n, stream);
+	if (checked) return instanced ? launch_query_inst<true, true>(scene, op, buffers, n, stream) : launch_query_inst<false, true>(scene, op, buffers, n, stream);
+	return instanced ? launch_query_inst<true, false>(scene, op, buffers, n, stream) : launch_query_inst<false, false>(scene, op, buffers, n, stream);
 }
 
 // ---------------------------------------------------------------------------------------------------------------------

@@ -304,6 +304,52 @@ class PreparedScene:
             _native.check(self._lib.echo_b200_occlude_batch_device_counted(self._handle, ctypes.c_void_p(rays_pointer), count, ctypes.c_void_p(occluded_pointer),
                                                                          ctypes.c_void_p(counts_pointer), ctypes.c_void_p(stream)))
 
+    # ---- the queries above on device buffers (include/echo_b200_query_device.h): raw device addresses (ints; None for a
+    # nullable buffer) in the order of the C calls, asynchronous on `stream`. Tokens and layers are checked on the device: every
+    # refused query lowers the uint64 at `status_pointer` (set it to _native.QUERY_STATUS_CLEAR first; _native.query_status reads it) ----
+    def _query_device(self, function, *arguments, stream=0):
+        _native.check(getattr(self._lib, function)(self._handle, *arguments, stream))
+
+    def interact_device(self, rays_pointer, hits_pointer, layers_pointer, count, out_pointer, status_pointer, stream=0):
+        """interact: structs.CONTACT records at out_pointer"""
+        self._query_device("echo_b200_interact_batch_device", rays_pointer, hits_pointer, layers_pointer, count, out_pointer, status_pointer, stream=stream)
+
+    def scatter_sample_device(self, rays_pointer, hits_pointer, layers_pointer, samples_pointer, count, out_pointer, status_pointer, stream=0):
+        """scatter_sample with float32[n, 2] samples: structs.SCATTER records"""
+        self._query_device("echo_b200_scatter_sample_batch_device", rays_pointer, hits_pointer, layers_pointer, samples_pointer, count, out_pointer, status_pointer, stream=stream)
+
+    def scatter_evaluate_device(self, rays_pointer, hits_pointer, layers_pointer, incident_pointer, count, out_pointer, status_pointer, stream=0):
+        """scatter_evaluate towards float32[n, 3] directions: float32[n, 4]"""
+        self._query_device("echo_b200_scatter_evaluate_batch_device", rays_pointer, hits_pointer, layers_pointer, incident_pointer, count, out_pointer, status_pointer, stream=stream)
+
+    def pick_device(self, points_pointer, samples_pointer, count, tokens_pointer, layers_pointer, pmf_pointer, status_pointer, stream=0):
+        """pick: uint32 tokens, structs.TOKEN_HIERARCHY layers (nullable) and float32 pmf"""
+        self._query_device("echo_b200_light_pick_batch_device", points_pointer, samples_pointer, count, tokens_pointer, layers_pointer, pmf_pointer, status_pointer, stream=stream)
+
+    def probability_mass_device(self, tokens_pointer, layers_pointer, points_pointer, count, out_pointer, status_pointer, stream=0):
+        """probability_mass: float32[n]"""
+        self._query_device("echo_b200_light_mass_batch_device", tokens_pointer, layers_pointer, points_pointer, count, out_pointer, status_pointer, stream=stream)
+
+    def sample_device(self, tokens_pointer, layers_pointer, points_pointer, samples_pointer, count, out_pointer, status_pointer, stream=0):
+        """sample with float32[n, 2] samples: structs.LIGHT_SAMPLE records"""
+        self._query_device("echo_b200_light_sample_batch_device", tokens_pointer, layers_pointer, points_pointer, samples_pointer, count, out_pointer, status_pointer, stream=stream)
+
+    def probability_density_device(self, tokens_pointer, layers_pointer, points_pointer, incident_pointer, count, out_pointer, status_pointer, stream=0):
+        """probability_density towards float32[n, 3] directions: float32[n]"""
+        self._query_device("echo_b200_light_pdf_batch_device", tokens_pointer, layers_pointer, points_pointer, incident_pointer, count, out_pointer, status_pointer, stream=stream)
+
+    def evaluate_infinite_device(self, directions_pointer, count, direct, out_pointer, status_pointer, stream=0):
+        """evaluate_infinite along float32[n, 3] directions: float32[n, 3]"""
+        self._query_device("echo_b200_evaluate_infinite_batch_device", directions_pointer, count, 1 if direct else 0, out_pointer, status_pointer, stream=stream)
+
+    def trace_hierarchy_device(self, rays_pointer, ignore_pointer, count, hits_pointer, layers_pointer, stream=0):
+        """trace_hierarchy: structs.HIT and structs.TOKEN_HIERARCHY (nullable) records; ignore layers nullable"""
+        self._query_device("echo_b200_trace_batch_hierarchy_device", rays_pointer, ignore_pointer, count, hits_pointer, layers_pointer, stream=stream)
+
+    def occlude_hierarchy_device(self, rays_pointer, ignore_pointer, count, occluded_pointer, stream=0):
+        """occlude_hierarchy: uint8 0/1"""
+        self._query_device("echo_b200_occlude_batch_hierarchy_device", rays_pointer, ignore_pointer, count, occluded_pointer, stream=stream)
+
     # ---- tile rendering ----
     def render_tiles(self, params, tile_xy):
         """One EvaluationOperation worth of tiles -> (tiles[n, tileSize, tileSize, 4] float32, stats record)."""
