@@ -5,7 +5,7 @@ scene preparation in C++), the ctypes binding, and the host-side mirror of the r
 """
 from . import structs  # noqa: F401
 from .host import InstanceDescription, PackDescription, PreparedArrays, SceneDescription, TextureDescription, prepare  # noqa: F401
-from .scene import (AlbedoEvaluator, EvaluationOperation, EvaluationProfile, NormalDepthEvaluator, PathTracedEvaluator,  # noqa: F401
+from .scene import (AlbedoEvaluator, DeviceEvaluator, Evaluation, EvaluationOperation, EvaluationProfile, NormalDepthEvaluator, PathTracedEvaluator,  # noqa: F401
                     PreparedScene, RenderTexture, StandardNaiveEvaluator, build_light_tree_device, build_packs_device, build_qbvh_device, hilbert_curve_pattern, ordered_pattern,
                     shard_epochs, shard_tiles)
 from ._native import EchoNativeError  # noqa: F401

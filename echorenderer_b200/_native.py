@@ -50,6 +50,12 @@ DEVICE_QUERY_EXPORTS = [
     "echo_b200_evaluate_infinite_batch_device", "echo_b200_trace_batch_hierarchy_device", "echo_b200_occlude_batch_hierarchy_device", "echo_b200_query_reason",
 ]
 
+# every symbol include/echo_b200_evaluation.h declares: one EvaluationOperation driven by a host's own evaluator
+EVALUATION_EXPORTS = [
+    "echo_b200_evaluation_create", "echo_b200_evaluation_next_epoch", "echo_b200_evaluation_spawn_device", "echo_b200_evaluation_draw_device",
+    "echo_b200_evaluation_accumulate_device", "echo_b200_evaluation_finish", "echo_b200_evaluation_destroy",
+]
+
 QUERY_STATUS_CLEAR = 0xFFFFFFFFFFFFFFFF  # ECHO_QUERY_STATUS_CLEAR: what a status word holds before the calls, and after them when no query was refused
 
 
@@ -133,6 +139,13 @@ def library():
         "echo_b200_evaluate_infinite_batch_device": [p, p, u64, i32, p, p, p],
         "echo_b200_trace_batch_hierarchy_device": [p, p, p, u64, p, p, p],
         "echo_b200_occlude_batch_hierarchy_device": [p, p, p, u64, p, p],
+        "echo_b200_evaluation_create": [p, p, p, u32, p, ctypes.POINTER(p)],
+        "echo_b200_evaluation_next_epoch": [p, ctypes.POINTER(u64)],
+        "echo_b200_evaluation_spawn_device": [p, p, p, p],
+        "echo_b200_evaluation_draw_device": [p, u32, u32, p],
+        "echo_b200_evaluation_accumulate_device": [p, p],
+        "echo_b200_evaluation_finish": [p, p, p, p],
+        "echo_b200_evaluation_destroy": [p],
     }
 
     for name, argtypes in signatures.items():

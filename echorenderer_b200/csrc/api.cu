@@ -303,6 +303,16 @@ bool single_device(EchoScene* scene)
 	return true;
 }
 
+// an include/echo_b200_evaluation.h call on a live evaluation, on its device
+template<class Call>
+int32_t evaluation_call(EchoEvaluation* evaluation, Call call)
+{
+	if (!evaluation) return fail(ECHO_B200_ERR_INVALID, "evaluation is null");
+	DeviceGuard guard(evaluation_device(evaluation));
+	if (!guard.ok) return ECHO_B200_ERR_NO_DEVICE;
+	return call();
+}
+
 constexpr uint32_t kDealBlock = 64; // consecutive tiles of the caller's sequence that stay on one device (echo_b200.h, scene_create_multi)
 
 } // namespace
@@ -1694,6 +1704,51 @@ int32_t echo_b200_frame_resolve_device(EchoScene* scene, float* frame, int32_t w
 	cudaStream_t s = stream ? (cudaStream_t)stream : scene->stream;
 	return launch_frame_resolve((float4*)frame, width, height, s) ? ECHO_B200_OK : ECHO_B200_ERR_CUDA;
 }
+
+// ---- include/echo_b200_evaluation.h: the state and the launches are render.cu's (evaluation_*); here the arguments and the device ----
+
+int32_t echo_b200_evaluation_create(EchoScene* scene, const EchoRenderParams* params, const int32_t* tileXY, uint32_t tileCount, void* stream, EchoEvaluation** out)
+{
+	if (!require_committed(scene) || !single_device(scene)) return ECHO_B200_ERR_INVALID;
+	if (!params || (!tileXY && tileCount) || !out) return fail(ECHO_B200_ERR_INVALID, "null argument");
+	*out = nullptr;
+	if (!evaluation_params_valid(*params, tileCount)) return ECHO_B200_ERR_INVALID;
+	DeviceGuard guard(scene->device);
+	if (!guard.ok) return ECHO_B200_ERR_NO_DEVICE;
+	return evaluation_create(scene->d, scene->device, *params, tileXY, tileCount, (cudaStream_t)stream, out);
+}
+
+int32_t echo_b200_evaluation_next_epoch(EchoEvaluation* evaluation, uint64_t* count)
+{
+	if (evaluation && !count) return fail(ECHO_B200_ERR_INVALID, "null argument");
+	return evaluation_call(evaluation, [&] { return evaluation_next_epoch(evaluation, count); });
+}
+
+int32_t echo_b200_evaluation_spawn_device(EchoEvaluation* evaluation, EchoRay* rays, int32_t* pixelXY, uint32_t* sampleIndex)
+{
+	return evaluation_call(evaluation, [&] { return evaluation_spawn(evaluation, rays, pixelXY, sampleIndex); });
+}
+
+int32_t echo_b200_evaluation_draw_device(EchoEvaluation* evaluation, uint32_t dimension, uint32_t components, float* out)
+{
+	return evaluation_call(evaluation, [&] { return evaluation_draw(evaluation, dimension, components, out); });
+}
+
+int32_t echo_b200_evaluation_accumulate_device(EchoEvaluation* evaluation, const float* samples)
+{
+	return evaluation_call(evaluation, [&] { return evaluation_accumulate(evaluation, samples); });
+}
+
+int32_t echo_b200_evaluation_finish(EchoEvaluation* evaluation, float* outRGBA, float* frame, EchoStats* stats)
+{
+	return evaluation_call(evaluation, [&] { return evaluation_finish(evaluation, outRGBA, frame, stats); });
+}
+
+int32_t echo_b200_evaluation_destroy(EchoEvaluation* evaluation)
+{
+	return evaluation_call(evaluation, [&] { evaluation_destroy(evaluation); return (int32_t)ECHO_B200_OK; });
+}
+
 
 int32_t echo_b200_debug_evaluate_samples(EchoScene* scene, const EchoRenderParams* params, const int32_t* pixelXY, const uint32_t* sampleIndex, uint64_t n, float* outRGB)
 {

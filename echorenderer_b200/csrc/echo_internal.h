@@ -6,6 +6,7 @@
 #include <string>
 #include <vector>
 
+#include "../../include/echo_b200_evaluation.h"
 #include "../../include/echo_b200_query.h"
 #include "echo_scene.cuh"
 
@@ -71,6 +72,20 @@ bool render_tiles(RenderState* state, const DeviceScene& scene, const EchoRender
                   float4* tilesOut, float4* frame, EchoStats* stats, cudaStream_t stream);
 
 bool launch_frame_resolve(float4* frame, int32_t width, int32_t height, cudaStream_t stream);
+
+// render.cu: one EvaluationOperation driven by a host's own evaluator (include/echo_b200_evaluation.h). `params` must have passed
+// evaluation_params_valid. Each call checks its own order and inputs and returns an ECHO_B200_* status with the error set; the
+// caller has made `device` current.
+bool evaluation_params_valid(const EchoRenderParams& params, uint32_t tileCount);
+int32_t evaluation_create(const DeviceScene& scene, int device, const EchoRenderParams& params, const int32_t* tileXY, uint32_t tileCount, cudaStream_t stream,
+                          EchoEvaluation** out);
+int evaluation_device(const EchoEvaluation* evaluation);
+int32_t evaluation_next_epoch(EchoEvaluation* evaluation, uint64_t* count);
+int32_t evaluation_spawn(EchoEvaluation* evaluation, EchoRay* rays, int32_t* pixelXY, uint32_t* sampleIndex);
+int32_t evaluation_draw(EchoEvaluation* evaluation, uint32_t dimension, uint32_t components, float* out);
+int32_t evaluation_accumulate(EchoEvaluation* evaluation, const float* samples);
+int32_t evaluation_finish(EchoEvaluation* evaluation, float* outRGBA, float* frame, EchoStats* stats);
+void evaluation_destroy(EchoEvaluation* evaluation);
 
 // render.cu: the batched PreparedScene queries of echo_b200_query.h, one thread per query over device buffers, in the instantiation
 // the renderer picks for `scene`. Unchecked (`checked` = false), inputs must have passed the host-side validation of api.cu; checked,

@@ -1133,6 +1133,32 @@ ECHO_DEVICE Strata path_strata(const EchoRenderParams& params, const PathBuffers
 	return { 0u, 0u, 0u };
 }
 
+ECHO_DEVICE uint32_t pixel_index(const EchoRenderParams& params, int2 pixel) { return (uint32_t)pixel.y * (uint32_t)params.width + (uint32_t)pixel.x; }
+
+// the key of a sample's draws: Distribution.BeginSeries per epoch (stratified) or per sample
+template<bool STRAT>
+ECHO_DEVICE uint32_t slot_key(const EchoRenderParams& params, uint32_t pixelIndex, uint32_t sampleIndex)
+{
+	return STRAT ? stratified_series(params.seed, pixelIndex, sampleIndex / (uint32_t)params.extend) : sample_key(params.seed, pixelIndex, sampleIndex);
+}
+
+// Camera.SpawnRay with CameraSample.Create (CameraSample.cs:19-23) of one sample: the camera ray of raygen_kernel and spawn_kernel.
+// The stratified draws take the sample's place in its epoch from *strataSample (raygen_kernel reads it through PathBuffers), the key
+// from *sample. Returns the key.
+template<bool STRAT>
+ECHO_DEVICE uint32_t camera_ray(const EchoCamera& camera, const EchoRenderParams& params, int2 pixel, const uint32_t* sample, const uint32_t* strataSample,
+                                vec3& origin, vec3& direction)
+{
+	const uint32_t pixelIndex = pixel_index(params, pixel);
+	const Strata strata = STRAT ? make_strata((uint32_t)params.extend, *strataSample) : Strata{ 0u, 0u, 0u };
+	uint32_t key = slot_key<STRAT>(params, pixelIndex, *sample);
+
+	vec2 shift = draw2d<STRAT>(key, strata, 0u);
+	vec2 lens = draw2d<STRAT>(key, strata, 2u);
+	camera_spawn(camera, params.width, params.height, pixel.x, pixel.y, shift, lens, origin, direction);
+	return key;
+}
+
 template<bool STRAT>
 __global__ void __launch_bounds__(kBlock) raygen_kernel(DeviceScene scene, EchoRenderParams params, uint32_t count, const int2* __restrict__ pixelXY,
                                                        const uint32_t* __restrict__ sampleIndex, PathBuffers paths)
@@ -1141,16 +1167,8 @@ __global__ void __launch_bounds__(kBlock) raygen_kernel(DeviceScene scene, EchoR
 	if (i >= count) return;
 
 	int2 pixel = pixelXY[i];
-	const uint32_t pixelIndex = (uint32_t)pixel.y * (uint32_t)params.width + (uint32_t)pixel.x;
-	const Strata strata = path_strata<STRAT>(params, paths, i);
-	uint32_t key = STRAT ? stratified_series(params.seed, pixelIndex, sampleIndex[i] / (uint32_t)params.extend) // Distribution.BeginSeries per epoch
-	                     : sample_key(params.seed, pixelIndex, sampleIndex[i]);
-
-	vec2 shift = draw2d<STRAT>(key, strata, 0u); // CameraSample.Create, CameraSample.cs:19-23
-	vec2 lens = draw2d<STRAT>(key, strata, 2u);
-
 	vec3 origin, direction;
-	camera_spawn(scene.camera, params.width, params.height, pixel.x, pixel.y, shift, lens, origin, direction);
+	uint32_t key = camera_ray<STRAT>(scene.camera, params, pixel, sampleIndex + i, paths.sampleIndex + i, origin, direction);
 
 	stream_store(paths.rayQueue[0] + i * 2u, make_float4(origin.x, origin.y, origin.z, direction.x));
 	stream_store(paths.rayQueue[0] + i * 2u + 1u, make_float4(direction.y, direction.z, kInfinity, __uint_as_float(ECHO_TOKEN_EMPTY)));
@@ -1159,6 +1177,46 @@ __global__ void __launch_bounds__(kBlock) raygen_kernel(DeviceScene scene, EchoR
 	stream_store(paths.energy + i, make_float4(1.0f, 1.0f, 1.0f, 0.0f));
 	stream_store(paths.result + i, make_float4(0.0f, 0.0f, 0.0f, __uint_as_float(MODE_FIRST << 16)));
 	stream_store(paths.key + i, key);
+}
+
+// ---- a host's own evaluator (echo_b200_evaluation.h): the camera ray and the draws of every slot of an epoch ----
+
+template<bool STRAT>
+__global__ void __launch_bounds__(kBlock) spawn_kernel(EchoCamera camera, EchoRenderParams params, uint32_t count, const int2* __restrict__ pixelXY,
+                                                      const uint32_t* __restrict__ sampleIndex, EchoRay* __restrict__ rays, int2* __restrict__ outPixelXY,
+                                                      uint32_t* __restrict__ outSampleIndex)
+{
+	uint32_t i = blockIdx.x * kBlock + threadIdx.x;
+	if (i >= count) return;
+
+	int2 pixel = pixelXY[i];
+	vec3 origin, direction;
+	camera_ray<STRAT>(camera, params, pixel, sampleIndex + i, sampleIndex + i, origin, direction);
+
+	rays[i] = EchoRay{ { origin.x, origin.y, origin.z }, { direction.x, direction.y, direction.z }, kInfinity, ECHO_TOKEN_EMPTY };
+	if (outPixelXY) outPixelXY[i] = pixel;
+	if (outSampleIndex) outSampleIndex[i] = sampleIndex[i];
+}
+
+// Next1D (components 1) or Next2D (components 2, dimensions d and d + 1) of every slot at `dimension`
+template<bool STRAT>
+__global__ void __launch_bounds__(kBlock) draw_kernel(EchoRenderParams params, uint32_t count, const int2* __restrict__ pixelXY, const uint32_t* __restrict__ sampleIndex,
+                                                     uint32_t dimension, uint32_t components, float* __restrict__ out)
+{
+	uint32_t i = blockIdx.x * kBlock + threadIdx.x;
+	if (i >= count) return;
+
+	uint32_t sample = sampleIndex[i];
+	uint32_t key = slot_key<STRAT>(params, pixel_index(params, pixelXY[i]), sample);
+	const Strata strata = STRAT ? make_strata((uint32_t)params.extend, sample) : Strata{ 0u, 0u, 0u };
+
+	if (components == 1u) out[i] = draw1d<STRAT>(key, strata, dimension);
+	else
+	{
+		vec2 value = draw2d<STRAT>(key, strata, dimension);
+		out[(size_t)i * 2u] = value.x;
+		out[(size_t)i * 2u + 1u] = value.y;
+	}
 }
 
 ECHO_DEVICE int classify_material(const DeviceScene& scene, uint32_t materialIndex)
@@ -3018,15 +3076,77 @@ static bool evaluate_paths_dispatch(WorkerState* state, const DeviceScene& scene
 	}
 }
 
-static void collect_stats(WorkerState* state, EchoStats* stats, uint64_t launches, cudaStream_t stream)
+static void collect_stats(const unsigned long long* deviceStats, EchoStats* stats, uint64_t launches, cudaStream_t stream)
 {
 	if (!stats) return;
 	unsigned long long host[STAT_COUNT];
-	cudaMemcpyAsync(host, state->paths.stats, sizeof(host), cudaMemcpyDeviceToHost, stream);
+	cudaMemcpyAsync(host, deviceStats, sizeof(host), cudaMemcpyDeviceToHost, stream);
 	cudaStreamSynchronize(stream);
 	uint64_t* out = reinterpret_cast<uint64_t*>(stats);
 	for (int i = 0; i < STAT_COUNT; i++) out[i] += host[i];
 	stats->kernelLaunches += launches;
+}
+
+// The per-pixel side of EvaluationOperation.Execute over one batch of tiles (EvaluationOperation.cs:100-141): the pixel list, the
+// (pixel, sample index) of every slot of an epoch, the Accumulator of every pixel and the epoch loop. render_batch runs it on a
+// worker's wavefront state with the built-in evaluators, an EchoEvaluation on buffers of its own with the host's evaluator.
+struct EpochState
+{
+	int2* batchPixelXY;        // per pixel of the batch
+	uint32_t* activePixels[2]; // this epoch's and the next epoch's active pixels
+	float4* accumulator;
+	uint32_t* sampleCount;
+	int32_t* tileXYDevice;
+	int2* pixelXY;             // per slot of an epoch
+	uint32_t* sampleIndex;
+	uint32_t* counters;        // 64 words, COUNTER_PIXELS
+	unsigned long long* stats; // EchoStats layout
+	uint32_t* hostCount;       // pinned: the active-pixel count read after a synchronise
+};
+
+// lays out the batch's pixels; `activePixels` = the pixels inside the image. Synchronises `stream`.
+static bool epochs_begin(const EpochState& e, const EchoRenderParams& params, const int32_t* tileXY, uint32_t tiles, uint32_t pixelTotal, cudaStream_t stream,
+                         uint64_t& launches, uint32_t& activePixels)
+{
+	if (!check_cuda(cudaMemcpyAsync(e.tileXYDevice, tileXY, sizeof(int32_t) * 2 * tiles, cudaMemcpyHostToDevice, stream), "cudaMemcpyAsync(tiles)")) return false;
+	if (!check_cuda(cudaMemsetAsync(e.counters, 0, sizeof(uint32_t) * 64, stream), "cudaMemsetAsync(counters)")) return false;
+
+	batch_pixels_kernel<<<blocks_for(pixelTotal), kBlock, 0, stream>>>(params, e.tileXYDevice, tiles, e.batchPixelXY, e.activePixels[0], e.counters, e.accumulator, e.sampleCount);
+	++launches;
+
+	if (!check_cuda(cudaMemcpyAsync(e.hostCount, e.counters + COUNTER_PIXELS, sizeof(uint32_t), cudaMemcpyDeviceToHost, stream), "cudaMemcpyAsync(pixels)")) return false;
+	if (!check_cuda(cudaStreamSynchronize(stream), "batch setup")) return false;
+	activePixels = *e.hostCount;
+	return true;
+}
+
+static void epoch_slots(const EpochState& e, const EchoRenderParams& params, uint32_t activePixels, int list, uint32_t epoch, cudaStream_t stream, uint64_t& launches)
+{
+	epoch_slots_kernel<<<blocks_for((uint64_t)activePixels * (uint32_t)params.extend), kBlock, 0, stream>>>(params, activePixels, e.activePixels[list], e.batchPixelXY, epoch,
+	                                                                                                      e.pixelXY, e.sampleIndex);
+	++launches;
+}
+
+// Accumulator.Add of the epoch's samples and the stop test; the count of the pixels that go on is on its way to *e.hostCount
+static bool epoch_accumulate(const EpochState& e, const EchoRenderParams& params, uint32_t activePixels, int list, uint32_t epoch, const float4* samples, cudaStream_t stream,
+                             uint64_t& launches, KernelTimer* timer)
+{
+	if (!check_cuda(cudaMemsetAsync(e.counters + COUNTER_PIXELS, 0, sizeof(uint32_t), stream), "cudaMemsetAsync(pixel counter)")) return false;
+
+	if (timer) timer->start(stream);
+	accumulate_kernel<<<blocks_for(activePixels), kBlock, 0, stream>>>(params, activePixels, e.activePixels[list], samples, e.accumulator, e.sampleCount, epoch,
+	                                                                 e.activePixels[list ^ 1], e.counters, e.stats);
+	if (timer) timer->stop(KernelTimer::ACCUMULATE, stream);
+	++launches;
+
+	return check_cuda(cudaMemcpyAsync(e.hostCount, e.counters + COUNTER_PIXELS, sizeof(uint32_t), cudaMemcpyDeviceToHost, stream), "cudaMemcpyAsync(pixels)");
+}
+
+static bool epochs_resolve(const EpochState& e, const EchoRenderParams& params, uint32_t pixelTotal, float4* tilesOut, float4* frame, cudaStream_t stream, uint64_t& launches)
+{
+	resolve_tiles_kernel<<<blocks_for(pixelTotal), kBlock, 0, stream>>>(params, pixelTotal, e.batchPixelXY, e.accumulator, e.sampleCount, tilesOut, frame, e.stats);
+	++launches;
+	return check_cuda(cudaGetLastError(), "resolve_tiles_kernel launch");
 }
 
 // one batch of tiles: pixel loop -> epoch loop -> sample loop of EvaluationOperation.Execute (EvaluationOperation.cs:100-141)
@@ -3038,46 +3158,27 @@ static bool render_batch(WorkerState* state, const DeviceScene& scene, const Ech
 	uint32_t pixelTotal = (uint32_t)(tiles * perTile);
 
 	if (!ensure_capacity(state, (uint64_t)pixelTotal * params.extend, pixelTotal, tiles, scene.packCount != 0u || scene.textureCount != 0u)) return false;
-	if (!check_cuda(cudaMemcpyAsync(state->tileXYDevice, tileXY, sizeof(int32_t) * 2 * tiles, cudaMemcpyHostToDevice, stream), "cudaMemcpyAsync(tiles)")) return false;
-	if (!check_cuda(cudaMemsetAsync(state->paths.counters, 0, sizeof(uint32_t) * 64, stream), "cudaMemsetAsync(counters)")) return false;
 
-	batch_pixels_kernel<<<blocks_for(pixelTotal), kBlock, 0, stream>>>(params, state->tileXYDevice, tiles, state->batchPixelXY, state->activePixels[0],
-	                                                                 state->paths.counters, state->accumulator, state->sampleCount);
-	++launches;
-
-	if (!check_cuda(cudaMemcpyAsync(state->hostCounters + 8, state->paths.counters + COUNTER_PIXELS, sizeof(uint32_t), cudaMemcpyDeviceToHost, stream), "cudaMemcpyAsync(pixels)")) return false;
-	if (!check_cuda(cudaStreamSynchronize(stream), "batch setup")) return false;
-
-	uint32_t activePixels = state->hostCounters[8];
+	const EpochState e = { state->batchPixelXY, { state->activePixels[0], state->activePixels[1] }, state->accumulator, state->sampleCount, state->tileXYDevice,
+	                       state->pixelXY, state->sampleIndex, state->paths.counters, state->paths.stats, state->hostCounters + 8 };
+	uint32_t activePixels = 0;
+	if (!epochs_begin(e, params, tileXY, tiles, pixelTotal, stream, launches, activePixels)) return false;
 	int list = 0;
 
 	for (uint32_t epoch = 1; activePixels > 0 && epoch <= (uint32_t)params.maxEpoch; epoch++)
 	{
 		uint32_t slots = activePixels * (uint32_t)params.extend;
 
-		epoch_slots_kernel<<<blocks_for(slots), kBlock, 0, stream>>>(params, activePixels, state->activePixels[list], state->batchPixelXY, epoch, state->pixelXY, state->sampleIndex);
-		++launches;
-
+		epoch_slots(e, params, activePixels, list, epoch, stream, launches);
 		if (!evaluate_paths_dispatch(state, scene, params, slots, launches, stream)) return false;
-
-		if (!check_cuda(cudaMemsetAsync(state->paths.counters + COUNTER_PIXELS, 0, sizeof(uint32_t), stream), "cudaMemsetAsync(pixel counter)")) return false;
-
-		state->timer.start(stream);
-		accumulate_kernel<<<blocks_for(activePixels), kBlock, 0, stream>>>(params, activePixels, state->activePixels[list], state->sampleOut, state->accumulator,
-		                                                                 state->sampleCount, epoch, state->activePixels[list ^ 1], state->paths.counters, state->paths.stats);
-		state->timer.stop(KernelTimer::ACCUMULATE, stream);
-		++launches;
-
-		if (!check_cuda(cudaMemcpyAsync(state->hostCounters + 8, state->paths.counters + COUNTER_PIXELS, sizeof(uint32_t), cudaMemcpyDeviceToHost, stream), "cudaMemcpyAsync(pixels)")) return false;
+		if (!epoch_accumulate(e, params, activePixels, list, epoch, state->sampleOut, stream, launches, &state->timer)) return false;
 		if (!check_cuda(cudaStreamSynchronize(stream), "epoch")) return false;
 
-		activePixels = state->hostCounters[8];
+		activePixels = *e.hostCount;
 		list ^= 1;
 	}
 
-	resolve_tiles_kernel<<<blocks_for(pixelTotal), kBlock, 0, stream>>>(params, pixelTotal, state->batchPixelXY, state->accumulator, state->sampleCount, tilesOut, frame, state->paths.stats);
-	++launches;
-	return check_cuda(cudaGetLastError(), "resolve_tiles_kernel launch");
+	return epochs_resolve(e, params, pixelTotal, tilesOut, frame, stream, launches);
 }
 
 bool stratified_extend_valid(const EchoRenderParams& params)
@@ -3085,14 +3186,28 @@ bool stratified_extend_valid(const EchoRenderParams& params)
 	return (params.evaluator & ECHO_DISTRIBUTION_STRATIFIED) == 0 || (params.extend > 0 && params.extend <= ECHO_DISTRIBUTION_STRATIFIED_EXTEND_MAX);
 }
 
-bool render_tiles(RenderState* state, const DeviceScene& scene, const EchoRenderParams& params, const int32_t* tileXY, uint32_t tileCount,
-                  float4* tilesOut, float4* frame, EchoStats* stats, cudaStream_t stream)
+// the checks every EvaluationOperation makes of its parameters, whoever evaluates: sizes, extend, epochs, the stratified extend
+static bool operation_params_valid(const EchoRenderParams& params)
 {
 	if (params.width <= 0 || params.height <= 0 || params.tileSize <= 0 || params.extend <= 0 || params.maxEpoch < 1 || params.minEpoch > params.maxEpoch)
 	{
 		set_error("invalid EchoRenderParams");
 		return false;
 	}
+
+	if (!stratified_extend_valid(params))
+	{
+		set_error("ECHO_DISTRIBUTION_STRATIFIED takes an extend of 1 to 2^23");
+		return false;
+	}
+
+	return true;
+}
+
+bool render_tiles(RenderState* state, const DeviceScene& scene, const EchoRenderParams& params, const int32_t* tileXY, uint32_t tileCount,
+                  float4* tilesOut, float4* frame, EchoStats* stats, cudaStream_t stream)
+{
+	if (!operation_params_valid(params)) return false;
 
 	if ((params.evaluator & ECHO_EVALUATOR_KIND_MASK) == ECHO_EVALUATOR_NAIVE && (params.bounceLimit < 0 || params.bounceLimit > kNaiveBounceCap))
 	{
@@ -3110,12 +3225,6 @@ bool render_tiles(RenderState* state, const DeviceScene& scene, const EchoRender
 	if ((params.evaluator & ECHO_EVALUATOR_COUNT_VISITS) != 0 && (params.evaluator & ECHO_EVALUATOR_KIND_MASK) != ECHO_EVALUATOR_PATH_TRACED)
 	{
 		set_error("ECHO_EVALUATOR_COUNT_VISITS is a switch of the path-traced evaluator");
-		return false;
-	}
-
-	if (!stratified_extend_valid(params))
-	{
-		set_error("ECHO_DISTRIBUTION_STRATIFIED takes an extend of 1 to 2^23");
 		return false;
 	}
 
@@ -3210,9 +3319,213 @@ bool render_tiles(RenderState* state, const DeviceScene& scene, const EchoRender
 		return false;
 	}
 
-	for (int i = 0; i < workerCount; i++) collect_stats(state->workers[i], stats, launches[i], state->workers[i]->stream);
+	for (int i = 0; i < workerCount; i++) collect_stats(state->workers[i]->paths.stats, stats, launches[i], state->workers[i]->stream);
 	if (profiling()) state->workers[0]->timer.report();
 	return true;
+}
+
+} // namespace echo
+
+// One EvaluationOperation a host drives with its own evaluator (echo_b200_evaluation.h): the EpochState of one batch of tiles on
+// buffers of its own, and the order of the calls
+struct EchoEvaluation
+{
+	int device = 0;
+	cudaStream_t stream = nullptr;
+	EchoCamera camera = {};
+	EchoRenderParams params = {};
+	uint32_t pixelTotal = 0;
+	echo::EpochState e = {};
+	std::vector<void*> allocations;
+	uint32_t activePixels = 0; // of the open epoch; after accumulate, the count of the next one is on its way to *e.hostCount
+	uint32_t epoch = 0;        // the last epoch opened, from 1
+	int list = 0;              // e.activePixels[list] lists the pixels of the open epoch
+	bool open = false;         // opened by next_epoch, closed by accumulate
+	bool counting = false;     // accumulate ran: next_epoch reads the count of the pixels that go on
+	bool done = false;         // next_epoch returned 0
+	uint64_t launches = 0;
+};
+
+namespace echo
+{
+
+constexpr uint64_t kEvaluationSlots = 1ull << 31;
+constexpr uint64_t kEvaluationPixels = 1ull << 30; // the accumulator of pixel p is at p * 4 (32-bit index)
+
+bool evaluation_params_valid(const EchoRenderParams& params, uint32_t tileCount)
+{
+	if (!operation_params_valid(params)) return false;
+
+	if ((params.evaluator & ~ECHO_DISTRIBUTION_STRATIFIED) != 0)
+	{
+		set_error("an evaluation takes EchoRenderParams.evaluator 0 or ECHO_DISTRIBUTION_STRATIFIED: the host is the evaluator");
+		return false;
+	}
+
+	uint64_t pixels = (uint64_t)tileCount * (uint64_t)params.tileSize * (uint64_t)params.tileSize;
+	if (pixels > kEvaluationPixels || pixels * (uint64_t)params.extend > kEvaluationSlots)
+	{
+		set_error("an evaluation holds at most 2^31 slots (tiles x tileSize^2 x extend) and 2^30 pixels: split the tiles into several evaluations");
+		return false;
+	}
+
+	return true;
+}
+
+static int32_t refuse(const char* message)
+{
+	set_error(message);
+	return ECHO_B200_ERR_INVALID;
+}
+
+static bool aligned(const void* pointer, uintptr_t bytes) { return ((uintptr_t)pointer & (bytes - 1u)) == 0u; }
+
+template<class T>
+static bool allocate(EchoEvaluation* evaluation, T*& pointer, uint64_t count)
+{
+	void* p = nullptr;
+	if (!check_cuda(cudaMalloc(&p, sizeof(T) * std::max<uint64_t>(count, 1)), "cudaMalloc(evaluation)")) return false;
+	evaluation->allocations.push_back(p);
+	pointer = (T*)p;
+	return true;
+}
+
+void evaluation_destroy(EchoEvaluation* evaluation)
+{
+	if (!evaluation) return;
+	if (evaluation->e.hostCount) cudaFreeHost(evaluation->e.hostCount);
+	for (void* p : evaluation->allocations) cudaFree(p);
+	delete evaluation;
+}
+
+int evaluation_device(const EchoEvaluation* evaluation) { return evaluation->device; }
+
+int32_t evaluation_create(const DeviceScene& scene, int device, const EchoRenderParams& params, const int32_t* tileXY, uint32_t tileCount, cudaStream_t stream,
+                          EchoEvaluation** out)
+{
+	for (uint64_t i = 0; i < (uint64_t)tileCount * 2; i++)
+		if (tileXY[i] < 0 || ((int64_t)tileXY[i] + 1) * params.tileSize > INT32_MAX) return refuse("a tile position is negative or beyond the largest image");
+
+	EchoEvaluation* evaluation = new EchoEvaluation();
+	evaluation->device = device;
+	evaluation->stream = stream;
+	evaluation->camera = scene.camera;
+	evaluation->params = params;
+	evaluation->pixelTotal = (uint32_t)((uint64_t)tileCount * params.tileSize * params.tileSize);
+
+	const uint64_t pixels = evaluation->pixelTotal, slots = pixels * (uint64_t)params.extend;
+	EpochState& e = evaluation->e;
+	bool ok = allocate(evaluation, e.batchPixelXY, pixels) && allocate(evaluation, e.activePixels[0], pixels) && allocate(evaluation, e.activePixels[1], pixels)
+		&& allocate(evaluation, e.accumulator, pixels * 4) && allocate(evaluation, e.sampleCount, pixels) && allocate(evaluation, e.tileXYDevice, (uint64_t)tileCount * 2)
+		&& allocate(evaluation, e.pixelXY, slots) && allocate(evaluation, e.sampleIndex, slots) && allocate(evaluation, e.counters, 64)
+		&& allocate(evaluation, e.stats, STAT_COUNT) && check_cuda(cudaMallocHost((void**)&e.hostCount, sizeof(uint32_t)), "cudaMallocHost(evaluation)")
+		&& check_cuda(cudaMemsetAsync(e.stats, 0, sizeof(unsigned long long) * STAT_COUNT, stream), "cudaMemsetAsync(stats)")
+		&& epochs_begin(e, params, tileXY, tileCount, evaluation->pixelTotal, stream, evaluation->launches, evaluation->activePixels);
+
+	if (!ok)
+	{
+		evaluation_destroy(evaluation);
+		return ECHO_B200_ERR_CUDA;
+	}
+
+	*out = evaluation;
+	return ECHO_B200_OK;
+}
+
+int32_t evaluation_next_epoch(EchoEvaluation* evaluation, uint64_t* count)
+{
+	EchoEvaluation& v = *evaluation;
+	if (v.open) return refuse("echo_b200_evaluation_next_epoch: the open epoch has not been accumulated (echo_b200_evaluation_accumulate_device)");
+
+	if (v.counting)
+	{
+		if (!check_cuda(cudaStreamSynchronize(v.stream), "epoch")) return ECHO_B200_ERR_CUDA;
+		v.activePixels = *v.e.hostCount;
+		v.list ^= 1;
+		v.counting = false;
+	}
+
+	if (v.done || v.activePixels == 0u || v.epoch >= (uint32_t)v.params.maxEpoch)
+	{
+		v.done = true;
+		*count = 0;
+		return ECHO_B200_OK;
+	}
+
+	++v.epoch;
+	epoch_slots(v.e, v.params, v.activePixels, v.list, v.epoch, v.stream, v.launches);
+	if (!check_cuda(cudaGetLastError(), "epoch_slots_kernel launch")) return ECHO_B200_ERR_CUDA;
+	v.open = true;
+	*count = (uint64_t)v.activePixels * (uint32_t)v.params.extend;
+	return ECHO_B200_OK;
+}
+
+int32_t evaluation_spawn(EchoEvaluation* evaluation, EchoRay* rays, int32_t* pixelXY, uint32_t* sampleIndex)
+{
+	EchoEvaluation& v = *evaluation;
+	if (!v.open) return refuse("echo_b200_evaluation_spawn_device: no epoch is open (echo_b200_evaluation_next_epoch)");
+	if (!rays) return refuse("echo_b200_evaluation_spawn_device: d_rays is null");
+	if (!aligned(rays, 4) || !aligned(pixelXY, 8) || !aligned(sampleIndex, 4)) return refuse("echo_b200_evaluation_spawn_device: a misaligned buffer");
+
+	uint32_t count = v.activePixels * (uint32_t)v.params.extend;
+	if ((v.params.evaluator & ECHO_DISTRIBUTION_STRATIFIED) != 0)
+		spawn_kernel<true><<<blocks_for(count), kBlock, 0, v.stream>>>(v.camera, v.params, count, v.e.pixelXY, v.e.sampleIndex, rays, (int2*)pixelXY, sampleIndex);
+	else spawn_kernel<false><<<blocks_for(count), kBlock, 0, v.stream>>>(v.camera, v.params, count, v.e.pixelXY, v.e.sampleIndex, rays, (int2*)pixelXY, sampleIndex);
+	++v.launches;
+	return check_cuda(cudaGetLastError(), "spawn_kernel launch") ? ECHO_B200_OK : ECHO_B200_ERR_CUDA;
+}
+
+int32_t evaluation_draw(EchoEvaluation* evaluation, uint32_t dimension, uint32_t components, float* out)
+{
+	EchoEvaluation& v = *evaluation;
+	if (!v.open) return refuse("echo_b200_evaluation_draw_device: no epoch is open (echo_b200_evaluation_next_epoch)");
+	if (components != 1u && components != 2u) return refuse("echo_b200_evaluation_draw_device: components is 1 (Next1D) or 2 (Next2D)");
+	if (!out) return refuse("echo_b200_evaluation_draw_device: d_out is null");
+	if (!aligned(out, 4)) return refuse("echo_b200_evaluation_draw_device: a misaligned buffer");
+
+	uint32_t count = v.activePixels * (uint32_t)v.params.extend;
+	if ((v.params.evaluator & ECHO_DISTRIBUTION_STRATIFIED) != 0)
+		draw_kernel<true><<<blocks_for(count), kBlock, 0, v.stream>>>(v.params, count, v.e.pixelXY, v.e.sampleIndex, dimension, components, out);
+	else draw_kernel<false><<<blocks_for(count), kBlock, 0, v.stream>>>(v.params, count, v.e.pixelXY, v.e.sampleIndex, dimension, components, out);
+	++v.launches;
+	return check_cuda(cudaGetLastError(), "draw_kernel launch") ? ECHO_B200_OK : ECHO_B200_ERR_CUDA;
+}
+
+int32_t evaluation_accumulate(EchoEvaluation* evaluation, const float* samples)
+{
+	EchoEvaluation& v = *evaluation;
+	if (!v.open) return refuse("echo_b200_evaluation_accumulate_device: no epoch is open (echo_b200_evaluation_next_epoch); an epoch is accumulated once");
+	if (!samples) return refuse("echo_b200_evaluation_accumulate_device: d_samples_rgba is null");
+	if (!aligned(samples, 16)) return refuse("echo_b200_evaluation_accumulate_device: d_samples_rgba is not 16-byte aligned");
+
+	if (!epoch_accumulate(v.e, v.params, v.activePixels, v.list, v.epoch, (const float4*)samples, v.stream, v.launches, nullptr)) return ECHO_B200_ERR_CUDA;
+	v.open = false;
+	v.counting = true;
+	return ECHO_B200_OK;
+}
+
+int32_t evaluation_finish(EchoEvaluation* evaluation, float* outRGBA, float* frame, EchoStats* stats)
+{
+	EchoEvaluation& v = *evaluation;
+	if (v.open) return refuse("echo_b200_evaluation_finish: an epoch is open; accumulate it first");
+	if (!aligned(frame, 16)) return refuse("echo_b200_evaluation_finish: d_frame_rgba is not 16-byte aligned");
+
+	// Pixel/Evaluated counts the pixels of this resolve only: a preview followed by the final finish reports each pixel once
+	float4* tiles = nullptr;
+	bool ok = check_cuda(cudaMemsetAsync(v.e.stats + STAT_PIXEL_EVALUATED, 0, sizeof(unsigned long long), v.stream), "cudaMemsetAsync(stats)");
+	if (ok && outRGBA) ok = check_cuda(cudaMallocAsync((void**)&tiles, sizeof(float4) * std::max<uint32_t>(v.pixelTotal, 1u), v.stream), "cudaMallocAsync(tiles)");
+	ok = ok && epochs_resolve(v.e, v.params, v.pixelTotal, tiles, (float4*)frame, v.stream, v.launches);
+	if (ok && outRGBA) ok = check_cuda(cudaMemcpyAsync(outRGBA, tiles, sizeof(float4) * v.pixelTotal, cudaMemcpyDeviceToHost, v.stream), "cudaMemcpyAsync(tiles)");
+	if (tiles) cudaFreeAsync(tiles, v.stream);
+	ok = check_cuda(cudaStreamSynchronize(v.stream), "echo_b200_evaluation_finish") && ok;
+	if (!ok) return ECHO_B200_ERR_CUDA;
+
+	if (stats)
+	{
+		*stats = EchoStats{};
+		collect_stats(v.e.stats, stats, v.launches, v.stream);
+	}
+	return ECHO_B200_OK;
 }
 
 // debug: explicit (pixel, sample) lists -> per-sample radiance (device pointers in, device pointer out)

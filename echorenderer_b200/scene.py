@@ -382,6 +382,11 @@ class PreparedScene:
     def frame_resolve_device(self, frame_pointer, width, height, stream=0):
         _native.check(self._lib.echo_b200_frame_resolve_device(self._handle, ctypes.c_void_p(frame_pointer), width, height, ctypes.c_void_p(stream)))
 
+    def evaluation(self, params, tile_xy, stream=0):
+        """One EvaluationOperation over `tile_xy` driven by the caller's own evaluator (include/echo_b200_evaluation.h), every call on
+        `stream` (a cudaStream_t as an int; 0 = the legacy default stream). An Evaluation: close it, or use it as a context manager."""
+        return Evaluation(self, params, tile_xy, stream)
+
     def evaluate_samples(self, params, pixel_xy, sample_index, channels=3):
         """Diagnostic: one Evaluator.Evaluate per (pixel, sample index) -> radiance[n, 3] (channels=4 keeps the W lane the
         auxiliary evaluators use, e.g. NormalDepth128's depth)."""
@@ -391,6 +396,78 @@ class PreparedScene:
         entry = self._lib.echo_b200_debug_evaluate_samples if channels == 3 else self._lib.echo_b200_debug_evaluate_samples4
         _native.check(entry(self._handle, _native.pointer(params), _native.pointer(pixel_xy), _native.pointer(sample_index), len(sample_index), _native.pointer(out)))
         return out
+
+
+class Evaluation:
+    """echo_b200_evaluation_*: the camera rays, the sample sequence and the per-pixel Accumulator of one EvaluationOperation, on
+    device buffers. Each epoch: next_epoch() -> count slots (0: done), spawn_device / draw_device into the caller's buffers, the
+    caller's evaluator, accumulate_device of count Float4s. Slot = active-pixel position x extend + sample of the epoch. Buffers are
+    raw device addresses (ints), like the other *_device methods."""
+
+    def __init__(self, scene, params, tile_xy, stream=0):
+        self.scene = scene  # the native scene must outlive the evaluation
+        self._lib = _native.library()
+        self.tile_xy = np.ascontiguousarray(tile_xy, dtype=np.int32).reshape(-1, 2)
+        self.tile_size = int(params["tileSize"][0])
+        self.stream = stream
+        self._handle = ctypes.c_void_p()
+        _native.check(self._lib.echo_b200_evaluation_create(scene.handle, _native.pointer(params), _native.pointer(self.tile_xy), len(self.tile_xy),
+                                                            ctypes.c_void_p(stream), ctypes.byref(self._handle)))
+
+    def next_epoch(self):
+        """closes the previous epoch and opens the next one: its slot count, 0 once every pixel has stopped (synchronises the stream)"""
+        count = ctypes.c_uint64()
+        _native.check(self._lib.echo_b200_evaluation_next_epoch(self._handle, ctypes.byref(count)))
+        return count.value
+
+    def spawn_device(self, rays, pixel_xy=None, sample_index=None):
+        """structs.RAY camera rays of every slot; optionally int32 (x, y) pixels and uint32 sample indices"""
+        _native.check(self._lib.echo_b200_evaluation_spawn_device(self._handle, ctypes.c_void_p(rays), ctypes.c_void_p(pixel_xy), ctypes.c_void_p(sample_index)))
+
+    def draw_device(self, dimension, components, out):
+        """float32[count, components]: Next1D (1) or Next2D (2, dimensions d and d + 1) of every slot at `dimension`"""
+        _native.check(self._lib.echo_b200_evaluation_draw_device(self._handle, int(dimension), int(components), ctypes.c_void_p(out)))
+
+    def accumulate_device(self, samples):
+        """Accumulator.Add of float32[count, 4] samples and the epoch stop test"""
+        _native.check(self._lib.echo_b200_evaluation_accumulate_device(self._handle, ctypes.c_void_p(samples)))
+
+    def finish(self, frame_pointer=None):
+        """(tiles[n, tileSize, tileSize, 4] float32, stats record); a device frame (width x height Float4) gets (mean * n, n) added"""
+        tiles = np.zeros((len(self.tile_xy), self.tile_size, self.tile_size, 4), dtype=np.float32)
+        stats = np.zeros(1, dtype=structs.STATS)
+        _native.check(self._lib.echo_b200_evaluation_finish(self._handle, _native.pointer(tiles), ctypes.c_void_p(frame_pointer), _native.pointer(stats)))
+        return tiles, stats
+
+    def close(self):
+        if getattr(self, "_handle", None) is not None and self._handle.value:
+            self._lib.echo_b200_evaluation_destroy(self._handle)
+            self._handle = ctypes.c_void_p()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:  # interpreter shutdown: the library may already be gone
+            pass
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *_):
+        self.close()
+
+
+class DeviceEvaluator:
+    """Evaluation/Evaluators/Evaluator.cs: the base of an evaluator the host writes itself, on device buffers. EvaluationOperation runs
+    it through an Evaluation: each epoch, evaluate(scene, evaluation, count, stream) computes one Float4 per slot (its camera ray from
+    evaluation.spawn_device, its random numbers from evaluation.draw_device; its queries are the scene's *_device calls on `stream`)
+    and returns the device address of the count Float4s, valid until its next call."""
+    bounce_limit = 0     # EchoRenderParams fields of the built-in evaluators, not read by an evaluation
+    survivability = 0.0
+    code = 0
+
+    def evaluate(self, scene, evaluation, count, stream):
+        raise NotImplementedError
 
 
 @dataclass(frozen=True)
@@ -708,9 +785,11 @@ class EvaluationOperation:
     """Processes/Evaluation/EvaluationOperation.cs:21-177 on the GPU: same public surface (tile_positions, destination,
     profile, total_samples, statistics), Execute renders every tile through libecho_b200 and applies it to the destination."""
 
-    def __init__(self, scene: PreparedScene, profile: EvaluationProfile, destination: RenderTexture, tile_positions=None):
+    def __init__(self, scene: PreparedScene, profile: EvaluationProfile, destination: RenderTexture, tile_positions=None, stream=0):
+        """`stream`: the cudaStream_t (an int) a DeviceEvaluator profile runs on; the built-in evaluators do not use it."""
         profile.validate()
         self.scene = scene
+        self.stream = stream
         self.profile = profile
         self.destination = destination
         self.tile_positions = destination.tile_positions if tile_positions is None else np.asarray(tile_positions, dtype=np.int32).reshape(-1, 2)
@@ -729,12 +808,26 @@ class EvaluationOperation:
         return int(self.statistics["sampleEvaluated"][0])
 
     def execute(self):
-        tiles, stats = self.scene.render_tiles(self.params, self.tile_positions)
+        if isinstance(self.profile.evaluator, DeviceEvaluator):
+            tiles, stats = self._evaluate_on_device()
+        else:
+            tiles, stats = self.scene.render_tiles(self.params, self.tile_positions)
         for position, tile in zip(self.tile_positions, tiles):
             self.destination.apply(position, tile)
         for name in structs.STATS_FIELDS:
             self.statistics[name] += stats[name]
         return self.destination
+
+    def _evaluate_on_device(self):
+        """EvaluationOperation.cs:100-141 with the profile's DeviceEvaluator: the epoch loop of one Evaluation over every tile"""
+        evaluator = self.profile.evaluator
+        with self.scene.evaluation(self.params, self.tile_positions, stream=self.stream) as evaluation:
+            while True:
+                count = evaluation.next_epoch()
+                if count == 0:
+                    break
+                evaluation.accumulate_device(evaluator.evaluate(self.scene, evaluation, count, self.stream))
+            return evaluation.finish()
 
     def statistics_report(self):
         """label -> count, the labels EvaluatorStatistics.Report uses on this path."""
